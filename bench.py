@@ -35,6 +35,13 @@ no collective.  Rank 0 prints ONE JSON line.
             tensor path), C4 (D=E=64 attention, tensor path), C5 (CG solve, N=10^6) through the plugin API, each
             with ms, its roofline (SURVEY.md section 8d formulas) and oracle parity on sampled rows; under
             torchrun C3/C4 shard target rows and C5 runs the solver across the ranks
+  --dump-outputs DIR
+            after the run, what each timed path returned in its last step: product.npy (the device-resident output,
+            float32), e2e_product.npy (the plugin's float64 result), and one file per config (c1.npy, c3.npy, c4.npy,
+            c5.npy: the plugin's result).  Every file holds all N target rows, also under torchrun: bench.py gathers
+            the row shards of the headline paths and the plugin's get_result gathers those of the configs.  The inputs
+            are seeded, so two builds run with the same arguments can be compared file for file; an output over 6 MiB
+            keeps a seeded sample of its rows, the same one in every run
 """
 import argparse
 import json
@@ -72,7 +79,15 @@ def parse_args():
     ap.add_argument("--parity-rows", type=int, default=256, help="sampled rows checked against the C oracle")
     ap.add_argument("--workload", default="product", choices=["product", "solve"],
                     help="product: the headline C2 product (default); solve: BASELINE config C5, (K + I) b = a at N = 10^6, as the line's own metric")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what each timed path returned in its last step as DIR/<name>.npy (float32 / float64) so that two "
+                         "builds can be compared output for output; an output over 6 MiB is stored as a fixed, seeded sample of rows")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU paths; the reference arm keeps none")
+    return args
 
 
 def workload_config(n, n_gpus, path="auto"):
@@ -132,6 +147,28 @@ def oracle_parity(kernel, y, x, b, got_rows, rows, tol, normalize_rows=False):
 def sample_rows(n, k, seed=2):
     k = int(min(n, k))
     return np.sort(np.random.RandomState(seed).choice(n, k, replace=False))
+
+
+DUMP_ARRAY_BYTES = 6 << 20    # at most eight outputs (product, e2e_product, c1, c3, c4, c4g, c5, c5s) stay under 64 MB
+DUMP_TOTAL_BYTES = 64_000_000
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: name -> array as DIR/<name>.npy.  An array over DUMP_ARRAY_BYTES keeps as many rows as fit,
+    chosen by sample_rows(..., seed=3): the same rows in every run with the same arguments."""
+    os.makedirs(directory, exist_ok=True)
+    total = 0
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a)
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError(f"output {name} is {a.dtype}, not float32 / float64")
+        if a.nbytes > DUMP_ARRAY_BYTES:
+            a = a[sample_rows(a.shape[0], DUMP_ARRAY_BYTES // (a.nbytes // a.shape[0]), seed=3)]
+        path = os.path.join(directory, name + ".npy")
+        np.save(path, a)
+        total += os.path.getsize(path)
+    if total > DUMP_TOTAL_BYTES:
+        raise RuntimeError(f"--dump-outputs wrote {total} bytes, more than {DUMP_TOTAL_BYTES}")
 
 
 # ------------------------------------------------------------------------------------ CPU arm
@@ -389,19 +426,19 @@ def run_b200_arm(args):
     product.set_profiling(True)
     for _ in range(args.warmup):
         step()
-    launches_per_step = product.last_launch_count()
     sampler = ClockSampler(local_rank)
     barrier()
     if rank == 0:
         sampler.start()
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
-    kernel_ms = []
+    kernel_ms, launches = [], 0
     for e0, e1 in ev:
         flush.fill_(1)  # evict L2 between timed steps (outside the event bracket)
         e0.record()
         step()
         e1.record()
         kernel_ms.append(product.last_main_kernel_ms())
+        launches += product.last_launch_count()   # the library's launches of this step's call
     barrier()
     clocks = sampler.stop() if rank == 0 else None
     step_ms = sum(a.elapsed_time(b_) for a, b_ in ev) / args.steps
@@ -446,6 +483,20 @@ def run_b200_arm(args):
     if rank == 0:
         parity = oracle_parity("gaussian", ds.source_points, None, ds.source_signal, timed_rows, prows, tol=1e-5)
         parity["of"] = "the device-resident output of the last timed step"
+
+    dumps = {} if args.dump_outputs else None
+
+    def whole(part):
+        """All N rows of an output whose rows [lo, hi) this rank holds (untimed; every rank must call it)."""
+        if sym or world == 1:
+            return part.cpu().numpy()
+        full = torch.zeros((N,) + tuple(part.shape[1:]), dtype=part.dtype, device=dev)
+        full[lo:hi] = part
+        dist.all_reduce(full)
+        return full.cpu().numpy()
+
+    if dumps is not None:
+        dumps["product"] = whole(out)
 
     # ---- end-to-end arm: plugin API, host float64 arrays in, host float64 result out ------------
     e2e = None
@@ -497,6 +548,8 @@ def run_b200_arm(args):
             "host_ms_per_call": {k: round(1e3 * v / args.steps, 3) for k, v in phases.items()},   # rank 0's clock
         }
         assert res.shape == (n_out, 1)
+        if dumps is not None:
+            dumps["e2e_product"] = whole(torch.from_numpy(res).to(dev))
         if rank == 0:
             sel = prows if (sym or world == 1) else prows[prows < hi]
             e2e["parity"] = oracle_parity("gaussian", ds.source_points, None, ds.source_signal, res[sel], sel, tol=1e-5)
@@ -534,7 +587,7 @@ def run_b200_arm(args):
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
             "ms_per_step": step_ms, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic", "config": workload_config(args.n, world, args.path),
-            "clocks": clocks, "e2e": e2e, "gpu_launches": int(launches_per_step * args.steps),
+            "clocks": clocks, "e2e": e2e, "gpu_launches": launches,
             "roofline": roofline, "parity": parity,
         }
         if general is not None:
@@ -546,12 +599,14 @@ def run_b200_arm(args):
         from bench_configs import run_config_block   # tools/bench_configs.py
 
         configs = run_config_block([c.strip() for c in args.configs.split(",") if c.strip()], local_rank=local_rank, rank=rank,
-                                   world=world, parity_rows=args.parity_rows, peaks=read_peaks())
+                                   world=world, parity_rows=args.parity_rows, peaks=read_peaks(), outputs=dumps)
     if rank == 0:
         if configs is not None:
             line["configs"] = configs
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline(ds, pick_cpu_rows(ds, args.cpu_rows))
+        if dumps is not None:
+            dump_outputs(args.dump_outputs, dumps)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
@@ -561,7 +616,8 @@ def run_b200_arm(args):
 def run_solve_workload(args):
     """--workload solve: config C5 (Gaussian solve (K + I) b = a, N = M = 10^6, preconditioned CG through B200Solver) as the
     line's metric, so that a 1/2/4/8-GPU sweep reports the solve like the product: time of query() (device, max over ranks),
-    iterations, ms per iteration, fit() time, the collective, oracle-scored residual.  One step = one solve."""
+    iterations, ms per iteration, fit() time, the collective, oracle-scored residual.  One step = one solve: --warmup untimed
+    solves, then --steps timed ones."""
     import torch
     import torch.distributed as dist
 
@@ -577,13 +633,18 @@ def run_solve_workload(args):
     if rank == 0:
         sampler.start()
     peaks, _ = read_peaks()
+    dumps = {} if args.dump_outputs else None
     c5 = run_solver("C5: gaussian solve (K + I) b = a, N=M=10^6, D=3, preconditioned CG", args.n, local_rank=local_rank, rank=rank,
-                    world=world, parity_rows=min(args.parity_rows, 128), peaks=peaks)
+                    world=world, parity_rows=min(args.parity_rows, 128), peaks=peaks, runs=args.steps, warm=args.warmup,
+                    outputs=dumps, key="c5")
     if rank == 0:
         clocks = sampler.stop()
+        if dumps is not None:
+            dump_outputs(args.dump_outputs, dumps)
         n = args.n
         print(json.dumps({
-            "metric": "gaussian_kernel_solve_ms", "value": c5["ms"], "unit": "ms", "n_gpus": world, "steps": 1, "warmup": 1,
+            "metric": "gaussian_kernel_solve_ms", "value": c5["ms"], "unit": "ms", "n_gpus": world, "steps": args.steps,
+            "warmup": args.warmup,
             "ms_per_step": c5["ms"], "higher_is_better": False, "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": c5["workload"], "N": n, "M": n, "D": 3, "E": 1, "lam": c5["lam"], "rtol": c5["rtol"],
                        "matvec": c5["matvec"], "preconditioner": c5["preconditioner"], "collective": c5["collective"],

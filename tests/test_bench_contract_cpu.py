@@ -42,3 +42,30 @@ def test_reference_arm_other_ranks_exit_quietly():
     lines = _run(["--impl", "reference", "--n", "20000", "--steps", "1", "--warmup", "1", "--gpus", "2"],
                  env={"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"})
     assert lines == []
+
+
+def test_steps_below_one_are_refused():
+    p = subprocess.run([sys.executable, os.path.join(REPO, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                       timeout=120, cwd=REPO)
+    assert p.returncode == 2 and "--steps" in p.stderr
+
+
+def test_dump_outputs_keeps_small_arrays_and_samples_large_ones_the_same_way(tmp_path):
+    import numpy as np
+    import pytest
+
+    import bench
+
+    big = np.arange(2_000_000, dtype=np.float64).reshape(-1, 2)   # 32 MB, over the per-array limit
+    small = np.linspace(0, 1, 10, dtype=np.float32).reshape(10, 1)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"big": big, "small": small})
+    a, b = np.load(tmp_path / "a" / "big.npy"), np.load(tmp_path / "b" / "big.npy")
+    assert np.array_equal(a, b) and a.dtype == np.float64 and a.shape[1] == 2
+    assert 0 < a.nbytes <= bench.DUMP_ARRAY_BYTES and a.shape[0] >= bench.DUMP_ARRAY_BYTES // 16 - 1
+    rows = a[:, 0] / 2   # whole rows of the original, in order
+    assert np.array_equal(rows, np.round(rows)) and np.all(np.diff(rows) > 0) and np.array_equal(a[:, 1], a[:, 0] + 1)
+    s = np.load(tmp_path / "a" / "small.npy")
+    assert s.dtype == np.float32 and np.array_equal(s, small)
+    with pytest.raises(TypeError):
+        bench.dump_outputs(str(tmp_path / "c"), {"ints": np.arange(4)})

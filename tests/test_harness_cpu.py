@@ -1,13 +1,17 @@
 """The offline harness layer (SURVEY.md section 8f ranks 1-2): the h5py stand-in, the extra dataset
-writers and the plugin's algos.yaml as the *reference's own* parser sees it.  Tests that need the
-reference tree skip when it is neither staged (baseline/_ref) nor mounted (/root/reference)."""
+writers and the plugin's algos.yaml as the *reference's own* parser sees it.  The dataset writers run against the
+stand-in of tests/reference_standin.py and are compared with the reference's outputs stored in tests/golden/; the
+tests that need the reference's parser or runner skip when its tree is neither staged (baseline/_ref) nor named by
+KMB_REFERENCE."""
 import os
 import sys
 
 import numpy as np
 import pytest
 
+from conftest import load_golden
 from kernel_matrix_benchmarks_b200.harness import bootstrap, h5lite
+from reference_standin import UPSTREAM_DATASET, standin_reference  # noqa: F401  (fixture)
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 needs_reference = pytest.mark.skipif(bootstrap.find_reference() is None, reason="reference harness not available")
@@ -70,9 +74,9 @@ def test_h5lite_never_unpickles_and_rejects_foreign_files(tmp_path):
     assert np.array_equal(f.attrs["v"], np.arange(3.0)) and f["metrics"].attrs["rmse"] == 0.5
 
 
-def test_offline_harness_refuses_to_download(tmp_path):
-    """get_dataset (datasets.py:106-109) tries an HTTP download first; the offline harness must not."""
-    bootstrap.activate()
+def test_offline_harness_refuses_to_download(tmp_path, standin_reference):
+    """get_dataset (datasets.py:106-109) tries an HTTP download first; the offline harness must not.  activate() swaps
+    the reference's ``datasets.download``; the stand-in's own ``download`` fails the test if the swap does not happen."""
     import kernel_matrix_benchmarks.datasets as ref_datasets
 
     with pytest.raises(OSError, match="not downloading"):
@@ -88,9 +92,7 @@ def test_shims_do_not_shadow_real_modules():
     assert "numpy" not in shimmed
 
 
-@needs_reference
-def test_extra_datasets_are_registered_and_named_by_contract():
-    bootstrap.activate()
+def test_extra_datasets_are_registered_and_named_by_contract(standin_reference):
     from kernel_matrix_benchmarks.datasets import DATASETS
 
     from kernel_matrix_benchmarks_b200.harness import datasets_ext
@@ -99,36 +101,45 @@ def test_extra_datasets_are_registered_and_named_by_contract():
         assert name in DATASETS
         task, label, d, e, m, n, kernel = name.split("-", 6)  # algos.yaml:38
         assert task in ("product", "attention", "solver") and d[0] == "D" and e[0] == "E" and m[0] == "M" and n[0] == "N"
-    assert "product-sphere-D3-E1-M1000-N1000-inverse-distance" in DATASETS  # the reference's own are kept
+    assert DATASETS[UPSTREAM_DATASET].__name__ == "_upstream_writer"  # the reference's own are kept
 
 
-@needs_reference
-def test_blocked_ground_truth_equals_the_reference_writer(tmp_path, monkeypatch):
-    """write_dataset (blocked GroundTruth) == the reference's write_output on the same arrays."""
-    bootstrap.activate()
-    import h5py
-    from kernel_matrix_benchmarks.datasets import write_output
-
+def _golden_dataset(name):
     from kernel_matrix_benchmarks_b200 import datasets as gen
+
+    g = load_golden(name)
+    ds = gen.KernelDataset(name=name, task=g["task"], kernel=g["kernel"], source_points=g["source_points"],
+                           target_points=g["source_points"] if g["same_points"] else g["target_points"],
+                           source_signal=g["source_signal"], same_points=g["same_points"], normalize_rows=g["normalize_rows"],
+                           density_estimation=g["density_estimation"])
+    return g, ds
+
+
+@pytest.mark.parametrize("name", ["product_gaussian_d16_e2", "product_gaussian_cube_d3", "product_absexp_cube_d3_e3_xy",
+                                  "attention_absoluteexponential_d64_e8"])
+def test_blocked_ground_truth_equals_the_reference_writer(tmp_path, monkeypatch, standin_reference, name):
+    """write_dataset (blocked GroundTruth) == the reference's float64 result on the same arrays (tests/golden, written by
+    the reference's BruteForceProductBLAS in float64 with difference-form distances, which is its GroundTruth)."""
+    import h5py
+
     from kernel_matrix_benchmarks_b200.harness import datasets_ext
 
-    ds = gen.uniform_cube(300, 3, 1.0, "gaussian", "product", n_targets=200, signal_dim=2)
+    g, ds = _golden_dataset(name)
     monkeypatch.setattr(datasets_ext, "TEMP_BYTES", 2 * 8 * ds.M * ds.D * 37)  # force blocks of 37 rows
-    mine, ref = str(tmp_path / "mine.hdf5"), str(tmp_path / "ref.hdf5")
-    datasets_ext.write_dataset(mine, ds, label="ucube", verbose=False)
-    write_output(filename=ref, task="product", kernel="gaussian", short_description="s", description="d",
-                 source_points=ds.source_points, target_points=ds.target_points, source_signal=ds.source_signal)
-    a, b = h5py.File(mine, "r"), h5py.File(ref, "r")
+    fn = str(tmp_path / "mine.hdf5")
+    datasets_ext.write_dataset(fn, ds, label="ucube", verbose=False)
+    a = h5py.File(fn, "r")
     for k in ("source_points", "target_points", "source_signal"):
-        np.testing.assert_array_equal(a[k][:], b[k][:])
-    np.testing.assert_allclose(a["target_signal"][:], b["target_signal"][:], rtol=1e-14, atol=1e-14)
-    for k in ("kernel", "task", "point_type", "normalize_rows", "same_points", "density_estimation"):
-        assert a.attrs[k] == b.attrs[k], k
+        np.testing.assert_array_equal(a[k][:], g[k])
+    got = a["target_signal"][:]
+    assert got.shape == g["truth"].shape
+    assert np.linalg.norm(got - g["truth"]) <= 1e-12 * np.linalg.norm(g["truth"])
+    for k in ("kernel", "task", "normalize_rows", "same_points", "density_estimation"):
+        assert a.attrs[k] == g[k], k
+    assert a.attrs["point_type"] == "float" and "GroundTruth" in a.attrs["truth_source"]
 
 
-@needs_reference
-def test_solver_dataset_rhs_is_lambda_consistent(tmp_path):
-    bootstrap.activate()
+def test_solver_dataset_rhs_is_lambda_consistent(tmp_path, standin_reference):
     import h5py
 
     from kernel_matrix_benchmarks_b200 import datasets as gen
@@ -142,6 +153,11 @@ def test_solver_dataset_rhs_is_lambda_consistent(tmp_path):
     K = np.exp(-((y[:, None, :] - y[None, :, :]) ** 2).sum(-1))
     np.testing.assert_allclose(a, K @ b + b, rtol=1e-12, atol=1e-12)
     assert f.attrs["task"] == "solver" and f.attrs["lam"] == 1.0
+    # and the right-hand side the reference built for the same system (K b through its float64 product, + lam b)
+    g, ds = _golden_dataset("solver_gaussian_cube_d3_lam1")
+    datasets_ext.write_dataset(fn, ds, label="ucubelam1", lam=float(g["lam"]), verbose=False)
+    a = h5py.File(fn, "r")["target_signal"][:]
+    assert np.linalg.norm(a - g["rhs"]) <= 1e-12 * np.linalg.norm(g["rhs"])
 
 
 @needs_reference

@@ -1,15 +1,18 @@
 """The B200 plugin driven by the reference's own runner.run / results / metrics on a B200
-(the drop-in claim of BASELINE.json's north star).  Needs the staged reference tree
-(baseline/_ref, written by ``__graft_entry__.build()`` where /root/reference exists); skips otherwise."""
+(the drop-in claim of BASELINE.json's north star).  The runner tests need the reference tree (staged in baseline/_ref
+or named by KMB_REFERENCE) and skip without it; the dataset tests run against the stand-in of
+tests/reference_standin.py and the reference's outputs stored in tests/golden/."""
 import os
 
 import numpy as np
 import pytest
 
+from conftest import load_golden
 from kernel_matrix_benchmarks_b200.harness import bootstrap
+from reference_standin import standin_reference  # noqa: F401  (fixture)
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(bootstrap.find_reference() is None, reason="reference harness not staged")]
+pytestmark = pytest.mark.gpu
+needs_reference = pytest.mark.skipif(bootstrap.find_reference() is None, reason="reference harness not staged")
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -39,6 +42,7 @@ def _run(dataset, task, dim, hardware="GPU", normalize_rows=False, kernel="gauss
     return rows
 
 
+@needs_reference
 def test_product_through_runner(tmp_path, monkeypatch):
     monkeypatch.chdir(tmp_path)
     rows = _run("product-ucube-D3-E1-M1000-N1000-gaussian", "product", 3)
@@ -51,6 +55,7 @@ def test_product_through_runner(tmp_path, monkeypatch):
         assert m["query-time"] > 0 and m["build-time"] >= 0
 
 
+@needs_reference
 def test_solver_through_runner(tmp_path, monkeypatch):
     monkeypatch.chdir(tmp_path)
     rows = _run("solver-ucubelam1-D3-E1-M2000-N2000-gaussian", "solver", 3)
@@ -70,41 +75,36 @@ def test_solver_through_runner(tmp_path, monkeypatch):
     assert pcg * 4 <= cg, its
 
 
-@pytest.mark.parametrize("case", ["product_d3", "attention_d64", "solver_d3"])
-def test_gpu_written_ground_truth_equals_the_reference(tmp_path, monkeypatch, case):
-    """The BASELINE-size datasets (C2-C5) get their ``target_signal`` from kmb_product_f64; here the same writer on sizes
-    the reference's GroundTruth (datasets.py:180-195) can do in full: every row must agree to 1e-12."""
-    bootstrap.activate()
+@pytest.mark.parametrize("case, golden", [("product_d3", "product_absexp_cube_d3_e3_xy"),
+                                           ("attention_d64", "attention_absoluteexponential_d64_e8"),
+                                           ("solver_d3", "solver_gaussian_cube_d3_lam1")], ids=["product_d3", "attention_d64", "solver_d3"])
+def test_gpu_written_ground_truth_equals_the_reference(tmp_path, monkeypatch, standin_reference, case, golden):
+    """The BASELINE-size datasets (C2-C5) get their ``target_signal`` from kmb_product_f64; here the same writer on the
+    reference's own float64 outputs stored in tests/golden (a product with independent targets and E = 3, row-normalised
+    attention with D = 64, and the right-hand side K b + b of a solve): every row must agree to 1e-12."""
     import h5py
 
     from kernel_matrix_benchmarks_b200 import datasets as gen
     from kernel_matrix_benchmarks_b200.harness import datasets_ext
 
-    if case == "product_d3":
-        ds, lam = gen.uniform_cube(3000, 3, 1.0, "gaussian", "product", n_targets=2000, signal_dim=2), 0.0
-    elif case == "attention_d64":
-        ds, lam = gen.config_c4(1024, 64, 8, "absolute-exponential"), 0.0
-    else:
-        ds, lam = gen.uniform_cube(2500, 3, 1.0, "gaussian", "solver"), 1.0
+    g = load_golden(golden)
+    ds = gen.KernelDataset(name=golden, task=g["task"], kernel=g["kernel"], source_points=g["source_points"],
+                           target_points=g["source_points"] if g["same_points"] else g["target_points"],
+                           source_signal=g["source_signal"], same_points=g["same_points"], normalize_rows=g["normalize_rows"])
+    lam, want = (float(g["lam"]), g["rhs"]) if case == "solver_d3" else (0.0, g["truth"])
     monkeypatch.setattr(datasets_ext, "GPU_TRUTH_MIN_WORK", 1.0)
     monkeypatch.setattr(datasets_ext, "VERIFY_ROWS", 64)
     fn = str(tmp_path / "gpu_truth.hdf5")
     datasets_ext.write_dataset(fn, ds, label="ucube", lam=lam, verbose=False)
     f = h5py.File(fn, "r")
     assert "kmb_product_f64" in f.attrs["truth_source"] and "64 sampled target rows" in f.attrs["truth_source"]
-    want = datasets_ext._ground_truth_blocked(kernel=ds.kernel, source_points=ds.source_points,
-                                              target_points=None if ds.same_points else ds.target_points,
-                                              source_signal=ds.source_signal, normalize_rows=ds.normalize_rows)
-    if lam:
-        want = want + lam * ds.source_signal
     got = f["target_signal"][:]
     assert got.shape == want.shape
     assert np.linalg.norm(got - want) <= 1e-12 * np.linalg.norm(want)
 
 
-def test_baseline_size_datasets_are_registered():
+def test_baseline_size_datasets_are_registered(standin_reference):
     """C2, C3, C4, C5 by the reference's naming contract (algos.yaml:38), with globs of this repo's algos.yaml matching."""
-    bootstrap.activate()
     from kernel_matrix_benchmarks.datasets import DATASETS
 
     for name in ("product-ucube-D3-E1-M1000000-N1000000-gaussian", "product-ucube-D784-E1-M60000-N10000-gaussian",

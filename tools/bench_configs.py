@@ -48,8 +48,10 @@ def _rows(n, k, seed=2):
     return np.sort(np.random.RandomState(seed).choice(n, int(min(n, k)), replace=False))
 
 
-def run_product(name, ds, *, local_rank=0, rank=0, world=1, runs=5, warm=3, parity_rows=256, tol=1e-5, peaks=None, **kw):
-    """One product / attention config through B200Product.  Returns the config's JSON object (rank 0) or None."""
+def run_product(name, ds, *, local_rank=0, rank=0, world=1, runs=5, warm=3, parity_rows=256, tol=1e-5, peaks=None, outputs=None,
+                key=None, **kw):
+    """One product / attention config through B200Product.  Returns the config's JSON object (rank 0) or None.  With
+    `outputs` (a dict), rank 0 also stores the result of the last timed query there under `key`."""
     import torch
 
     from kernel_matrix_benchmarks_b200 import product as _product
@@ -84,6 +86,8 @@ def run_product(name, ds, *, local_rank=0, rank=0, world=1, runs=5, warm=3, pari
     query_ms, kernel_ms, fit_ms = _max_over_ranks([sum(q_ms) / len(q_ms), sum(k_ms) / len(k_ms), fit_ms], dev, world)
     if rank != 0:
         return None
+    if outputs is not None:
+        outputs[key] = res
     pairs = float(ds.N) * ds.M
     rows = _rows(ds.N, parity_rows)
     out = {"workload": name, "kernel": ds.kernel, "N": ds.N, "M": ds.M, "D": ds.D, "E": ds.E, "normalize_rows": bool(ds.normalize_rows),
@@ -123,9 +127,12 @@ def run_product(name, ds, *, local_rank=0, rank=0, world=1, runs=5, warm=3, pari
     return out
 
 
-def run_solver(name, n, *, lam=1.0, rtol=1e-6, local_rank=0, rank=0, world=1, parity_rows=128, peaks=None):
+def run_solver(name, n, *, lam=1.0, rtol=1e-6, local_rank=0, rank=0, world=1, parity_rows=128, peaks=None, runs=1, warm=1,
+               outputs=None, key=None):
     """C5: (K + lam I) b = a through B200Solver; the right-hand side is built by the product under test (B200Product) and
-    checked on sampled rows against the oracle, like the residual of the solution."""
+    checked on sampled rows against the oracle, like the residual of the solution.  `warm` untimed solves, then `runs`
+    timed ones (ms = their mean).  With `outputs` (a dict), rank 0 also stores the solution of the last timed query there
+    under `key`."""
     import torch
 
     from kernel_matrix_benchmarks_b200 import datasets
@@ -153,7 +160,7 @@ def run_solver(name, n, *, lam=1.0, rtol=1e-6, local_rank=0, rank=0, world=1, pa
         fits.append(1e3 * (time.perf_counter() - t0))
     algo.prepare_query(target_signal=rhs)
     queries = []
-    for _ in range(2):
+    for _ in range(warm + runs):
         torch.cuda.synchronize(dev)
         t0 = time.perf_counter()
         algo.query()
@@ -168,9 +175,13 @@ def run_solver(name, n, *, lam=1.0, rtol=1e-6, local_rank=0, rank=0, world=1, pa
     algo.get_result()
     e2e_ms = 1e3 * (time.perf_counter() - t0)
     algo.done()
-    fit_first, fit_ms, q_first, q_ms, e2e_ms = _max_over_ranks([fits[0], fits[1], queries[0][1], queries[1][1], e2e_ms], dev, world)
+    timed = [q[1] for q in queries[warm:]]
+    fit_first, fit_ms, q_first, q_ms, e2e_ms = _max_over_ranks([fits[0], fits[1], queries[0][1], sum(timed) / len(timed), e2e_ms],
+                                                               dev, world)
     if rank != 0:
         return None
+    if outputs is not None:
+        outputs[key] = x
     it = max(1, int(extra["cg_iterations"]))
     rows = _rows(n, parity_rows, seed=5)
     from oracle import c_oracle
@@ -207,31 +218,32 @@ def run_solver(name, n, *, lam=1.0, rtol=1e-6, local_rank=0, rank=0, world=1, pa
     }
 
 
-def run_config_block(which, *, local_rank=0, rank=0, world=1, parity_rows=256, peaks=None):
-    """bench.py's "configs" object: name -> result (rank 0), None elsewhere.  Every rank must call it (collectives)."""
+def run_config_block(which, *, local_rank=0, rank=0, world=1, parity_rows=256, peaks=None, outputs=None):
+    """bench.py's "configs" object: name -> result (rank 0), None elsewhere.  Every rank must call it (collectives).
+    With `outputs` (a dict), rank 0 also stores each config's result there under its entry of `which` ("c1", ...)."""
     from kernel_matrix_benchmarks_b200 import datasets
 
     if isinstance(peaks, tuple):
         peaks = peaks[0]
     out = {}
-    common = dict(local_rank=local_rank, rank=rank, world=world, peaks=peaks)
+    common = dict(local_rank=local_rank, rank=rank, world=world, peaks=peaks, outputs=outputs)
     if "c1" in which:
         out["C1"] = run_product("C1: gaussian product N=M=10^4, D=3, E=1", datasets.config_c1(), parity_rows=parity_rows, tol=1e-5,
-                                runs=10, **common)
+                                runs=10, key="c1", **common)
     if "c3" in which:
         out["C3"] = run_product("C3: gaussian product M=60000, N=10000, D=784, E=1 (tcgen05, FP16 hi/lo planes, CTA pairs)",
-                                datasets.config_c3(), parity_rows=min(parity_rows, 128), tol=1e-4, runs=10, **common)
+                                datasets.config_c3(), parity_rows=min(parity_rows, 128), tol=1e-4, runs=10, key="c3", **common)
     if "c4" in which:
         out["C4"] = run_product("C4: absolute-exponential attention N=M=262144, D=64, E=64 (row-normalised; both contractions on tcgen05)",
-                                datasets.config_c4(), parity_rows=min(parity_rows, 128), tol=1e-4, runs=3, warm=2, **common)
+                                datasets.config_c4(), parity_rows=min(parity_rows, 128), tol=1e-4, runs=3, warm=2, key="c4", **common)
     if "c4g" in which:
         out["C4-gaussian"] = run_product("C4 with the gaussian kernel", datasets.config_c4(kernel="gaussian"),
-                                         parity_rows=min(parity_rows, 128), tol=1e-4, runs=3, warm=2, **common)
+                                         parity_rows=min(parity_rows, 128), tol=1e-4, runs=3, warm=2, key="c4g", **common)
     if "c5" in which:
         out["C5"] = run_solver("C5: gaussian solve (K + I) b = a, N=M=10^6, D=3, preconditioned CG", 1_000_000,
-                               parity_rows=min(parity_rows, 128), **common)
+                               parity_rows=min(parity_rows, 128), key="c5", **common)
     if "c5s" in which:
-        out["C5-small"] = run_solver("C5 at N=10^5", 100_000, parity_rows=min(parity_rows, 128), **common)
+        out["C5-small"] = run_solver("C5 at N=10^5", 100_000, parity_rows=min(parity_rows, 128), key="c5s", **common)
     return out if rank == 0 else None
 
 

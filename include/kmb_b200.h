@@ -222,6 +222,35 @@ int kmb_debug_plan_waves(int64_t n_tiles, int64_t n_source_blocks, int grid, siz
  * exponential kernels, whose K b is a dense contraction and runs on the tensor cores as well.  Host logic only. */
 int kmb_resolved_path(int D, int E, int kernel_id, int path);
 
+/* Diagnostics (host logic only, no GPU needed): what kmb_product_f32 would launch for this problem on a device with
+ * `sms` SMs.  out10 = {resolved path, family (KMB_FAMILY_*), difference-form table, index, product-form table, index,
+ * signal columns per pass, passes, row tiles, source blocks}; -1 where a field does not apply.
+ *   direct:  (table, index) name kmb_debug_direct_entry entries (the product form only for the Gaussian kernel off
+ *            KMB_PATH_DIRECT_DIFF; the data pick one of the two forms on the device); row tiles and source blocks
+ *            are those of the difference form.
+ *   tensor families: signal columns per pass is min(E, 4) for kprod_tensor (E = 3 runs on its EP = 4
+ *            instantiation) and the signal block of the P.B kernels.
+ * The CTA-pair decision honours the KMB_TENSOR_PAIR this process has read.  Errors as kmb_product_workspace_bytes. */
+enum {
+    KMB_FAMILY_DIRECT = 0,       /* kprod_direct (FP32, D <= 16) */
+    KMB_FAMILY_SYM = 1,          /* kprod_sym (KMB_PATH_DIRECT_SYM) */
+    KMB_FAMILY_TENSOR = 2,       /* kprod_tensor, one CTA per row tile (TF32 or FP16 planes), E <= 4 per pass */
+    KMB_FAMILY_TENSOR_PAIR = 3,  /* kprod_tensor_pair: CTA pairs, FP16 planes */
+    KMB_FAMILY_PV = 4,           /* kprod_tensor_pv: P.B on the tensor cores, TF32 planes (E > 4, D <= 128) */
+    KMB_FAMILY_PV16 = 5,         /* kprod_tensor_pv16, one CTA per row tile (FP16 planes, Gaussian / exponential) */
+    KMB_FAMILY_PV16_PAIR = 6,    /* kprod_tensor_pv16_pair */
+    KMB_FAMILY_FILL = 7,         /* normalised density: out = 1 */
+    KMB_FAMILY_UNSUPPORTED = 8   /* kmb_product_f32 would return KMB_ERR_UNSUPPORTED */
+};
+int kmb_debug_product_plan(int64_t n_targets, int64_t n_sources, int D, int E, int kernel_id, int flags, int path, int sms,
+                           int64_t* out10);
+
+/* Diagnostics (host logic only): entry `index` of direct-kernel table `table` (0..7: Gaussian difference form n0, n1,
+ * exponential n0, n1, inverse distance n0, n1, Gaussian product form n0, n1; nK = row normalisation off / on).
+ * out11 = {entries in the table, KID, NORM, FORM, DP, EP, R (rows per thread), TILE_ROWS, SB (sources per block),
+ * RECV (float4 per source record), PS (partial floats per row)}; an index outside the table only fills the first. */
+int kmb_debug_direct_entry(int table, int index, int32_t* out11);
+
 /* Diagnostics (host logic only, no GPU needed): where unit `u` of the strip-ordered unit list of the symmetric path
  * sits when n points are worked on by `total_ctas` CTAs over all parts (kprod_sym.cuh).
  * out8 = {total units, strips, strip width in source blocks, strip, row tile, source block, first unit of the

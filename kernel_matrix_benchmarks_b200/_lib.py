@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import ctypes
 import os
-from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int64, c_size_t, c_void_p
+from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_size_t, c_void_p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # KMB_B200_LIB: another build of the same library (instrumented or A/B variants made by csrc/Makefile with EXTRA=...)
@@ -19,6 +19,8 @@ KMB_OK, KMB_ERR_INVALID, KMB_ERR_UNSUPPORTED, KMB_ERR_WORKSPACE, KMB_ERR_CUDA = 
 KERNEL_IDS = {"gaussian": 0, "absolute-exponential": 1, "inverse-distance": 2}
 FLAG_NORMALIZE_ROWS, FLAG_DENSITY, FLAG_PREPARED = 1, 2, 4
 PATH_IDS = {"auto": 0, "direct": 1, "tensor": 5, "tensor_tf32": 2, "tensor_f16": 5, "direct_diff": 3, "direct_sym": 4}
+# KMB_FAMILY_* of kmb_debug_product_plan, by value
+FAMILIES = ("direct", "sym", "tensor", "tensor_pair", "pv", "pv16", "pv16_pair", "fill", "unsupported")
 
 
 class DeviceInfo(ctypes.Structure):
@@ -81,6 +83,8 @@ SIGNATURES = {
     "kmb_debug_plan_waves": (c_int, [c_int64, c_int64, c_int, c_size_t, POINTER(c_int64)]),
     "kmb_debug_sym_unit": (c_int, [c_int64, c_int64, c_int64, POINTER(c_int64)]),
     "kmb_resolved_path": (c_int, [c_int, c_int, c_int, c_int]),
+    "kmb_debug_product_plan": (c_int, [c_int64, c_int64, c_int, c_int, c_int, c_int, c_int, c_int, POINTER(c_int64)]),
+    "kmb_debug_direct_entry": (c_int, [c_int, c_int, POINTER(c_int32)]),
     "kmb_set_profiling": (c_int, [c_int]),
     "kmb_last_main_kernel_ms": (c_int, [POINTER(c_float)]),
     "kmb_cg_scratch_bytes": (c_size_t, []),

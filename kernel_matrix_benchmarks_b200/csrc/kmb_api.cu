@@ -57,26 +57,47 @@ void sym_geometry(long long n_tiles, long long nsb, long long total_ctas, SymGeo
 SymSeg sym_segment_of(const SymGeom& g, long long u);
 int sym_launch(int D, int kernel_id, int form, const SymParams& P, cudaStream_t stream);
 
+// the direct tables in the order above (kmb_debug_direct_entry numbers them so)
+struct DirectTable { const DirectEntry* tab; const int* count; };
+static const DirectTable kDirectTables[8] = {
+    {kDirect_gauss_n0, &kDirect_gauss_n0_count},       {kDirect_gauss_n1, &kDirect_gauss_n1_count},
+    {kDirect_absexp_n0, &kDirect_absexp_n0_count},     {kDirect_absexp_n1, &kDirect_absexp_n1_count},
+    {kDirect_invdist_n0, &kDirect_invdist_n0_count},   {kDirect_invdist_n1, &kDirect_invdist_n1_count},
+    {kDirect_gaussprod_n0, &kDirect_gaussprod_n0_count}, {kDirect_gaussprod_n1, &kDirect_gaussprod_n1_count}};
+
 static const DirectEntry* find_direct(int D, int e_chunk, int kid, bool norm, int form) {
-    const DirectEntry* tab = nullptr;
-    int n = 0;
-#define KMB_PICK(K, F, NAME0, NAME1)              \
-    if (kid == K && form == F) {                  \
-        tab = norm ? NAME1 : NAME0;               \
-        n = norm ? NAME1##_count : NAME0##_count; \
-    }
-    KMB_PICK(KMB_KERNEL_GAUSSIAN, 0, kDirect_gauss_n0, kDirect_gauss_n1)
-    KMB_PICK(KMB_KERNEL_GAUSSIAN, 1, kDirect_gaussprod_n0, kDirect_gaussprod_n1)
-    KMB_PICK(KMB_KERNEL_ABSOLUTE_EXPONENTIAL, 0, kDirect_absexp_n0, kDirect_absexp_n1)
-    KMB_PICK(KMB_KERNEL_INVERSE_DISTANCE, 0, kDirect_invdist_n0, kDirect_invdist_n1)
-#undef KMB_PICK
+    if (form == 1 && kid != KMB_KERNEL_GAUSSIAN) return nullptr;
+    const DirectTable& t = kDirectTables[form == 1 ? 6 + norm : kid * 2 + norm];
     const DirectEntry* best = nullptr;
-    for (int i = 0; i < n; ++i) {
-        const DirectEntry& e = tab[i];
+    for (int i = 0; i < *t.count; ++i) {
+        const DirectEntry& e = t.tab[i];
         if (e.DP < D || e.EP < e_chunk) continue;
         if (!best || e.DP < best->DP || (e.DP == best->DP && e.EP < best->EP)) best = &e;
     }
     return best;
+}
+
+// The direct kernels of a product: signal columns per pass and the entry of each evaluation form (D <= 16).
+struct DirectChoice {
+    const DirectEntry* ent[2];   // [0] difference form (nullptr: no kernel), [1] Gaussian product form (optional)
+    int e_chunk, n_passes;
+};
+static void choose_direct(int D, int E, int kid, bool norm, int path, DirectChoice* c) {
+    // signal columns per pass: every pass re-evaluates the kernel (~8 FMA-pipe slots' worth per pair, MUFU included) and
+    // adds one FMA per column; pick the width that minimises passes x (8 + width)
+    static const int max_chunk = [] {   // tuning knob: KMB_DIRECT_MAX_EP=4 restores one pass per 4 columns
+        const char* e = getenv("KMB_DIRECT_MAX_EP");
+        const int v = e ? atoi(e) : 16;
+        return v < 1 ? 1 : v > 16 ? 16 : v;
+    }();
+    c->e_chunk = 1;
+    for (int w = 1, best = 0; w <= max_chunk; w *= 2) {
+        const int cost = ((E + w - 1) / w) * (8 + w);
+        if (best == 0 || cost < best) { best = cost; c->e_chunk = w; }
+    }
+    c->n_passes = (E + c->e_chunk - 1) / c->e_chunk;
+    c->ent[0] = find_direct(D, c->e_chunk, kid, norm, 0);
+    c->ent[1] = (kid == KMB_KERNEL_GAUSSIAN && path != KMB_PATH_DIRECT_DIFF) ? find_direct(D, c->e_chunk, kid, norm, 1) : nullptr;
 }
 
 static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
@@ -161,22 +182,13 @@ int device_sm_count(int* sms) {
 static int plan_direct(int64_t N, int64_t M, int D, int E, int kid, int flags, int path, DirectPlan* pl) {
     const bool norm = flags & KMB_FLAG_NORMALIZE_ROWS;
     if (D > 16) return set_error(KMB_ERR_UNSUPPORTED, "direct FP32 path supports D <= 16 (got D=%d)", D);
-    // signal columns per pass: every pass re-evaluates the kernel (~8 FMA-pipe slots' worth per pair, MUFU included) and
-    // adds one FMA per column; pick the width that minimises passes x (8 + width)
-    static const int max_chunk = [] {   // tuning knob: KMB_DIRECT_MAX_EP=4 restores one pass per 4 columns
-        const char* e = getenv("KMB_DIRECT_MAX_EP");
-        const int v = e ? atoi(e) : 16;
-        return v < 1 ? 1 : v > 16 ? 16 : v;
-    }();
-    pl->e_chunk = 1;
-    for (int c = 1, best = 0; c <= max_chunk; c *= 2) {
-        const int cost = ((E + c - 1) / c) * (8 + c);
-        if (best == 0 || cost < best) { best = cost; pl->e_chunk = c; }
-    }
-    pl->n_passes = (E + pl->e_chunk - 1) / pl->e_chunk;
-    pl->form[0].ent = find_direct(D, pl->e_chunk, kid, norm, 0);
+    DirectChoice ch;
+    choose_direct(D, E, kid, norm, path, &ch);
+    pl->e_chunk = ch.e_chunk;
+    pl->n_passes = ch.n_passes;
+    pl->form[0].ent = ch.ent[0];
     if (!pl->form[0].ent) return set_error(KMB_ERR_UNSUPPORTED, "no direct kernel for D=%d E=%d kernel=%d", D, E, kid);
-    pl->form[1].ent = (kid == KMB_KERNEL_GAUSSIAN && path != KMB_PATH_DIRECT_DIFF) ? find_direct(D, pl->e_chunk, kid, norm, 1) : nullptr;
+    pl->form[1].ent = ch.ent[1];
     int sms = 0;
     if (int rc = device_sm_count(&sms)) return rc;
     pl->grid_max = sms * 2;
@@ -524,6 +536,65 @@ int kmb_resolved_path(int D, int E, int kernel_id, int path) {
         path > KMB_PATH_TENSOR_3XF16)
         return -1;
     return resolve_path(D, E, kernel_id, path);
+}
+
+int kmb_debug_direct_entry(int table, int index, int32_t* out11) {
+    if (!out11 || table < 0 || table >= 8) return set_error(KMB_ERR_INVALID, "bad arguments");
+    const DirectTable& t = kDirectTables[table];
+    out11[0] = *t.count;
+    for (int i = 1; i < 11; ++i) out11[i] = -1;
+    if (index < 0 || index >= *t.count) return KMB_OK;
+    const DirectEntry& e = t.tab[index];
+    const int32_t v[10] = {e.KID, e.NORM, e.FORM, e.DP, e.EP, e.R, e.TILE_ROWS, e.SB, e.RECV, e.PS};
+    for (int i = 0; i < 10; ++i) out11[1 + i] = v[i];
+    return KMB_OK;
+}
+
+int kmb_debug_product_plan(int64_t N, int64_t M, int D, int E, int kernel_id, int flags, int path, int sms, int64_t* out10) {
+    if (!out10 || sms < 1) return set_error(KMB_ERR_INVALID, "bad arguments");
+    if (int rc = check_product_args(N, M, D, E, kernel_id, flags, path)) return rc;
+    for (int i = 0; i < 10; ++i) out10[i] = -1;
+    const int p = resolve_path(D, E, kernel_id, path);
+    out10[0] = p;
+    if ((flags & KMB_FLAG_NORMALIZE_ROWS) && (flags & KMB_FLAG_DENSITY)) {
+        out10[1] = KMB_FAMILY_FILL;
+        return KMB_OK;
+    }
+    if (p == KMB_PATH_DIRECT_SYM) {
+        out10[1] = KMB_FAMILY_SYM;
+        return KMB_OK;
+    }
+    if (p == KMB_PATH_TENSOR_3XTF32 || p == KMB_PATH_TENSOR_3XF16) {
+        long long t[4];
+        tensor_plan_debug(N, D, E, kernel_id, p == KMB_PATH_TENSOR_3XF16 ? 1 : 0, sms, t);
+        out10[1] = t[0];
+        out10[6] = t[1];
+        out10[7] = t[2];
+        out10[8] = t[3];
+        return KMB_OK;
+    }
+    DirectChoice ch;
+    if (D <= 16) choose_direct(D, E, kernel_id, flags & KMB_FLAG_NORMALIZE_ROWS, p, &ch);
+    if (D > 16 || !ch.ent[0]) {
+        out10[1] = KMB_FAMILY_UNSUPPORTED;
+        return KMB_OK;
+    }
+    out10[1] = KMB_FAMILY_DIRECT;
+    for (int f = 0; f < 2; ++f) {
+        if (!ch.ent[f]) continue;
+        for (int t = 0; t < 8; ++t) {
+            const DirectTable& tab = kDirectTables[t];
+            if (ch.ent[f] >= tab.tab && ch.ent[f] < tab.tab + *tab.count) {
+                out10[2 + 2 * f] = t;
+                out10[3 + 2 * f] = ch.ent[f] - tab.tab;
+            }
+        }
+    }
+    out10[6] = ch.e_chunk;
+    out10[7] = ch.n_passes;
+    out10[8] = (N + ch.ent[0]->TILE_ROWS - 1) / ch.ent[0]->TILE_ROWS;
+    out10[9] = (M + ch.ent[0]->SB - 1) / ch.ent[0]->SB;
+    return KMB_OK;
 }
 
 int kmb_debug_sym_unit(int64_t n, int64_t total_ctas, int64_t u, int64_t* out8) {

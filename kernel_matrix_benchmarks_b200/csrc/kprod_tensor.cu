@@ -971,9 +971,28 @@ int f16_points_prepass(const float* x, const float* y, int64_t N, int64_t M, int
                                   ws + L.off_ul, ws + L.off_vh, ws + L.off_vl, F(L.off_un), F(L.off_vn), stream);
 }
 
+bool tensor_use_pair(long long n_tiles, int sms) {
+    static const bool pair_enabled = [] {   // tuning knob: KMB_TENSOR_PAIR=0 keeps the single-CTA kernels
+        const char* e = getenv("KMB_TENSOR_PAIR");
+        return !(e && e[0] == '0');
+    }();
+    return pair_enabled && n_tiles >= 2 && sms >= 2;
+}
+
 namespace {
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// signal columns per pass of kprod_tensor (E = 3 runs on the EP = 4 instantiation, see launch_ep)
+int tensor_e_chunk(int E) { return E >= 4 ? 4 : E; }
+
+// which kernel family tensor_product hands the product to
+enum { KIND_TENSOR, KIND_PV, KIND_PV16 };
+int tensor_kind(int D, int E, int kid, int elt) {
+    if (elt == tc::ELT_F16 && tensor_pv16_applicable(D, E, kid)) return KIND_PV16;
+    if (tensor_pv_applicable(D, E)) return KIND_PV;
+    return KIND_TENSOR;
+}
 
 struct TensorPlan {
     bool pair;   // CTA-pair kernel (cta_group::2): FP16 planes, at least two row tiles
@@ -991,7 +1010,7 @@ int plan_tensor(int64_t N, int64_t M, int D, int E, int elt, TensorPlan* pl) {
     pl->kblocks = (pl->Dp + tke - 1) / tke;
     pl->ksteps_last = (pl->Dp - (pl->kblocks - 1) * tke) / (f16 ? 16 : 8);
     pl->esz = f16 ? 2 : 4;
-    pl->e_chunk = E >= 4 ? 4 : E;
+    pl->e_chunk = tensor_e_chunk(E);
     pl->n_passes = (E + pl->e_chunk - 1) / pl->e_chunk;
     pl->n_tiles = (N + tc::TM - 1) / tc::TM;
     pl->nsb = (M + tc::TN - 1) / tc::TN;
@@ -999,11 +1018,7 @@ int plan_tensor(int64_t N, int64_t M, int D, int E, int elt, TensorPlan* pl) {
     KMB_CUDA_CHECK(cudaGetDevice(&dev));
     KMB_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     pl->grid = sms;
-    static const bool pair_enabled = [] {   // tuning knob: KMB_TENSOR_PAIR=0 keeps the single-CTA kernel
-        const char* e = getenv("KMB_TENSOR_PAIR");
-        return !(e && e[0] == '0');
-    }();
-    pl->pair = f16 && pair_enabled && pl->n_tiles >= 2 && sms >= 2;
+    pl->pair = f16 && tensor_use_pair(pl->n_tiles, sms);
     if (pl->pair) {
         // the wave plan counts pairs of row tiles and clusters of two CTAs
         pl->grid = sms / 2 * 2;
@@ -1108,10 +1123,30 @@ void tensor_plan_waves_debug(long long n_tiles, long long nsb, int grid, size_t 
     out[6] = wp.partial_slots;
 }
 
+void tensor_plan_debug(int64_t N, int D, int E, int kid, int elt, int sms, long long out[4]) {
+    const long long n_tiles = (N + tc::TM - 1) / tc::TM;
+    const int kind = tensor_kind(D, E, kid, elt);
+    int chunk;
+    if (kind == KIND_TENSOR) {
+        out[0] = (elt == tc::ELT_F16 && tensor_use_pair(n_tiles, sms)) ? KMB_FAMILY_TENSOR_PAIR : KMB_FAMILY_TENSOR;
+        chunk = tensor_e_chunk(E);
+    } else if (kind == KIND_PV) {
+        out[0] = KMB_FAMILY_PV;
+        chunk = tensor_pv_signal_block();
+    } else {
+        out[0] = tensor_use_pair(n_tiles, sms) ? KMB_FAMILY_PV16_PAIR : KMB_FAMILY_PV16;
+        chunk = tensor_pv16_signal_block();
+    }
+    out[1] = chunk;
+    out[2] = (E + chunk - 1) / chunk;
+    out[3] = n_tiles;
+}
+
 int tensor_workspace_bytes(int64_t N, int64_t M, int D, int E, int kid, int flags, int elt, size_t* bytes) {
     (void)flags;
-    if (elt == tc::ELT_F16 && tensor_pv16_applicable(D, E, kid)) return tensor_pv16_workspace_bytes(N, M, D, E, bytes);
-    if (tensor_pv_applicable(D, E)) return tensor_pv_workspace_bytes(N, M, D, E, bytes);
+    const int kind = tensor_kind(D, E, kid, elt);
+    if (kind == KIND_PV16) return tensor_pv16_workspace_bytes(N, M, D, E, bytes);
+    if (kind == KIND_PV) return tensor_pv_workspace_bytes(N, M, D, E, bytes);
     TensorPlan pl{};
     if (int rc = plan_tensor(N, M, D, E, elt, &pl)) return rc;
     *bytes = pl.total;
@@ -1131,9 +1166,10 @@ int tensor_prepare(const float* x, const float* y, int64_t N, int64_t M, int D, 
 int tensor_product(const float* x, const float* y, const float* b, float* out, int64_t N, int64_t M, int D, int E,
                    int kid, int flags, int elt, int64_t row_offset, void* workspace, size_t workspace_bytes,
                    cudaStream_t stream, cudaEvent_t ev0, cudaEvent_t ev1, bool prepared) {
-    if (elt == tc::ELT_F16 && tensor_pv16_applicable(D, E, kid))
+    const int kind = tensor_kind(D, E, kid, elt);
+    if (kind == KIND_PV16)
         return tensor_pv16_product(x, y, b, out, N, M, D, E, kid, flags, workspace, workspace_bytes, stream, ev0, ev1, prepared);
-    if (tensor_pv_applicable(D, E))
+    if (kind == KIND_PV)
         return tensor_pv_product(x, y, b, out, N, M, D, E, kid, flags, row_offset, workspace, workspace_bytes, stream, ev0, ev1);
     TensorPlan pl{};
     if (int rc = plan_tensor(N, M, D, E, elt, &pl)) return rc;

@@ -26,4 +26,8 @@ int tensor_prepare(const float* x, const float* y, int64_t N, int64_t M, int D, 
 // out = {R, C, W, R_last, C_last, slots_per_wave, partial_slots}.  Host logic only (tests/test_abi_cpu.py).
 void tensor_plan_waves_debug(long long n_tiles, long long nsb, int grid, size_t row_tile_bytes, long long out[7]);
 
+// What tensor_product launches for this shape on `sms` SMs: out = {KMB_FAMILY_*, signal columns per pass, passes, row
+// tiles}.  Host logic only, the same decisions as tensor_product (kmb_debug_product_plan).
+void tensor_plan_debug(int64_t N, int D, int E, int kid, int elt, int sms, long long out[4]);
+
 }  // namespace kmb

@@ -585,6 +585,7 @@ int launch_pv(const CUtensorMap* m, const pv::Params& P, int grid, int smem, cud
 }  // namespace
 
 bool tensor_pv_applicable(int D, int E) { return E > 4 && D <= 128; }
+int tensor_pv_signal_block() { return pv::MAX_EB; }
 
 int tensor_pv_workspace_bytes(int64_t N, int64_t M, int D, int E, size_t* bytes) {
     PvPlan pl{};

@@ -936,11 +936,7 @@ int plan_pv16(int64_t N, int64_t M, int D, int E, Pv16Plan* pl) {
     KMB_CUDA_CHECK(cudaGetDevice(&dev));
     KMB_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     KMB_CUDA_CHECK(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-    static const bool pair_enabled = [] {   // tuning knob: KMB_TENSOR_PAIR=0 keeps the single-CTA kernel
-        const char* e = getenv("KMB_TENSOR_PAIR");
-        return !(e && e[0] == '0');
-    }();
-    pl->pair = pair_enabled && pl->n_tiles >= 2 && sms >= 2;
+    pl->pair = tensor_use_pair(pl->n_tiles, sms);
     pl->grid = pl->pair ? sms / 2 * 2 : sms;
     const int slot = pl->pair ? pv16::SLOT_BYTES / 2 : pv16::SLOT_BYTES;
     const int fixed = 1024 + (pl->kblocks * 2 + (pv16::kExtraK ? 1 : 0)) * pv16::A_TILE_BYTES + pv16::EPI_WARPS * 2 * pv16::CPT * 4 + 2 * pv16::NG * tc::TM * 4 + 512;
@@ -995,6 +991,7 @@ int launch_pv16(const CUtensorMap* m, const pv16::Params& P, int grid, int smem,
 bool tensor_pv16_applicable(int D, int E, int kid) {
     return E > 4 && D <= 128 && (kid == KMB_KERNEL_GAUSSIAN || kid == KMB_KERNEL_ABSOLUTE_EXPONENTIAL);
 }
+int tensor_pv16_signal_block() { return pv16::MAX_EB; }
 
 int tensor_pv16_workspace_bytes(int64_t N, int64_t M, int D, int E, size_t* bytes) {
     Pv16Plan pl{};

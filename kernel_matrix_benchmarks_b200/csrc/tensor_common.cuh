@@ -272,8 +272,14 @@ void plan_waves(long long n_tiles, long long nsb, int grid, size_t row_tile_byte
 
 }  // namespace tc
 
+// CTA pairs (cta_group::2) for an FP16-plane problem of n_tiles row tiles on `sms` SMs: at least two row tiles, unless
+// KMB_TENSOR_PAIR=0 (read once per process).  Host logic only (kprod_tensor.cu; kprod_tensor and kprod_tensor_pv16).
+bool tensor_use_pair(long long n_tiles, int sms);
+
 // E > 4 with D <= 128: second GEMM on the tensor cores (kprod_tensor_pv.cu)
 bool tensor_pv_applicable(int D, int E);
+int tensor_pv_signal_block();     // signal columns per pass of kprod_tensor_pv
+int tensor_pv16_signal_block();   // ... of kprod_tensor_pv16
 int tensor_pv_workspace_bytes(int64_t N, int64_t M, int D, int E, size_t* bytes);
 int tensor_pv_product(const float* x, const float* y, const float* b, float* out, int64_t N, int64_t M, int D, int E,
                       int kid, int flags, int64_t row_offset, void* workspace, size_t workspace_bytes,

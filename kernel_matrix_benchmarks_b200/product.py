@@ -74,6 +74,38 @@ def resolved_path(D, E, kernel="gaussian", path="auto"):
     return names[pid]
 
 
+PLAN_FIELDS = ("path", "family", "diff_table", "diff_index", "prod_table", "prod_index", "chunk", "passes", "row_tiles",
+               "source_blocks")
+
+
+def dispatch_plan(N, M, D, E, *, kernel="gaussian", normalize_rows=False, density_estimation=False, path="auto", sms=148):
+    """What kernel_product would launch for this problem on a device with ``sms`` SMs (kmb_debug_product_plan, host logic
+    only, no GPU needed): a dict of PLAN_FIELDS, ``path`` and ``family`` as names, -1 where a field does not apply."""
+    flags = (_lib.FLAG_NORMALIZE_ROWS if normalize_rows else 0) | (_lib.FLAG_DENSITY if density_estimation else 0)
+    out = (ctypes.c_int64 * len(PLAN_FIELDS))()
+    _lib.check(_lib.load().kmb_debug_product_plan(int(N), int(M), int(D), int(E), _lib.KERNEL_IDS[kernel], flags,
+                                                  _lib.PATH_IDS[path], int(sms), out))
+    plan = dict(zip(PLAN_FIELDS, (int(v) for v in out)))
+    plan["path"] = {v: k for k, v in _lib.PATH_IDS.items() if k != "tensor"}[plan["path"]]
+    plan["family"] = _lib.FAMILIES[plan["family"]]
+    return plan
+
+
+DIRECT_ENTRY_FIELDS = ("KID", "NORM", "FORM", "DP", "EP", "R", "TILE_ROWS", "SB", "RECV", "PS")
+
+
+def direct_entries(table):
+    """Every entry of direct-kernel table ``table`` (0..7, kmb_debug_direct_entry) as dicts of DIRECT_ENTRY_FIELDS."""
+    lib = _lib.load()
+    out = (ctypes.c_int32 * 11)()
+    _lib.check(lib.kmb_debug_direct_entry(int(table), -1, out))
+    entries = []
+    for i in range(out[0]):
+        _lib.check(lib.kmb_debug_direct_entry(int(table), i, out))
+        entries.append(dict(zip(DIRECT_ENTRY_FIELDS, out[1:])))
+    return entries
+
+
 def prepare_points(x, y, *, kernel="gaussian", path="auto", workspace=None, min_bytes=0):
     """The points-only part of a product (kmb_product_prepare_f32): for the FP16 tensor path the prepass (centre, scale,
     operand planes, squared norms) is written to the head of ``workspace``.  Returns the buffer it was written to: a

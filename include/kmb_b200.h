@@ -245,6 +245,19 @@ enum {
 int kmb_debug_product_plan(int64_t n_targets, int64_t n_sources, int D, int E, int kernel_id, int flags, int path, int sms,
                            int64_t* out10);
 
+/* Diagnostics (host logic only, no GPU needed): how the P.B kernel (KMB_FAMILY_PV, _PV16, _PV16_PAIR) would run this
+ * problem on a device with `sms` SMs and `smem_optin` bytes of opt-in shared memory per block -- the launchers' own
+ * plan.  out19 = {family, CTA pairs (0 / 1), grid (CTAs), ring stages, K blocks, K steps of the last K block, signal
+ * passes, columns of the first pass, the same padded to 32, columns of the last pass, the same padded to 32, row tiles,
+ * source blocks, R, C, W, R_last, C_last (the wave plan, see kmb_debug_plan_waves; with CTA pairs R and R_last count
+ * pairs of row tiles), source blocks the P.B accumulators collect between two flushes}.  Another family only fills
+ * out19[0] (the others are -1).  The CTA-pair decision and the flush interval honour the KMB_TENSOR_PAIR and
+ * KMB_PV16_FLUSH_BLOCKS this process has read.  Errors as kmb_product_workspace_bytes; KMB_ERR_UNSUPPORTED when the
+ * kernel's ring does not fit `smem_optin`. */
+#define KMB_PV_PLAN_FIELDS 19
+int kmb_debug_pv_plan(int64_t n_targets, int64_t n_sources, int D, int E, int kernel_id, int flags, int path, int sms,
+                      int smem_optin, int64_t* out19);
+
 /* Diagnostics (host logic only): entry `index` of direct-kernel table `table` (0..7: Gaussian difference form n0, n1,
  * exponential n0, n1, inverse distance n0, n1, Gaussian product form n0, n1; nK = row normalisation off / on).
  * out11 = {entries in the table, KID, NORM, FORM, DP, EP, R (rows per thread), TILE_ROWS, SB (sources per block),

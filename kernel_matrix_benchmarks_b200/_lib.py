@@ -85,6 +85,7 @@ SIGNATURES = {
     "kmb_resolved_path": (c_int, [c_int, c_int, c_int, c_int]),
     "kmb_debug_product_plan": (c_int, [c_int64, c_int64, c_int, c_int, c_int, c_int, c_int, c_int, POINTER(c_int64)]),
     "kmb_debug_direct_entry": (c_int, [c_int, c_int, POINTER(c_int32)]),
+    "kmb_debug_pv_plan": (c_int, [c_int64, c_int64, c_int, c_int, c_int, c_int, c_int, c_int, c_int, POINTER(c_int64)]),
     "kmb_set_profiling": (c_int, [c_int]),
     "kmb_last_main_kernel_ms": (c_int, [POINTER(c_float)]),
     "kmb_cg_scratch_bytes": (c_size_t, []),

@@ -597,6 +597,22 @@ int kmb_debug_product_plan(int64_t N, int64_t M, int D, int E, int kernel_id, in
     return KMB_OK;
 }
 
+int kmb_debug_pv_plan(int64_t N, int64_t M, int D, int E, int kernel_id, int flags, int path, int sms, int smem_optin,
+                      int64_t* out19) {
+    if (!out19 || sms < 1 || smem_optin < 1) return set_error(KMB_ERR_INVALID, "bad arguments");
+    if (int rc = check_product_args(N, M, D, E, kernel_id, flags, path)) return rc;
+    int64_t plan[10];
+    if (int rc = kmb_debug_product_plan(N, M, D, E, kernel_id, flags, path, sms, plan)) return rc;
+    long long o[KMB_PV_PLAN_FIELDS];
+    for (int i = 0; i < KMB_PV_PLAN_FIELDS; ++i) o[i] = -1;
+    o[0] = plan[1];
+    if (plan[1] == KMB_FAMILY_PV || plan[1] == KMB_FAMILY_PV16 || plan[1] == KMB_FAMILY_PV16_PAIR)
+        if (int rc = tensor_pv_plan_query(N, M, D, E, kernel_id, plan[0] == KMB_PATH_TENSOR_3XF16 ? 1 : 0, sms, smem_optin, o))
+            return rc;
+    for (int i = 0; i < KMB_PV_PLAN_FIELDS; ++i) out19[i] = o[i];
+    return KMB_OK;
+}
+
 int kmb_debug_sym_unit(int64_t n, int64_t total_ctas, int64_t u, int64_t* out8) {
     if (!out8 || n < 1 || total_ctas < 1) return set_error(KMB_ERR_INVALID, "bad arguments");
     SymGeom g;

@@ -1142,6 +1142,18 @@ void tensor_plan_debug(int64_t N, int D, int E, int kid, int elt, int sms, long 
     out[3] = n_tiles;
 }
 
+int tensor_pv_plan_query(int64_t N, int64_t M, int D, int E, int kid, int elt, int sms, int smem_optin, long long* out) {
+    static_assert(PVQ_FIELDS == KMB_PV_PLAN_FIELDS, "kmb_debug_pv_plan fields");
+    for (int i = 0; i < PVQ_FIELDS; ++i) out[i] = -1;
+    long long t[4];
+    tensor_plan_debug(N, D, E, kid, elt, sms, t);
+    out[PVQ_FAMILY] = t[0];
+    const int kind = tensor_kind(D, E, kid, elt);
+    if (kind == KIND_PV16) return tensor_pv16_plan_debug(N, M, D, E, sms, smem_optin, out);
+    if (kind == KIND_PV) return tensor_pv_plan_debug(N, M, D, E, sms, smem_optin, out);
+    return KMB_OK;   // an E <= 4 kernel: only the family
+}
+
 int tensor_workspace_bytes(int64_t N, int64_t M, int D, int E, int kid, int flags, int elt, size_t* bytes) {
     (void)flags;
     const int kind = tensor_kind(D, E, kid, elt);

@@ -30,4 +30,9 @@ void tensor_plan_waves_debug(long long n_tiles, long long nsb, int grid, size_t 
 // tiles}.  Host logic only, the same decisions as tensor_product (kmb_debug_product_plan).
 void tensor_plan_debug(int64_t N, int D, int E, int kid, int elt, int sms, long long out[4]);
 
+// What the P.B kernel (kprod_tensor_pv / kprod_tensor_pv16) launches for this shape on a device of `sms` SMs with
+// `smem_optin` bytes of opt-in shared memory per block: out = the KMB_PV_PLAN_FIELDS of kmb_debug_pv_plan.  Host logic
+// only, the launchers' own plan functions; for an E <= 4 kernel only the family is filled.
+int tensor_pv_plan_query(int64_t N, int64_t M, int D, int E, int kid, int elt, int sms, int smem_optin, long long* out);
+
 }  // namespace kmb

@@ -537,17 +537,15 @@ struct PvPlan {
     size_t off_center, off_cpart, off_uh, off_ul, off_vh, off_vl, off_un, off_vn, off_sh, off_sl, off_partial, off_olong, off_counter, total;
 };
 
-int plan_pv(int64_t N, int64_t M, int D, int E, PvPlan* pl) {
+// host arithmetic only, for a device of `sms` SMs and `smem_max` bytes of opt-in shared memory per block: the launcher
+// (plan_pv) and the plan query (tensor_pv_plan_debug) share it
+int plan_pv_host(int64_t N, int64_t M, int D, int E, int sms, int smem_max, PvPlan* pl) {
     pl->Dp = (D + tc::TK - 1) / tc::TK * tc::TK;
     pl->kblocks = pl->Dp / tc::TK;
     pl->Ep = (E + pv::MAX_EB - 1) / pv::MAX_EB * pv::MAX_EB;
     pl->Mp = (M + pv::TN - 1) / pv::TN * pv::TN;
     pl->n_tiles = (N + tc::TM - 1) / tc::TM;
     pl->nsb = (M + pv::TN - 1) / pv::TN;
-    int dev = 0, sms = 0, smem_max = 0;
-    KMB_CUDA_CHECK(cudaGetDevice(&dev));
-    KMB_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    KMB_CUDA_CHECK(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
     pl->grid_max = sms;
     const int fixed = 1024 + pl->kblocks * 2 * pv::A_TILE_BYTES + 2 * pv::TN * 4 + 3 * pv::NG * tc::TM * 4 + 512;
     pl->stages = std::min(12, (smem_max - fixed) / pv::SLOT_BYTES);
@@ -573,6 +571,14 @@ int plan_pv(int64_t N, int64_t M, int D, int E, PvPlan* pl) {
     return KMB_OK;
 }
 
+int plan_pv(int64_t N, int64_t M, int D, int E, PvPlan* pl) {
+    int dev = 0, sms = 0, smem_max = 0;
+    KMB_CUDA_CHECK(cudaGetDevice(&dev));
+    KMB_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    KMB_CUDA_CHECK(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    return plan_pv_host(N, M, D, E, sms, smem_max, pl);
+}
+
 template <int KID, bool NORM>
 int launch_pv(const CUtensorMap* m, const pv::Params& P, int grid, int smem, cudaStream_t stream) {
     auto fn = pv::kprod_tensor_pv_kernel<KID, NORM>;
@@ -586,6 +592,19 @@ int launch_pv(const CUtensorMap* m, const pv::Params& P, int grid, int smem, cud
 
 bool tensor_pv_applicable(int D, int E) { return E > 4 && D <= 128; }
 int tensor_pv_signal_block() { return pv::MAX_EB; }
+
+int tensor_pv_plan_debug(int64_t N, int64_t M, int D, int E, int sms, int smem_optin, long long out[PVQ_FIELDS]) {
+    PvPlan pl{};
+    if (int rc = plan_pv_host(N, M, D, E, sms, smem_optin, &pl)) return rc;
+    pv_plan_fill(E, pv::MAX_EB, pl.n_tiles, pl.nsb, pl.waves, out);
+    out[PVQ_PAIR] = 0;
+    out[PVQ_GRID] = pl.grid_max;
+    out[PVQ_STAGES] = pl.stages;
+    out[PVQ_KBLOCKS] = pl.kblocks;
+    out[PVQ_KSTEPS_LAST] = tc::TK / tc::UMMA_K;   // D is zero-padded to whole K blocks
+    out[PVQ_FLUSH_BLOCKS] = pv::kFlushBlocks;
+    return KMB_OK;
+}
 
 int tensor_pv_workspace_bytes(int64_t N, int64_t M, int D, int E, size_t* bytes) {
     PvPlan pl{};

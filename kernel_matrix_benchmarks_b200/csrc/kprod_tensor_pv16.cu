@@ -845,7 +845,10 @@ static __global__ void __launch_bounds__(256) signal_absmax_kernel(const float* 
         pmax[static_cast<size_t>(blockIdx.x) * E + col] = h;
     }
 }
-// bscale[e] = 2^q with 2^q max_j |b[j][e]| in [2^13, 2^14); binv[e] = 2^-q
+// bscale[e] = 2^q with 2^q max_j |b[j][e]| in [2^13, 2^14); binv[e] = 2^-q.  q is clamped to [-114, 126], the range in
+// which both 2^q and 2^-q are finite FP32 normals: every column whose largest |b| is an FP32 normal number then lands in
+// [2^13, 2^14) (max |b| >= 2^-113) or in [1, 2^14) (the smallest normals), never above FP16's 65504 and never where the
+// lo plane would lose bits to FP16 subnormals (tests/test_split_accuracy_cpu.py)
 static __global__ void signal_scale_kernel(const float* __restrict__ pmax, int blocks, int E, int Ep, float* __restrict__ bscale,
                                            float* __restrict__ binv) {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
@@ -855,7 +858,7 @@ static __global__ void signal_scale_kernel(const float* __restrict__ pmax, int b
         for (int b = 0; b < blocks; ++b) m = fmaxf(m, pmax[static_cast<size_t>(b) * E + e]);
     int q = 0;
     if (m > 0.f && m < INFINITY) q = 13 - ilogbf(m);
-    q = max(-100, min(100, q));
+    q = max(-114, min(126, q));
     bscale[e] = exp2f(static_cast<float>(q));
     binv[e] = exp2f(static_cast<float>(-q));
 }
@@ -924,7 +927,9 @@ struct Pv16Plan {
         off_binv, off_partial, off_olong, off_counter, off_ue, off_ve, total;
 };
 
-int plan_pv16(int64_t N, int64_t M, int D, int E, Pv16Plan* pl) {
+// host arithmetic only, for a device of `sms` SMs and `smem_max` bytes of opt-in shared memory per block: the launcher
+// (plan_pv16) and the plan query (tensor_pv16_plan_debug) share it
+int plan_pv16_host(int64_t N, int64_t M, int D, int E, int sms, int smem_max, Pv16Plan* pl) {
     pl->Dp = (D + 15) / 16 * 16;
     pl->kblocks = (pl->Dp + 63) / 64;
     pl->ksteps_last = (pl->Dp - (pl->kblocks - 1) * 64) / 16;
@@ -932,10 +937,6 @@ int plan_pv16(int64_t N, int64_t M, int D, int E, Pv16Plan* pl) {
     pl->Mp = (M + pv16::TNS - 1) / pv16::TNS * pv16::TNS;
     pl->n_tiles = (N + tc::TM - 1) / tc::TM;
     pl->nsb = (M + pv16::TNS - 1) / pv16::TNS;
-    int dev = 0, sms = 0, smem_max = 0;
-    KMB_CUDA_CHECK(cudaGetDevice(&dev));
-    KMB_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    KMB_CUDA_CHECK(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
     pl->pair = tensor_use_pair(pl->n_tiles, sms);
     pl->grid = pl->pair ? sms / 2 * 2 : sms;
     const int slot = pl->pair ? pv16::SLOT_BYTES / 2 : pv16::SLOT_BYTES;
@@ -971,6 +972,14 @@ int plan_pv16(int64_t N, int64_t M, int D, int E, Pv16Plan* pl) {
     return KMB_OK;
 }
 
+int plan_pv16(int64_t N, int64_t M, int D, int E, Pv16Plan* pl) {
+    int dev = 0, sms = 0, smem_max = 0;
+    KMB_CUDA_CHECK(cudaGetDevice(&dev));
+    KMB_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    KMB_CUDA_CHECK(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    return plan_pv16_host(N, M, D, E, sms, smem_max, pl);
+}
+
 template <int KID, bool NORM>
 int launch_pv16(const CUtensorMap* m, const pv16::Params& P, int grid, int smem, bool pair, cudaStream_t stream) {
     if (pair) {
@@ -992,6 +1001,28 @@ bool tensor_pv16_applicable(int D, int E, int kid) {
     return E > 4 && D <= 128 && (kid == KMB_KERNEL_GAUSSIAN || kid == KMB_KERNEL_ABSOLUTE_EXPONENTIAL);
 }
 int tensor_pv16_signal_block() { return pv16::MAX_EB; }
+
+int tensor_pv16_flush_blocks() {
+    static const int flush_blocks = [] {   // tuning knob
+        const char* e = getenv("KMB_PV16_FLUSH_BLOCKS");
+        const int v = e ? atoi(e) : pv16::kFlushBlocks;
+        return v < 1 ? 1 : v;
+    }();
+    return flush_blocks;
+}
+
+int tensor_pv16_plan_debug(int64_t N, int64_t M, int D, int E, int sms, int smem_optin, long long out[PVQ_FIELDS]) {
+    Pv16Plan pl{};
+    if (int rc = plan_pv16_host(N, M, D, E, sms, smem_optin, &pl)) return rc;
+    pv_plan_fill(E, pv16::MAX_EB, pl.n_tiles, pl.nsb, pl.waves, out);   // pairs: R, C, R_last count pairs of row tiles
+    out[PVQ_PAIR] = pl.pair ? 1 : 0;
+    out[PVQ_GRID] = pl.grid;
+    out[PVQ_STAGES] = pl.stages;
+    out[PVQ_KBLOCKS] = pl.kblocks;
+    out[PVQ_KSTEPS_LAST] = pl.ksteps_last;
+    out[PVQ_FLUSH_BLOCKS] = tensor_pv16_flush_blocks();
+    return KMB_OK;
+}
 
 int tensor_pv16_workspace_bytes(int64_t N, int64_t M, int D, int E, size_t* bytes) {
     Pv16Plan pl{};
@@ -1083,12 +1114,7 @@ int tensor_pv16_product(const float* x, const float* y, const float* b, float* o
         P.ksteps_last = pl.ksteps_last;
         P.stages = pl.stages;
         P.ep_rows = pl.Ep;
-        static const int flush_blocks = [] {   // tuning knob
-            const char* e = getenv("KMB_PV16_FLUSH_BLOCKS");
-            const int v = e ? atoi(e) : pv16::kFlushBlocks;
-            return v < 1 ? 1 : v;
-        }();
-        P.flush_blocks = flush_blocks;
+        P.flush_blocks = tensor_pv16_flush_blocks();
         P.R = pl.waves.R;
         P.C = pl.waves.C;
         P.W = pl.waves.W;

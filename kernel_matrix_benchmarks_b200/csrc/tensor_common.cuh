@@ -276,8 +276,35 @@ void plan_waves(long long n_tiles, long long nsb, int grid, size_t row_tile_byte
 // KMB_TENSOR_PAIR=0 (read once per process).  Host logic only (kprod_tensor.cu; kprod_tensor and kprod_tensor_pv16).
 bool tensor_use_pair(long long n_tiles, int sms);
 
+// What a P.B kernel launches (kmb_debug_pv_plan, include/kmb_b200.h): the fields of its `out`, in this order.
+enum {
+    PVQ_FAMILY, PVQ_PAIR, PVQ_GRID, PVQ_STAGES, PVQ_KBLOCKS, PVQ_KSTEPS_LAST, PVQ_PASSES, PVQ_EB_FIRST, PVQ_EBP_FIRST,
+    PVQ_EB_LAST, PVQ_EBP_LAST, PVQ_ROW_TILES, PVQ_SOURCE_BLOCKS, PVQ_R, PVQ_C, PVQ_W, PVQ_R_LAST, PVQ_C_LAST,
+    PVQ_FLUSH_BLOCKS, PVQ_FIELDS
+};
+// the fields both P.B kernels derive alike: signal passes of max_eb columns (each padded to 32), tiling, wave plan
+inline void pv_plan_fill(int E, int max_eb, long long n_tiles, long long nsb, const tc::WavePlan& w, long long* out) {
+    const int passes = (E + max_eb - 1) / max_eb;
+    const int eb_first = E < max_eb ? E : max_eb, eb_last = E - (passes - 1) * max_eb;
+    out[PVQ_PASSES] = passes;
+    out[PVQ_EB_FIRST] = eb_first;
+    out[PVQ_EBP_FIRST] = (eb_first + 31) / 32 * 32;
+    out[PVQ_EB_LAST] = eb_last;
+    out[PVQ_EBP_LAST] = (eb_last + 31) / 32 * 32;
+    out[PVQ_ROW_TILES] = n_tiles;
+    out[PVQ_SOURCE_BLOCKS] = nsb;
+    out[PVQ_R] = w.R;
+    out[PVQ_C] = w.C;
+    out[PVQ_W] = w.W;
+    out[PVQ_R_LAST] = w.R_last;
+    out[PVQ_C_LAST] = w.C_last;
+}
+
 // E > 4 with D <= 128: second GEMM on the tensor cores (kprod_tensor_pv.cu)
 bool tensor_pv_applicable(int D, int E);
+// The plan of kprod_tensor_pv on a device of `sms` SMs with `smem_optin` bytes of opt-in shared memory per block (host
+// logic only, the launcher's own): fills every PVQ_* field but PVQ_FAMILY.  Errors as the launcher's plan.
+int tensor_pv_plan_debug(int64_t N, int64_t M, int D, int E, int sms, int smem_optin, long long out[PVQ_FIELDS]);
 int tensor_pv_signal_block();     // signal columns per pass of kprod_tensor_pv
 int tensor_pv16_signal_block();   // ... of kprod_tensor_pv16
 int tensor_pv_workspace_bytes(int64_t N, int64_t M, int D, int E, size_t* bytes);
@@ -288,6 +315,10 @@ int tensor_pv_product(const float* x, const float* y, const float* b, float* out
 
 // the same with FP16 hi/lo operand planes (kprod_tensor_pv16.cu): Gaussian and exponential kernels
 bool tensor_pv16_applicable(int D, int E, int kid);
+// source blocks the P.B accumulators collect between two flushes: KMB_PV16_FLUSH_BLOCKS (read once per process), else 128
+int tensor_pv16_flush_blocks();
+// as tensor_pv_plan_debug, for kprod_tensor_pv16 (PVQ_PAIR: the CTA-pair kernel)
+int tensor_pv16_plan_debug(int64_t N, int64_t M, int D, int E, int sms, int smem_optin, long long out[PVQ_FIELDS]);
 int tensor_pv16_workspace_bytes(int64_t N, int64_t M, int D, int E, size_t* bytes);
 int tensor_pv16_product(const float* x, const float* y, const float* b, float* out, int64_t N, int64_t M, int D, int E, int kid,
                         int flags, void* workspace, size_t workspace_bytes, cudaStream_t stream, cudaEvent_t ev0,

@@ -91,6 +91,26 @@ def dispatch_plan(N, M, D, E, *, kernel="gaussian", normalize_rows=False, densit
     return plan
 
 
+PV_PLAN_FIELDS = ("family", "pair", "grid", "stages", "kblocks", "ksteps_last", "passes", "eb_first", "ebp_first", "eb_last",
+                  "ebp_last", "row_tiles", "source_blocks", "R", "C", "W", "R_last", "C_last", "flush_blocks")
+
+
+def pv_plan(N, M, D, E, *, kernel="gaussian", normalize_rows=False, path="auto", sms, smem_optin):
+    """How the P.B kernel (families pv, pv16, pv16_pair) would run this problem on a device with ``sms`` SMs and
+    ``smem_optin`` bytes of opt-in shared memory per block (kmb_debug_pv_plan, the launchers' own plan; host logic only,
+    no GPU needed): a dict of PV_PLAN_FIELDS, ``family`` as a name, ``pair`` as a bool.  With CTA pairs R and R_last
+    count pairs of row tiles.  Another family only fills ``family`` (the rest are -1)."""
+    flags = _lib.FLAG_NORMALIZE_ROWS if normalize_rows else 0
+    out = (ctypes.c_int64 * len(PV_PLAN_FIELDS))()
+    _lib.check(_lib.load().kmb_debug_pv_plan(int(N), int(M), int(D), int(E), _lib.KERNEL_IDS[kernel], flags,
+                                             _lib.PATH_IDS[path], int(sms), int(smem_optin), out))
+    plan = dict(zip(PV_PLAN_FIELDS, (int(v) for v in out)))
+    plan["family"] = _lib.FAMILIES[plan["family"]]
+    if plan["pair"] >= 0:
+        plan["pair"] = bool(plan["pair"])
+    return plan
+
+
 DIRECT_ENTRY_FIELDS = ("KID", "NORM", "FORM", "DP", "EP", "R", "TILE_ROWS", "SB", "RECV", "PS")
 
 

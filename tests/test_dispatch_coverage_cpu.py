@@ -15,10 +15,15 @@ from conftest import REPO
 
 
 def _plan(case):
+    """dispatch_plan of the case; P.B cases also get their pv_plan as plan["pv"]."""
     from kernel_matrix_benchmarks_b200 import product
 
-    return product.dispatch_plan(case.N, case.M, case.D, case.E, kernel=case.kernel, normalize_rows=case.norm,
+    plan = product.dispatch_plan(case.N, case.M, case.D, case.E, kernel=case.kernel, normalize_rows=case.norm,
                                  density_estimation=case.density, path=case.path, sms=dc.SMS)
+    if case.group:
+        plan["pv"] = product.pv_plan(case.N, case.M, case.D, case.E, kernel=case.kernel, normalize_rows=case.norm,
+                                     path=case.path, sms=dc.SMS, smem_optin=dc.SMEM_OPTIN)
+    return plan
 
 
 def _env_plans(cases):
@@ -195,6 +200,104 @@ def test_inverse_distance_row_offsets_are_covered(plans):
     want = {(f, k) for f in ("direct", "tensor", "tensor_pair", "pv") for k in ("offset", "wrap")}
     want |= {("direct", "copy"), ("tensor_pair", "copy"), ("pv", "copy")}
     assert not sorted(want - seen), f"uncovered: {sorted(want - seen)}"
+
+
+def test_every_pb_case_reaches_its_launch_shape(plans):
+    """Each P.B case runs in the group it names (pv, pv16 on one row tile, pv16_pair, pv16 with KMB_TENSOR_PAIR=0) and
+    reaches every launch shape it is sized for (dc.pb_edges)."""
+    bad = []
+    for c in dc.all_cases():
+        if not c.group:
+            continue
+        pv = plans[c.name]["pv"]
+        group = dc.pb_group(pv, c.env)
+        missed = set(c.edges) - dc.pb_edges(pv, c.env)
+        if group != c.group or missed:
+            bad.append(f"{c.name}: group {group}, missed {sorted(missed)} ({pv})")
+    assert not bad, "\n".join(bad)
+
+
+def _pb_shapes(group):
+    """Ring stages and (K blocks, K steps of the last one) the group's kernel takes over D = 1 .. 128."""
+    from kernel_matrix_benchmarks_b200 import product
+
+    family, path, kernels, env, blk, F = dc.PB_GROUPS[group]
+    N = 401 if group == "pv16_pair" else 100   # pv16_pair_off: the single-CTA kernel's shapes (the pair knob is not set here)
+    out = set()
+    for D in range(1, 129):
+        p = product.pv_plan(N, 700, D, 40, kernel=kernels[0], path=path, sms=dc.SMS, smem_optin=dc.SMEM_OPTIN)
+        out |= {f"stages{p['stages']}", f"k{p['kblocks']}x{p['ksteps_last']}"}
+    return out
+
+
+def test_pb_launch_shapes_are_covered(plans):
+    """Every (group, kernel, normalisation) of the P.B kernels has a parity case for each launch shape that selects different
+    code: one pass padded to 32 and to 64 columns; two passes with a last pass of 1 and of 32 columns and three with a last
+    of 1; every ring-stage count and (K blocks, K steps) D can select; row tiles split over CTAs; and, unless the problem
+    has one row tile, two waves and CTA ranges of F - 1, F, F + 1 and 2F + 1 source blocks (F = the flush interval).  CTA
+    pairs: an odd row-tile count (ghost tile).  FP16 planes: KMB_PV16_FLUSH_BLOCKS = 1 and 3 (3 only with
+    KMB_TENSOR_PAIR=0).  Also: far rows under normalisation, signal columns of very different magnitudes (pv, pv16,
+    pv16_pair) and, for pairs, columns 0-31 and 32-63 2^100 apart."""
+    seen = set()
+    for c in dc.all_cases():
+        if c.group:
+            key = (c.group, c.kernel, c.norm)
+            seen |= {key + (e,) for e in dc.pb_edges(plans[c.name]["pv"], c.env)}
+            if c.far_rows:
+                seen.add(key + ("far",))
+            if c.data in ("magnitude", "halves"):
+                seen.add(key + (c.data,))
+    want = set()
+    for group, (family, path, kernels, env, blk, F) in dc.PB_GROUPS.items():
+        edges = {"ebp32", "ebp64", "2pass-narrow", "2pass-last32", "3pass-narrow", "split"} | _pb_shapes(group)
+        if group != "pv16":
+            edges |= {"waves", "flush-1", "flush", "flush+1", "2flush+1"}
+        if group == "pv16_pair":
+            edges |= {"ghost", "halves"}
+        if family != "pv":
+            edges |= {"knob3"} if group == "pv16_pair_off" else {"knob1", "knob3"}
+        if group != "pv16_pair_off":
+            edges.add("magnitude")
+        for kernel in kernels:
+            for norm in (False, True):
+                want |= {(group, kernel, norm, e) for e in edges | ({"far"} if norm else set())}
+    missing = sorted(want - seen, key=str)
+    assert not missing, "P.B launch shapes without a parity case:\n" + "\n".join(map(str, missing))
+
+
+def test_pv_plan_query():
+    """kmb_debug_pv_plan: argument checks, only the family for another family, and the fields it shares with
+    kmb_debug_product_plan; the ring stages shrink with D and are fewer with less shared memory, and too little for the
+    resident u tile is KMB_ERR_UNSUPPORTED."""
+    import ctypes
+
+    from kernel_matrix_benchmarks_b200 import _lib, product
+
+    lib = _lib.load()
+    out = (ctypes.c_int64 * len(product.PV_PLAN_FIELDS))()
+    assert lib.kmb_debug_pv_plan(300, 700, 64, 64, 0, 0, 5, 0, dc.SMEM_OPTIN, out) == _lib.KMB_ERR_INVALID   # sms < 1
+    assert lib.kmb_debug_pv_plan(300, 700, 64, 64, 0, 0, 5, dc.SMS, 0, out) == _lib.KMB_ERR_INVALID          # smem < 1
+    assert lib.kmb_debug_pv_plan(300, 0, 64, 64, 0, 0, 5, dc.SMS, dc.SMEM_OPTIN, out) == _lib.KMB_ERR_INVALID     # M < 1
+    assert lib.kmb_debug_pv_plan(300, 700, 64, 64, 0, 0, 5, dc.SMS, 100000, out) == _lib.KMB_ERR_UNSUPPORTED
+    plan = lambda *a, **k: product.pv_plan(*a, sms=dc.SMS, smem_optin=dc.SMEM_OPTIN, **k)  # noqa: E731
+    p = plan(100, 700, 64, 3)
+    assert p["family"] == "tensor" and set(p.values()) == {"tensor", -1}
+    for kernel in dc.KERNELS:
+        for path in ("auto", "tensor_f16", "tensor_tf32"):
+            for N, M, D, E in ((100, 700, 40, 5), (401, 50, 128, 129), (20000, 9000, 3, 64), (300, 700, 17, 96)):
+                p, d = plan(N, M, D, E, kernel=kernel, path=path), product.dispatch_plan(N, M, D, E, kernel=kernel, path=path)
+                assert p["family"] == d["family"], (kernel, path, N, M, D, E)
+                if d["family"] not in ("pv", "pv16", "pv16_pair"):
+                    continue
+                assert (p["passes"], p["row_tiles"]) == (d["passes"], d["row_tiles"])
+                assert p["pair"] == (d["family"] == "pv16_pair") and p["grid"] == dc.SMS
+                blk = 64 if d["family"] == "pv" else 128
+                assert p["source_blocks"] == -(-M // blk) and p["eb_first"] == min(E, 64)
+                assert p["eb_last"] == E - 64 * (p["passes"] - 1) and p["ebp_last"] == -(-p["eb_last"] // 32) * 32
+                assert p["flush_blocks"] == (64 if d["family"] == "pv" else 128)
+    stages = [plan(100, 700, D, 40, path=path)["stages"] for path in ("tensor_tf32", "tensor_f16") for D in (16, 128)]
+    assert stages[0] > stages[1] and stages[2] > stages[3], stages
+    assert product.pv_plan(100, 700, 128, 40, path="tensor_tf32", sms=dc.SMS, smem_optin=dc.SMEM_OPTIN - 20000)["stages"] < stages[1]
 
 
 def test_inverse_distance_never_resolves_to_pv16():

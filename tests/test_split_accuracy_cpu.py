@@ -15,6 +15,40 @@ def split_f16(w):
     return hi.astype(np.float64), lo.astype(np.float64), 2.0 ** (-2 * p)
 
 
+def signal_scale(m):
+    """What signal_scale_kernel (kprod_tensor_pv16.cu) does for a signal column whose largest |b| is m: q = 13 - ilogb(m),
+    clamped to [-114, 126], the range in which 2^q and 2^-q are both finite FP32 normals."""
+    q = 13 - (np.frexp(np.float32(m))[1] - 1) if 0 < m < np.inf else 0
+    return int(np.clip(q, -114, 126))
+
+
+def test_signal_scale_maps_every_normal_column_into_fp16_range():
+    """The FP16 signal planes of kprod_tensor_pv16 hold 2^q b per column.  For every column whose largest |b| is an FP32
+    normal number, 2^q max|b| lands in [2^13, 2^14) (in [1, 2^14) below 2^-113), so hi never overflows FP16 (65504) and
+    hi + lo keep 22 bits of the column's largest value: lo never sinks into FP16 subnormals far enough to lose them.  The
+    earlier clamp to [-100, 100] put max|b| = 1e35 at 7.9e4 (hi = inf, lo = -inf: NaN results) and max|b| = 1e-36 at 1.3e-6
+    (hi an FP16 subnormal: ~2e-2 relative)."""
+    rng = np.random.RandomState(9)
+    tiny = np.finfo(np.float32).tiny
+    for k in range(-126, 128):
+        m = np.float32(2.0 ** k * rng.uniform(1.0, 1.99))
+        q = signal_scale(m)
+        s, inv = np.float32(2.0 ** q), np.float32(2.0 ** -q)
+        assert np.isfinite(s) and np.isfinite(inv) and s >= tiny and inv >= tiny, k
+        top = float(m) * 2.0 ** q
+        assert (2.0 ** 13 <= top < 2.0 ** 14) if m >= 2.0 ** -113 else (1.0 <= top < 2.0 ** 14), (k, top)
+        col = np.float32(m) * np.float32(rng.uniform(-1.0, 1.0, 2000))
+        col[0] = m
+        v = col * s                                      # exact: a power of two
+        hi = v.astype(np.float16)
+        lo = (v - hi.astype(np.float32)).astype(np.float16)
+        assert np.isfinite(hi).all() and np.isfinite(lo).all(), k
+        rec = hi.astype(np.float64) + lo.astype(np.float64)
+        assert np.abs(rec - v.astype(np.float64)).max() <= 2.0 ** -22 * top, k
+    old = lambda m: int(np.clip(13 - (np.frexp(np.float32(m))[1] - 1), -100, 100))   # noqa: E731
+    assert np.float32(1e35) * 2.0 ** old(1e35) > 65504 and np.float32(1e-36) * 2.0 ** old(1e-36) < 2.0 ** -14
+
+
 def to_tf32(x):
     """cvt.rna.tf32.f32: round to nearest (ties away) on the 13 dropped mantissa bits."""
     u = np.float32(x).view(np.uint32).astype(np.uint64)

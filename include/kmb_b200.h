@@ -45,7 +45,13 @@ enum {
 enum {
     KMB_KERNEL_GAUSSIAN = 0,             /* exp(-|x-y|^2)              :20 */
     KMB_KERNEL_ABSOLUTE_EXPONENTIAL = 1, /* exp(-|x-y|)                :21 */
-    KMB_KERNEL_INVERSE_DISTANCE = 2      /* 1/|x-y|, flat indices k(M+1) zeroed  :8-15 */
+    KMB_KERNEL_INVERSE_DISTANCE = 2,     /* 1/|x-y|, flat indices k(M+1) zeroed  :8-15 */
+    KMB_KERNEL_DOT_EXPONENTIAL = 3       /* exp(<x, y>): NOT in bruteforce.py (an extension; with KMB_FLAG_NORMALIZE_ROWS
+                                            this is softmax attention softmax(x y^T) b).  Tensor paths only
+                                            (KMB_PATH_AUTO resolves to KMB_PATH_TENSOR_3XF16 at every D); the direct and
+                                            symmetric paths return KMB_ERR_UNSUPPORTED.  The plain product is FP32 and
+                                            overflows to inf where exp(<x, y>) does (<x, y> > ~88); row normalisation
+                                            runs under an online maximum and stays finite beyond that. */
 };
 
 /* query modes: BruteForceProductBLAS.query, bruteforce.py:130-153 */
@@ -140,6 +146,7 @@ int kmb_product_prepare_f32(const float* x, const float* y, int64_t n_targets, i
  * difference form otherwise (see KMB_PATH_DIRECT_F32; decided on the device), symmetric either way.
  * b == NULL means b == 1 (density estimation, bruteforce.py:150).
  * Workspace: O(n sqrt(CTAs)) floats (77 MB at n = 10^6 on one GPU), the same for every kernel_id.
+ * KMB_KERNEL_DOT_EXPONENTIAL is not symmetric in this sense (not a function of |x - y|): KMB_ERR_UNSUPPORTED.
  */
 int kmb_product_sym_workspace_bytes(int64_t n, int D, int part, int n_parts, size_t* bytes);
 int kmb_product_sym_f32(const float* y, const float* b, float* out, int64_t n, int D, int kernel_id,
@@ -196,7 +203,8 @@ int kmb_reduce_parts_f32(float* out, const float* const* parts, int n_parts, int
  * difference-form path (bruteforce.py:53-54).  All pointers are float64 device arrays; any D (one row per thread for
  * D <= 16, a tiled kernel above: what the D = 784 / D = 64 ground truth is written with); flags and
  * row_offset as kmb_product_f32.  No workspace.  Row normalisation divides by the plain row sum as the
- * reference does (a row whose kernels all underflow is 0/0 = NaN there and here).
+ * reference does (a row whose kernels all underflow is 0/0 = NaN there and here).  KMB_KERNEL_DOT_EXPONENTIAL:
+ * exp(sum_d x_d y_d) in double, the same way (as in kmb_kernel_block_f64).
  */
 int kmb_product_f64(const double* x, const double* y, const double* b, double* out, int64_t n_targets,
                     int64_t n_sources, int D, int E, int kernel_id, int flags, int64_t row_offset,
@@ -219,7 +227,8 @@ int kmb_debug_plan_waves(int64_t n_tiles, int64_t n_source_blocks, int grid, siz
 
 /* The path KMB_PATH_AUTO stands for with this D, E and kernel (any other `path` is returned unchanged; -1 on bad arguments):
  * D > 16 -> KMB_PATH_TENSOR_3XF16; D <= 16 -> KMB_PATH_DIRECT_F32, except wide signals (E >= 32) of the Gaussian /
- * exponential kernels, whose K b is a dense contraction and runs on the tensor cores as well.  Host logic only. */
+ * exponential kernels, whose K b is a dense contraction and runs on the tensor cores as well.  The dot-exponential
+ * kernel resolves to KMB_PATH_TENSOR_3XF16 at every D.  Host logic only. */
 int kmb_resolved_path(int D, int E, int kernel_id, int path);
 
 /* Diagnostics (host logic only, no GPU needed): what kmb_product_f32 would launch for this problem on a device with

@@ -16,7 +16,8 @@ LIB_PATH = os.environ.get("KMB_B200_LIB") or os.path.join(_HERE, "libkmb_b200.so
 
 KMB_OK, KMB_ERR_INVALID, KMB_ERR_UNSUPPORTED, KMB_ERR_WORKSPACE, KMB_ERR_CUDA = range(5)
 
-KERNEL_IDS = {"gaussian": 0, "absolute-exponential": 1, "inverse-distance": 2}
+# "dot-exponential" is exp(<x, y>) (softmax attention under normalize_rows): not in bruteforce.py, an extension
+KERNEL_IDS = {"gaussian": 0, "absolute-exponential": 1, "inverse-distance": 2, "dot-exponential": 3}
 FLAG_NORMALIZE_ROWS, FLAG_DENSITY, FLAG_PREPARED = 1, 2, 4
 PATH_IDS = {"auto": 0, "direct": 1, "tensor": 5, "tensor_tf32": 2, "tensor_f16": 5, "direct_diff": 3, "direct_sym": 4}
 # KMB_FAMILY_* of kmb_debug_product_plan, by value

@@ -413,7 +413,7 @@ class B200Solver(BaseSolver):
         the first device; only the matvec (10^12 pairs at config C5) is spread over the G devices of this process
         (multigpu.MultiDeviceSymmetricOps / MultiDeviceRowOps)."""
         super().__init__(kernel=kernel, dimension=dimension, normalize_rows=normalize_rows, precision=precision)
-        if kernel not in _lib.KERNEL_IDS:
+        if kernel not in _lib.KERNEL_IDS or kernel == "dot-exponential":   # exp(<x, y>): product / attention only
             raise NotImplementedError(f"B200Solver doesn't support kernel {kernel}.")
         if preconditioner not in ("auto", "nystrom", "none"):
             raise ValueError(f"unknown preconditioner {preconditioner!r} (expected 'auto', 'nystrom' or 'none')")

@@ -259,7 +259,9 @@ __global__ void fill_kernel(float* out, long long n, float v) {
 
 static int check_product_args(int64_t N, int64_t M, int D, int E, int kid, int flags, int path) {
     if (N < 0 || M < 1 || D < 1 || E < 1) return set_error(KMB_ERR_INVALID, "bad sizes N=%lld M=%lld D=%d E=%d", (long long)N, (long long)M, D, E);
-    if (kid < 0 || kid > KMB_KERNEL_INVERSE_DISTANCE) return set_error(KMB_ERR_UNSUPPORTED, "unknown kernel id %d", kid);
+    if (kid < 0 || kid > KMB_KERNEL_DOT_EXPONENTIAL) return set_error(KMB_ERR_UNSUPPORTED, "unknown kernel id %d", kid);
+    if (kid == KMB_KERNEL_DOT_EXPONENTIAL && (path == KMB_PATH_DIRECT_F32 || path == KMB_PATH_DIRECT_DIFF || path == KMB_PATH_DIRECT_SYM))
+        return set_error(KMB_ERR_UNSUPPORTED, "the dot-exponential kernel runs on the tensor paths only (path %d)", path);
     if (flags & ~(KMB_FLAG_NORMALIZE_ROWS | KMB_FLAG_DENSITY | KMB_FLAG_PREPARED)) return set_error(KMB_ERR_INVALID, "unknown flags 0x%x", flags);
     if ((flags & KMB_FLAG_DENSITY) && E != 1) return set_error(KMB_ERR_INVALID, "density estimation implies E == 1 (got %d)", E);
     if (path < KMB_PATH_AUTO || path > KMB_PATH_TENSOR_3XF16) return set_error(KMB_ERR_INVALID, "unknown path %d", path);
@@ -274,11 +276,12 @@ static int check_product_args(int64_t N, int64_t M, int D, int E, int kid, int f
 // KMB_PATH_AUTO.  D > 16: tensor path.  D <= 16: the direct FP32 kernel -- unless the signal is wide (E >= 32) and the
 // kernel is one the FP16-plane P.B kernel covers: then K b is a dense contraction and belongs on the tensor cores too
 // (D = 3, E = 64: 1531 against 231 Gpairs/s, 1.4e-5 against 7e-7 relative -- the tensor path's tolerance is 1e-4).
+// The dot-exponential kernel has no direct kernel: the FP16-plane tensor path at every D (the planes pad D to 16).
 constexpr int kWideSignal = 32;
 bool tensor_pv16_applicable(int D, int E, int kid);   // kprod_tensor_pv16.cu
 static int resolve_path(int D, int E, int kid, int path) {
     if (path != KMB_PATH_AUTO) return path;
-    if (D > 16) return KMB_PATH_TENSOR_3XF16;
+    if (D > 16 || kid == KMB_KERNEL_DOT_EXPONENTIAL) return KMB_PATH_TENSOR_3XF16;
     return (E >= kWideSignal && tensor_pv16_applicable(D, E, kid)) ? KMB_PATH_TENSOR_3XF16 : KMB_PATH_DIRECT_F32;
 }
 
@@ -532,7 +535,7 @@ int kmb_debug_plan_waves(int64_t n_tiles, int64_t n_source_blocks, int grid, siz
 }
 
 int kmb_resolved_path(int D, int E, int kernel_id, int path) {
-    if (D < 1 || E < 1 || kernel_id < KMB_KERNEL_GAUSSIAN || kernel_id > KMB_KERNEL_INVERSE_DISTANCE || path < KMB_PATH_AUTO ||
+    if (D < 1 || E < 1 || kernel_id < KMB_KERNEL_GAUSSIAN || kernel_id > KMB_KERNEL_DOT_EXPONENTIAL || path < KMB_PATH_AUTO ||
         path > KMB_PATH_TENSOR_3XF16)
         return -1;
     return resolve_path(D, E, kernel_id, path);
@@ -634,7 +637,7 @@ int kmb_debug_sym_unit(int64_t n, int64_t total_ctas, int64_t u, int64_t* out8) 
 int kmb_kernel_block_f64(const double* x, const double* y, double* out, int64_t n, int64_t m, int D, int kernel_id, void* stream_) {
     g_launches = 0;
     if (n < 0 || m < 1 || D < 1) return set_error(KMB_ERR_INVALID, "bad sizes n=%lld m=%lld D=%d", (long long)n, (long long)m, D);
-    if (kernel_id < KMB_KERNEL_GAUSSIAN || kernel_id > KMB_KERNEL_INVERSE_DISTANCE) return set_error(KMB_ERR_UNSUPPORTED, "unknown kernel %d", kernel_id);
+    if (kernel_id < KMB_KERNEL_GAUSSIAN || kernel_id > KMB_KERNEL_DOT_EXPONENTIAL) return set_error(KMB_ERR_UNSUPPORTED, "unknown kernel %d", kernel_id);
     if (!x || !y || !out) return set_error(KMB_ERR_INVALID, "x, y and out must not be NULL");
     if (n == 0) return KMB_OK;
     return kernel_block_f64(x, y, out, n, m, D, kernel_id, static_cast<cudaStream_t>(stream_));

@@ -7,6 +7,9 @@
 //
 // Row normalisation divides by the plain row sum like the reference does (no running maximum): a row
 // whose kernels all underflow in float64 is 0/0 = NaN there and here.
+//
+// The dot-exponential kernel exp(<x, y>) (not in bruteforce.py) runs through the same kernels: its pair term is the
+// product x_d y_d where the others have (x_d - y_d)^2.
 #include "kmb_common.cuh"
 
 namespace kmb {
@@ -17,9 +20,19 @@ constexpr int F64_THREADS = 128;
 constexpr int F64_SB = 256;        // sources per shared-memory stage
 constexpr int F64_MAX_D = 16, F64_MAX_E = 8;
 
+// what one coordinate adds to the kernel's argument: (a - b)^2 (squared distance, bruteforce.py:53-54) or a b (<x, y>)
 template <int KID>
-__device__ __forceinline__ double kernel_value_f64(double d2) {
+__device__ __forceinline__ double pair_term(double a, double b, double acc) {
+    if constexpr (KID == KMB_KERNEL_DOT_EXPONENTIAL) return fma(a, b, acc);
+    else {
+        const double diff = a - b;
+        return fma(diff, diff, acc);
+    }
+}
+template <int KID>
+__device__ __forceinline__ double kernel_value_f64(double d2) {   // d2: the sum of pair_term
     if constexpr (KID == KMB_KERNEL_GAUSSIAN) return exp(-d2);
+    else if constexpr (KID == KMB_KERNEL_DOT_EXPONENTIAL) return exp(d2);
     else if constexpr (KID == KMB_KERNEL_ABSOLUTE_EXPONENTIAL) return exp(-sqrt(fmax(d2, 0.0)));   // bruteforce.py:21
     else return 1.0 / sqrt(fmax(d2, 0.0));                                                          // bruteforce.py:10-11
 }
@@ -57,10 +70,7 @@ kprod_f64_kernel(const double* __restrict__ x, const double* __restrict__ y, con
                 double d2 = 0.0;
 #pragma unroll
                 for (int d = 0; d < F64_MAX_D; ++d) {
-                    if (d < D) {
-                        const double diff = xr[d] - sy[j * D + d];
-                        d2 = fma(diff, diff, d2);
-                    }
+                    if (d < D) d2 = pair_term<KID>(xr[d], sy[j * D + d], d2);
                 }
                 double k = kernel_value_f64<KID>(d2);
                 if constexpr (KID == KMB_KERNEL_INVERSE_DISTANCE) {
@@ -131,10 +141,7 @@ kprod_f64_wide_kernel(const double* __restrict__ x, const double* __restrict__ y
 #pragma unroll
                 for (int i = 0; i < 4; ++i)
 #pragma unroll
-                    for (int j = 0; j < 4; ++j) {
-                        const double diff = xv[i] - yv[j];
-                        d2[i][j] = fma(diff, diff, d2[i][j]);
-                    }
+                    for (int j = 0; j < 4; ++j) d2[i][j] = pair_term<KID>(xv[i], yv[j], d2[i][j]);
             }
         }
 #pragma unroll
@@ -217,10 +224,7 @@ __global__ void __launch_bounds__(256) kernel_block_f64_kernel(const double* __r
     const long long i = blockIdx.x * 8ll + threadIdx.y;
     if (i >= n || j >= m) return;
     double d2 = 0.0;
-    for (int d = 0; d < D; ++d) {
-        const double diff = x[i * D + d] - y[j * D + d];
-        d2 = fma(diff, diff, d2);
-    }
+    for (int d = 0; d < D; ++d) d2 = pair_term<KID>(x[i * D + d], y[j * D + d], d2);
     out[i * m + j] = kernel_value_f64<KID>(d2);
 }
 
@@ -232,6 +236,7 @@ int kernel_block_f64(const double* x, const double* y, double* out, int64_t n, i
     switch (kernel_id) {
         case KMB_KERNEL_GAUSSIAN: kernel_block_f64_kernel<KMB_KERNEL_GAUSSIAN><<<grid, block, 0, stream>>>(x, y, out, n, m, D); break;
         case KMB_KERNEL_ABSOLUTE_EXPONENTIAL: kernel_block_f64_kernel<KMB_KERNEL_ABSOLUTE_EXPONENTIAL><<<grid, block, 0, stream>>>(x, y, out, n, m, D); break;
+        case KMB_KERNEL_DOT_EXPONENTIAL: kernel_block_f64_kernel<KMB_KERNEL_DOT_EXPONENTIAL><<<grid, block, 0, stream>>>(x, y, out, n, m, D); break;
         default: kernel_block_f64_kernel<KMB_KERNEL_INVERSE_DISTANCE><<<grid, block, 0, stream>>>(x, y, out, n, m, D); break;
     }
     KMB_CUDA_CHECK(cudaGetLastError());
@@ -252,12 +257,14 @@ int product_f64(const double* x, const double* y, const double* b, double* out, 
         switch (kernel_id) {
             case KMB_KERNEL_GAUSSIAN: return launch_f64_wide<KMB_KERNEL_GAUSSIAN>(x, y, sig, out, N, M, D, E, flags, row_offset, stream);
             case KMB_KERNEL_ABSOLUTE_EXPONENTIAL: return launch_f64_wide<KMB_KERNEL_ABSOLUTE_EXPONENTIAL>(x, y, sig, out, N, M, D, E, flags, row_offset, stream);
+            case KMB_KERNEL_DOT_EXPONENTIAL: return launch_f64_wide<KMB_KERNEL_DOT_EXPONENTIAL>(x, y, sig, out, N, M, D, E, flags, row_offset, stream);
             default: return launch_f64_wide<KMB_KERNEL_INVERSE_DISTANCE>(x, y, sig, out, N, M, D, E, flags, row_offset, stream);
         }
     }
     switch (kernel_id) {
         case KMB_KERNEL_GAUSSIAN: return launch_f64<KMB_KERNEL_GAUSSIAN>(x, y, sig, out, N, M, D, E, flags, row_offset, stream);
         case KMB_KERNEL_ABSOLUTE_EXPONENTIAL: return launch_f64<KMB_KERNEL_ABSOLUTE_EXPONENTIAL>(x, y, sig, out, N, M, D, E, flags, row_offset, stream);
+        case KMB_KERNEL_DOT_EXPONENTIAL: return launch_f64<KMB_KERNEL_DOT_EXPONENTIAL>(x, y, sig, out, N, M, D, E, flags, row_offset, stream);
         default: return launch_f64<KMB_KERNEL_INVERSE_DISTANCE>(x, y, sig, out, N, M, D, E, flags, row_offset, stream);
     }
 }

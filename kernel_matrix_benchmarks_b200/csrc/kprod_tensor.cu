@@ -722,6 +722,33 @@ static __global__ void __launch_bounds__(256) split_points_kernel(const float* _
     if (lane == 0) norm2[row] = acc;
 }
 
+// One warp per point of the dot-exponential kernel: operand = s p (TF32) or s 2^p p (FP16; 2^p = sscale[0]), uncentred and
+// with multiplier 1 on both planes, split into hi + lo; norm2 = 0.  S = s^2 <x, y> = log2(e) <x, y> is then what the
+// Gaussian epilogue's S - |u|^2 - |v|^2 evaluates: the log2 of exp(<x, y>).
+constexpr float kDotScale = 1.2011224087864498f;   // sqrt(log2 e)
+template <int ELT>
+static __global__ void __launch_bounds__(256) split_points_dot_kernel(const float* __restrict__ pts, long long n, int D, int Dp,
+                                                                      float scale, const float* __restrict__ sscale, void* hi,
+                                                                      void* lo, float* __restrict__ norm2) {
+    const long long row = (blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (row >= n) return;
+    const float m = ELT == ELT_F16 ? scale * __ldg(sscale) : scale;
+    for (int d = lane; d < Dp; d += 32) {
+        const float w = d < D ? m * pts[row * D + d] : 0.f;
+        if constexpr (ELT == ELT_F16) {
+            const __half h = __float2half_rn(w);
+            static_cast<__half*>(hi)[row * Dp + d] = h;
+            static_cast<__half*>(lo)[row * Dp + d] = __float2half_rn(w - __half2float(h));
+        } else {
+            const float h = to_tf32(w);
+            static_cast<float*>(hi)[row * Dp + d] = h;
+            static_cast<float*>(lo)[row * Dp + d] = to_tf32(w - h);
+        }
+    }
+    if (lane == 0) norm2[row] = 0.f;
+}
+
 // (rows, cols) fp32 row-major; box = 32 floats x box_rows rows, 128-byte swizzle, out-of-bounds reads as zero
 int make_tensor_map(CUtensorMap* map, const float* base, long long rows, int cols, int box_rows) {
     using EncodeFn = CUresult (*)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
@@ -748,6 +775,14 @@ int make_tensor_map(CUtensorMap* map, const float* base, long long rows, int col
 
 int tensor_prepass(const float* x, const float* y, int64_t N, int64_t M, int D, int Dp, int kid, float* center, float* cpart,
                    float* uh, float* ul, float* vh, float* vl, float* un, float* vn, cudaStream_t stream) {
+    if (kid == KMB_KERNEL_DOT_EXPONENTIAL) {   // no centre, no squared norms
+        split_points_dot_kernel<ELT_TF32><<<static_cast<unsigned>((N * 32 + 255) / 256), 256, 0, stream>>>(x, N, D, Dp, kDotScale, nullptr, uh, ul, un);
+        KMB_CUDA_CHECK(cudaGetLastError());
+        split_points_dot_kernel<ELT_TF32><<<static_cast<unsigned>((M * 32 + 255) / 256), 256, 0, stream>>>(y, M, D, Dp, kDotScale, nullptr, vh, vl, vn);
+        KMB_CUDA_CHECK(cudaGetLastError());
+        count_launch(2);
+        return KMB_OK;
+    }
     // scale folds log2(e) into the data as in the direct path; the A operand carries the factor 2 of 2 u.v
     const float scale = kid == KMB_KERNEL_GAUSSIAN ? 1.2011224087864498f : kid == KMB_KERNEL_ABSOLUTE_EXPONENTIAL ? 1.4426950408889634f : 1.f;
     const int cblocks = static_cast<int>(std::min<long long>(CENTER_BLOCKS, (M + 7) / 8));
@@ -798,6 +833,23 @@ static __global__ void __launch_bounds__(256) column_stats_kernel(const float* _
         pmax[static_cast<size_t>(blockIdx.x) * D + col] = h;
     }
 }
+// red[0 .. 255] = per-thread largest |coordinate| (before the scale s): max-reduce, then sscale[0] = 2^p with
+// 2^p s max in [2^13, 2^14), sscale[1] = 2^-2p
+__device__ __forceinline__ void operand_scale(float* red, float scale, float* __restrict__ sscale) {
+    __syncthreads();
+    for (int o = 128; o > 0; o >>= 1) {
+        if (threadIdx.x < o) red[threadIdx.x] = fmaxf(red[threadIdx.x], red[threadIdx.x + o]);
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        const float mw = scale * red[0];
+        int p = 0;
+        if (mw > 0.f && mw < INFINITY) p = 13 - ilogbf(mw);   // 2^p mw in [2^13, 2^14)
+        p = max(-60, min(60, p));
+        sscale[0] = exp2f(static_cast<float>(p));
+        sscale[1] = exp2f(static_cast<float>(-2 * p));
+    }
+}
 // one block: centre = column means of y; the largest |point - centre| follows from the column extrema
 static __global__ void __launch_bounds__(256) center_scale_kernel(const float* __restrict__ ystats, int yblocks,
                                                                   const float* __restrict__ xstats, int xblocks, long long M,
@@ -825,19 +877,23 @@ static __global__ void __launch_bounds__(256) center_scale_kernel(const float* _
         center[col] = c;
     }
     red[threadIdx.x] = dev;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-        if (threadIdx.x < o) red[threadIdx.x] = fmaxf(red[threadIdx.x], red[threadIdx.x + o]);
-        __syncthreads();
+    operand_scale(red, scale, sscale);
+}
+// one block: the dot-exponential kernel's operands are not centred, so p follows from the largest |coordinate| of x and y
+static __global__ void __launch_bounds__(256) dot_scale_kernel(const float* __restrict__ ystats, int yblocks,
+                                                               const float* __restrict__ xstats, int xblocks, int D, float scale,
+                                                               float* __restrict__ sscale) {
+    __shared__ float red[256];
+    const size_t plane = static_cast<size_t>(CENTER_BLOCKS) * D;
+    float mag = 0.f;
+    for (int col = threadIdx.x; col < D; col += 256) {
+        for (int b = 0; b < yblocks; ++b)
+            mag = fmaxf(mag, fmaxf(-ystats[plane + static_cast<size_t>(b) * D + col], ystats[2 * plane + static_cast<size_t>(b) * D + col]));
+        for (int b = 0; b < xblocks; ++b)
+            mag = fmaxf(mag, fmaxf(-xstats[plane + static_cast<size_t>(b) * D + col], xstats[2 * plane + static_cast<size_t>(b) * D + col]));
     }
-    if (threadIdx.x == 0) {
-        const float mw = scale * red[0];
-        int p = 0;
-        if (mw > 0.f && mw < INFINITY) p = 13 - ilogbf(mw);   // 2^p mw in [2^13, 2^14)
-        p = max(-60, min(60, p));
-        sscale[0] = exp2f(static_cast<float>(p));
-        sscale[1] = exp2f(static_cast<float>(-2 * p));
-    }
+    red[threadIdx.x] = mag;
+    operand_scale(red, scale, sscale);
 }
 // One warp per point: w = s (p - c); operand = mult 2^p w split into FP16 hi + lo; norm2 = |w|^2.
 static __global__ void __launch_bounds__(256) split_points_f16_kernel(const float* __restrict__ pts, long long n, int D, int Dp,
@@ -899,6 +955,16 @@ int tensor_prepass_f16(const float* x, const float* y, int64_t N, int64_t M, int
     KMB_CUDA_CHECK(cudaGetLastError());
     column_stats_kernel<<<dim3(xblocks, (D + 31) / 32), 256, 0, stream>>>(x, N, D, xs, xs + plane, xs + 2 * plane);
     KMB_CUDA_CHECK(cudaGetLastError());
+    if (kid == KMB_KERNEL_DOT_EXPONENTIAL) {   // no centre, no squared norms (|v|^2 of padded sources: f16_points_prepass)
+        dot_scale_kernel<<<1, 256, 0, stream>>>(ys, yblocks, xs, xblocks, D, kDotScale, sscale);
+        KMB_CUDA_CHECK(cudaGetLastError());
+        split_points_dot_kernel<ELT_F16><<<static_cast<unsigned>((N * 32 + 255) / 256), 256, 0, stream>>>(x, N, D, Dp16, kDotScale, sscale, uh, ul, un);
+        KMB_CUDA_CHECK(cudaGetLastError());
+        split_points_dot_kernel<ELT_F16><<<static_cast<unsigned>((M * 32 + 255) / 256), 256, 0, stream>>>(y, M, D, Dp16, kDotScale, sscale, vh, vl, vn);
+        KMB_CUDA_CHECK(cudaGetLastError());
+        count_launch(5);
+        return KMB_OK;
+    }
     center_scale_kernel<<<1, 256, 0, stream>>>(ys, yblocks, xs, xblocks, M, D, Dp16, scale, center, sscale);
     KMB_CUDA_CHECK(cudaGetLastError());
     split_points_f16_kernel<<<static_cast<unsigned>((N * 32 + 255) / 256), 256, 0, stream>>>(
@@ -1254,9 +1320,10 @@ int tensor_product(const float* x, const float* y, const float* b, float* out, i
         P.C_last = pl.waves.C_last;
         P.slots_per_wave = pl.waves.slots_per_wave;
         if (ev0 && pass == pl.n_passes - 1) KMB_CUDA_CHECK(cudaEventRecord(ev0, stream));
-        if (int rc = pl.pair ? launch_pair_any(kid, norm, pl.e_chunk, maps, P, grid, stream)
-                 : f16   ? launch_any<tc::ELT_F16>(kid, norm, pl.e_chunk, maps, P, grid, stream)
-                         : launch_any<tc::ELT_TF32>(kid, norm, pl.e_chunk, maps, P, grid, stream))
+        const int ekid = tc::epilogue_kid(kid);
+        if (int rc = pl.pair ? launch_pair_any(ekid, norm, pl.e_chunk, maps, P, grid, stream)
+                 : f16   ? launch_any<tc::ELT_F16>(ekid, norm, pl.e_chunk, maps, P, grid, stream)
+                         : launch_any<tc::ELT_TF32>(ekid, norm, pl.e_chunk, maps, P, grid, stream))
             return rc;
         if (ev1 && pass == pl.n_passes - 1) KMB_CUDA_CHECK(cudaEventRecord(ev1, stream));
         count_launch();

@@ -676,7 +676,7 @@ int tensor_pv_product(const float* x, const float* y, const float* b, float* out
         P.slots_per_wave = pl.waves.slots_per_wave;
         if (ev0 && pass == n_passes - 1) KMB_CUDA_CHECK(cudaEventRecord(ev0, stream));
         int rc;
-        switch (kid * 2 + (norm ? 1 : 0)) {
+        switch (tc::epilogue_kid(kid) * 2 + (norm ? 1 : 0)) {   // dot-exponential: the Gaussian instantiations
             case 0: rc = launch_pv<KMB_KERNEL_GAUSSIAN, false>(maps, P, grid, pl.smem, stream); break;
             case 1: rc = launch_pv<KMB_KERNEL_GAUSSIAN, true>(maps, P, grid, pl.smem, stream); break;
             case 2: rc = launch_pv<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false>(maps, P, grid, pl.smem, stream); break;

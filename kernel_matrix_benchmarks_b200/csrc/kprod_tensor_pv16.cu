@@ -998,7 +998,7 @@ int launch_pv16(const CUtensorMap* m, const pv16::Params& P, int grid, int smem,
 }  // namespace
 
 bool tensor_pv16_applicable(int D, int E, int kid) {
-    return E > 4 && D <= 128 && (kid == KMB_KERNEL_GAUSSIAN || kid == KMB_KERNEL_ABSOLUTE_EXPONENTIAL);
+    return E > 4 && D <= 128 && (kid == KMB_KERNEL_GAUSSIAN || kid == KMB_KERNEL_ABSOLUTE_EXPONENTIAL || kid == KMB_KERNEL_DOT_EXPONENTIAL);
 }
 int tensor_pv16_signal_block() { return pv16::MAX_EB; }
 
@@ -1071,7 +1071,8 @@ int tensor_pv16_product(const float* x, const float* y, const float* b, float* o
     // CTA pairs: each CTA loads 64 of a block's 128 sources and half of the pass's signal columns
     if (int rc = tc::make_tensor_map_f16(&maps[2], vh, M, pl.Dp, pl.pair ? pv16::TNS / 2 : pv16::TNS)) return rc;
     if (int rc = tc::make_tensor_map_f16(&maps[3], vl, M, pl.Dp, pl.pair ? pv16::TNS / 2 : pv16::TNS)) return rc;
-    const bool xk = (kid == KMB_KERNEL_GAUSSIAN) ? pv16::extra_k<KMB_KERNEL_GAUSSIAN>() : pv16::extra_k<KMB_KERNEL_ABSOLUTE_EXPONENTIAL>();
+    const int ekid = tc::epilogue_kid(kid);   // dot-exponential: the Gaussian instantiations
+    const bool xk = (ekid == KMB_KERNEL_GAUSSIAN) ? pv16::extra_k<KMB_KERNEL_GAUSSIAN>() : pv16::extra_k<KMB_KERNEL_ABSOLUTE_EXPONENTIAL>();
     if (xk) {   // |u|^2, |v|^2 as operands of one more K step (16-bit elements: the FP16 map serves BF16 rows as well)
         const long long rows = N + pl.Mp;
         pv16::norm_tiles_kernel<<<static_cast<unsigned>((rows + 255) / 256), 256, 0, stream>>>(
@@ -1123,7 +1124,7 @@ int tensor_pv16_product(const float* x, const float* y, const float* b, float* o
         P.slots_per_wave = pl.waves.slots_per_wave;
         if (ev0 && pass == n_passes - 1) KMB_CUDA_CHECK(cudaEventRecord(ev0, stream));
         int rc;
-        switch (kid * 2 + (norm ? 1 : 0)) {
+        switch (ekid * 2 + (norm ? 1 : 0)) {
             case 0: rc = launch_pv16<KMB_KERNEL_GAUSSIAN, false>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
             case 1: rc = launch_pv16<KMB_KERNEL_GAUSSIAN, true>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
             case 2: rc = launch_pv16<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;

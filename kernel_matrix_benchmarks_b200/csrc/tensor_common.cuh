@@ -247,6 +247,10 @@ __device__ __forceinline__ float log2_kernel_from_parts(float s, float un, float
     else return -sqrt_approx(fmaxf((un + vn) - s, 0.f));
 }
 
+// The instantiation a kernel's tensor-path product launches.  The dot-exponential kernel has none of its own: its prepass
+// (no centre, multiplier 1 on both planes, |u|^2 = |v|^2 = 0) makes S = log2(e) <x, y>, so the Gaussian epilogues'
+// log2 k = S - |u|^2 - |v|^2 is log2 exp(<x, y>) exactly (DESIGN.md, "The dot-exponential kernel").
+__host__ __device__ constexpr int epilogue_kid(int kid) { return kid == KMB_KERNEL_DOT_EXPONENTIAL ? KMB_KERNEL_GAUSSIAN : kid; }
 
 // ---- host helpers shared by both tensor kernels (defined in kprod_tensor.cu) ----------------------
 int make_tensor_map(CUtensorMap* map, const float* base, long long rows, int cols, int box_rows);

@@ -49,10 +49,14 @@ SYM_MIN_POINTS = 32768
 last_path = None  # the path the last kernel_product call took ("auto" resolved: direct_sym here, otherwise kmb_resolved_path)
 
 
+# the kernels of bruteforce.py:18-22: functions of |x - y|, so K is symmetric when the targets are the sources
+SYMMETRIC_KERNELS = ("gaussian", "absolute-exponential", "inverse-distance")
+
+
 def symmetric_applies(x, y, kernel, normalize_rows=False, density_estimation=False, E=1):
-    """targets *are* the sources (same tensor), plain product or density of any kernel (all of bruteforce.py:18-22 are
-    functions of |x - y|, so K is symmetric), D <= 3, E == 1."""
-    return (x.data_ptr() == y.data_ptr() and x.shape == y.shape and kernel in _lib.KERNEL_IDS and not normalize_rows
+    """targets *are* the sources (same tensor), plain product or density of a kernel of bruteforce.py (all of :18-22 are
+    functions of |x - y|, so K is symmetric; dot-exponential has no symmetric kernel), D <= 3, E == 1."""
+    return (x.data_ptr() == y.data_ptr() and x.shape == y.shape and kernel in SYMMETRIC_KERNELS and not normalize_rows
             and E == 1 and x.shape[1] <= 3)
 
 
@@ -131,13 +135,14 @@ def prepare_points(x, y, *, kernel="gaussian", path="auto", workspace=None, min_
     operand planes, squared norms) is written to the head of ``workspace``.  Returns the buffer it was written to: a
     later ``kernel_product(..., prepared=token)`` on the same x, y, kernel, path and workspace skips the prepass as long
     as the workspace has not been reallocated since (``token`` is compared with the buffer in use; otherwise the
-    product silently does the prepass itself).  No-op (returns None) on the other paths."""
+    product silently does the prepass itself).  No-op (returns None) on the other paths.  The dot-exponential kernel
+    takes the FP16 tensor path at every D, so it is prepared at every D."""
     lib = _lib.load()
     _check_f32("target points", x)
     _check_f32("source points", y, x.shape[1])
     N, D = x.shape
     M = y.shape[0]
-    if D <= 16 or _lib.PATH_IDS[path] not in (_lib.PATH_IDS["auto"], _lib.PATH_IDS["tensor_f16"]):
+    if (D <= 16 and kernel != "dot-exponential") or _lib.PATH_IDS[path] not in (_lib.PATH_IDS["auto"], _lib.PATH_IDS["tensor_f16"]):
         return None
     kid, pid = _lib.KERNEL_IDS[kernel], _lib.PATH_IDS[path]
     need = ctypes.c_size_t(0)

@@ -76,6 +76,17 @@ enum {
                                   so that the largest operand lies in [2^13, 2^15); hi + lo carry 22 significand
                                   bits as the TF32 split does, kind::f16 MMAs run at twice the TF32 rate and the
                                   operand planes are half as large.  What KMB_PATH_AUTO picks for D > 16. */
+    KMB_PATH_TENSOR_1XF16 = 6, /* KMB_PATH_TENSOR_3XF16 with only the hi.hi term: the same prepass and hi planes (11 significand
+                                  bits per operand), but the lo planes of the points and of the signal are neither loaded
+                                  nor multiplied, S = u.v and (E > 4) P.B are one kind::f16 MMA per K step where the
+                                  three-term path issues three, and P is written to tensor memory as one FP16 plane (the
+                                  row sums use the same rounded weights).  Float16-class results: about 1e-5 relative for
+                                  E <= 4 (S alone), about 3e-4 to 1e-3 for E > 4 (dominated by rounding P and b to FP16),
+                                  still well inside what a float16 evaluation of the reference gives.  Gaussian,
+                                  exponential and dot-exponential kernels; the inverse distance (1/|x - y| amplifies the
+                                  cancellation error of S near coincident points) and shapes whose three-term product
+                                  would take the TF32 P.B kernel return KMB_ERR_UNSUPPORTED.  Never chosen by
+                                  KMB_PATH_AUTO.  A workspace prepared for one path belongs to that path. */
     KMB_PATH_DIRECT_SYM = 4    /* targets == sources (the reference's same_points, base.py:56-79): x must be the
                                   same pointer as y.  Plain product or density of any kernel, D <= 3, E == 1: every kernel
                                   value is evaluated once and feeds a_i += k b_j and a_j += k b_i (K is
@@ -119,8 +130,8 @@ int kmb_product_f32(const float* x, const float* y, const float* b, float* out, 
                     int64_t row_offset, void* workspace, size_t workspace_bytes, void* stream);
 
 /* The points-only part of a product: what the reference does in fit() (bruteforce.py:113-120 builds the kernel matrix
- * from the points; query() only multiplies, :130-153).  For the FP16 tensor path (KMB_PATH_TENSOR_3XF16 / KMB_PATH_AUTO
- * with D > 16) this is the prepass -- column statistics, centre, power-of-two scale, FP16 hi/lo operand planes, squared
+ * from the points; query() only multiplies, :130-153).  For the FP16 tensor paths (KMB_PATH_TENSOR_3XF16 / KMB_PATH_AUTO
+ * with D > 16, KMB_PATH_TENSOR_1XF16 at every D) this is the prepass -- column statistics, centre, power-of-two scale, FP16 hi/lo operand planes, squared
  * norms -- written to the head of `workspace`, whose layout does not depend on E.  A later kmb_product_f32 with the same
  * x, y, sizes, kernel and path on the SAME workspace memory may then pass KMB_FLAG_PREPARED and skips it; the caller
  * must prepare again if the workspace was reallocated (e.g. grown for a wider signal) or the points changed.  Other
@@ -225,7 +236,8 @@ int kmb_kernel_block_f64(const double* x, const double* y, double* out, int64_t 
  * [n_source_blocks (b % C) / C, n_source_blocks (b % C + 1) / C). */
 int kmb_debug_plan_waves(int64_t n_tiles, int64_t n_source_blocks, int grid, size_t row_tile_bytes, int64_t* out7);
 
-/* The path KMB_PATH_AUTO stands for with this D, E and kernel (any other `path` is returned unchanged; -1 on bad arguments):
+/* The path KMB_PATH_AUTO stands for with this D, E and kernel (any other `path`, KMB_PATH_TENSOR_1XF16 included, is returned
+ * unchanged; -1 on bad arguments):
  * D > 16 -> KMB_PATH_TENSOR_3XF16; D <= 16 -> KMB_PATH_DIRECT_F32, except wide signals (E >= 32) of the Gaussian /
  * exponential kernels, whose K b is a dense contraction and runs on the tensor cores as well.  The dot-exponential
  * kernel resolves to KMB_PATH_TENSOR_3XF16 at every D.  Host logic only. */

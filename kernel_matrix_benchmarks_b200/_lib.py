@@ -19,7 +19,9 @@ KMB_OK, KMB_ERR_INVALID, KMB_ERR_UNSUPPORTED, KMB_ERR_WORKSPACE, KMB_ERR_CUDA = 
 # "dot-exponential" is exp(<x, y>) (softmax attention under normalize_rows): not in bruteforce.py, an extension
 KERNEL_IDS = {"gaussian": 0, "absolute-exponential": 1, "inverse-distance": 2, "dot-exponential": 3}
 FLAG_NORMALIZE_ROWS, FLAG_DENSITY, FLAG_PREPARED = 1, 2, 4
-PATH_IDS = {"auto": 0, "direct": 1, "tensor": 5, "tensor_tf32": 2, "tensor_f16": 5, "direct_diff": 3, "direct_sym": 4}
+# "tensor_f16x1": the FP16 tensor path with one hi.hi term (float16-class accuracy; only when asked for, never "auto")
+PATH_IDS = {"auto": 0, "direct": 1, "tensor": 5, "tensor_tf32": 2, "tensor_f16": 5, "direct_diff": 3, "direct_sym": 4,
+            "tensor_f16x1": 6}
 # KMB_FAMILY_* of kmb_debug_product_plan, by value
 FAMILIES = ("direct", "sym", "tensor", "tensor_pair", "pv", "pv16", "pv16_pair", "fill", "unsupported")
 

@@ -169,6 +169,8 @@ class B200Product(BaseProduct):
             raise NotImplementedError(f"B200Product doesn't support kernel {kernel}.")
         if path not in _lib.PATH_IDS:
             raise ValueError(f"unknown path {path!r} (expected one of {sorted(_lib.PATH_IDS)})")
+        if path == "tensor_f16x1" and kernel == "inverse-distance":   # 1/|x - y| amplifies the error of a one-term S
+            raise NotImplementedError("B200Product doesn't support kernel inverse-distance on path tensor_f16x1.")
         self.dtype = _check_precision(precision, "B200Product", (np.float32, np.float64, np.float16))
         _lib.load()  # fail here, loudly, if the CUDA library is absent
         if not torch.cuda.is_available():
@@ -415,6 +417,9 @@ class B200Solver(BaseSolver):
         super().__init__(kernel=kernel, dimension=dimension, normalize_rows=normalize_rows, precision=precision)
         if kernel not in _lib.KERNEL_IDS or kernel == "dot-exponential":   # exp(<x, y>): product / attention only
             raise NotImplementedError(f"B200Solver doesn't support kernel {kernel}.")
+        if path == "tensor_f16x1":
+            raise ValueError("B200Solver doesn't support path tensor_f16x1: its matvec error (~3e-4 relative) cannot reach "
+                             "the solver's tolerances (rtol 1e-6); use path 'auto' or 'tensor_f16'.")
         if preconditioner not in ("auto", "nystrom", "none"):
             raise ValueError(f"unknown preconditioner {preconditioner!r} (expected 'auto', 'nystrom' or 'none')")
         self.preconditioner, self.precond_rank = preconditioner, int(precond_rank)

@@ -262,9 +262,12 @@ static int check_product_args(int64_t N, int64_t M, int D, int E, int kid, int f
     if (kid < 0 || kid > KMB_KERNEL_DOT_EXPONENTIAL) return set_error(KMB_ERR_UNSUPPORTED, "unknown kernel id %d", kid);
     if (kid == KMB_KERNEL_DOT_EXPONENTIAL && (path == KMB_PATH_DIRECT_F32 || path == KMB_PATH_DIRECT_DIFF || path == KMB_PATH_DIRECT_SYM))
         return set_error(KMB_ERR_UNSUPPORTED, "the dot-exponential kernel runs on the tensor paths only (path %d)", path);
+    if (kid == KMB_KERNEL_INVERSE_DISTANCE && path == KMB_PATH_TENSOR_1XF16)
+        return set_error(KMB_ERR_UNSUPPORTED, "the one-term FP16 path does not support the inverse-distance kernel (1/|x-y| amplifies "
+                                              "the error of a one-term S near coincident points)");
     if (flags & ~(KMB_FLAG_NORMALIZE_ROWS | KMB_FLAG_DENSITY | KMB_FLAG_PREPARED)) return set_error(KMB_ERR_INVALID, "unknown flags 0x%x", flags);
     if ((flags & KMB_FLAG_DENSITY) && E != 1) return set_error(KMB_ERR_INVALID, "density estimation implies E == 1 (got %d)", E);
-    if (path < KMB_PATH_AUTO || path > KMB_PATH_TENSOR_3XF16) return set_error(KMB_ERR_INVALID, "unknown path %d", path);
+    if (path < KMB_PATH_AUTO || path > KMB_PATH_TENSOR_1XF16) return set_error(KMB_ERR_INVALID, "unknown path %d", path);
     if (path == KMB_PATH_DIRECT_SYM) {
         if (N != M) return set_error(KMB_ERR_INVALID, "the symmetric path needs targets == sources (N=%lld, M=%lld)", (long long)N, (long long)M);
         if ((flags & KMB_FLAG_NORMALIZE_ROWS) || E != 1 || !sym_supported(D))
@@ -278,6 +281,10 @@ static int check_product_args(int64_t N, int64_t M, int D, int E, int kid, int f
 // (D = 3, E = 64: 1531 against 231 Gpairs/s, 1.4e-5 against 7e-7 relative -- the tensor path's tolerance is 1e-4).
 // The dot-exponential kernel has no direct kernel: the FP16-plane tensor path at every D (the planes pad D to 16).
 constexpr int kWideSignal = 32;
+// the operand planes of a tensor path (kprod_tensor.cuh: elt), -1 for the other paths
+static int tensor_elt(int path) {
+    return path == KMB_PATH_TENSOR_3XTF32 ? 0 : path == KMB_PATH_TENSOR_3XF16 ? 1 : path == KMB_PATH_TENSOR_1XF16 ? 2 : -1;
+}
 bool tensor_pv16_applicable(int D, int E, int kid);   // kprod_tensor_pv16.cu
 static int resolve_path(int D, int E, int kid, int path) {
     if (path != KMB_PATH_AUTO) return path;
@@ -457,7 +464,7 @@ int kmb_product_workspace_bytes(int64_t N, int64_t M, int D, int E, int kernel_i
         *bytes = pl.total_bytes;
         return KMB_OK;
     }
-    return tensor_workspace_bytes(N, M, D, E, kernel_id, flags, p == KMB_PATH_TENSOR_3XF16 ? 1 : 0, bytes);
+    return tensor_workspace_bytes(N, M, D, E, kernel_id, flags, tensor_elt(p), bytes);
 }
 
 int kmb_product_f32(const float* x, const float* y, const float* b, float* out, int64_t N, int64_t M, int D,
@@ -480,12 +487,12 @@ int kmb_product_f32(const float* x, const float* y, const float* b, float* out, 
     const int p = resolve_path(D, E, kernel_id, path);
     if (reinterpret_cast<uintptr_t>(workspace) % 256)
         return set_error(KMB_ERR_INVALID, "workspace must be 256-byte aligned");
-    if (p == KMB_PATH_TENSOR_3XTF32 || p == KMB_PATH_TENSOR_3XF16) {
+    if (tensor_elt(p) >= 0) {
         if (g_profile && !g_ev0) {
             KMB_CUDA_CHECK(cudaEventCreate(&g_ev0));
             KMB_CUDA_CHECK(cudaEventCreate(&g_ev1));
         }
-        const int rc = tensor_product(x, y, density ? nullptr : b, out, N, M, D, E, kernel_id, flags, p == KMB_PATH_TENSOR_3XF16 ? 1 : 0, row_offset, workspace,
+        const int rc = tensor_product(x, y, density ? nullptr : b, out, N, M, D, E, kernel_id, flags, tensor_elt(p), row_offset, workspace,
                                       workspace_bytes, stream, g_profile ? g_ev0 : nullptr, g_profile ? g_ev1 : nullptr,
                                       (flags & KMB_FLAG_PREPARED) != 0);
         if (rc == KMB_OK && g_profile) g_ev_valid = true;
@@ -511,9 +518,9 @@ int kmb_product_prepare_f32(const float* x, const float* y, int64_t N, int64_t M
     if (!x || !y) return set_error(KMB_ERR_INVALID, "x and y must not be NULL");
     if (N == 0) return KMB_OK;
     const int p = resolve_path(D, 1, kernel_id, path);   // (D <= 16 under KMB_PATH_AUTO: the signal width decides at query time)
-    if (p != KMB_PATH_TENSOR_3XF16) return KMB_OK;   // nothing worth keeping on the other paths
+    if (p != KMB_PATH_TENSOR_3XF16 && p != KMB_PATH_TENSOR_1XF16) return KMB_OK;   // nothing worth keeping on the other paths
     if (reinterpret_cast<uintptr_t>(workspace) % 256) return set_error(KMB_ERR_INVALID, "workspace must be 256-byte aligned");
-    return tensor_prepare(x, y, N, M, D, kernel_id, 1, workspace, workspace_bytes, static_cast<cudaStream_t>(stream_));
+    return tensor_prepare(x, y, N, M, D, kernel_id, tensor_elt(p), workspace, workspace_bytes, static_cast<cudaStream_t>(stream_));
 }
 
 int kmb_product_f64(const double* x, const double* y, const double* b, double* out, int64_t N, int64_t M, int D, int E,
@@ -536,7 +543,7 @@ int kmb_debug_plan_waves(int64_t n_tiles, int64_t n_source_blocks, int grid, siz
 
 int kmb_resolved_path(int D, int E, int kernel_id, int path) {
     if (D < 1 || E < 1 || kernel_id < KMB_KERNEL_GAUSSIAN || kernel_id > KMB_KERNEL_DOT_EXPONENTIAL || path < KMB_PATH_AUTO ||
-        path > KMB_PATH_TENSOR_3XF16)
+        path > KMB_PATH_TENSOR_1XF16)
         return -1;
     return resolve_path(D, E, kernel_id, path);
 }
@@ -567,9 +574,9 @@ int kmb_debug_product_plan(int64_t N, int64_t M, int D, int E, int kernel_id, in
         out10[1] = KMB_FAMILY_SYM;
         return KMB_OK;
     }
-    if (p == KMB_PATH_TENSOR_3XTF32 || p == KMB_PATH_TENSOR_3XF16) {
+    if (tensor_elt(p) >= 0) {
         long long t[4];
-        tensor_plan_debug(N, D, E, kernel_id, p == KMB_PATH_TENSOR_3XF16 ? 1 : 0, sms, t);
+        tensor_plan_debug(N, D, E, kernel_id, tensor_elt(p), sms, t);
         out10[1] = t[0];
         out10[6] = t[1];
         out10[7] = t[2];
@@ -610,7 +617,7 @@ int kmb_debug_pv_plan(int64_t N, int64_t M, int D, int E, int kernel_id, int fla
     for (int i = 0; i < KMB_PV_PLAN_FIELDS; ++i) o[i] = -1;
     o[0] = plan[1];
     if (plan[1] == KMB_FAMILY_PV || plan[1] == KMB_FAMILY_PV16 || plan[1] == KMB_FAMILY_PV16_PAIR)
-        if (int rc = tensor_pv_plan_query(N, M, D, E, kernel_id, plan[0] == KMB_PATH_TENSOR_3XF16 ? 1 : 0, sms, smem_optin, o))
+        if (int rc = tensor_pv_plan_query(N, M, D, E, kernel_id, tensor_elt(static_cast<int>(plan[0])), sms, smem_optin, o))
             return rc;
     for (int i = 0; i < KMB_PV_PLAN_FIELDS; ++i) out19[i] = o[i];
     return KMB_OK;

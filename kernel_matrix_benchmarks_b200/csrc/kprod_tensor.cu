@@ -20,6 +20,8 @@
 //             ELT_F16:  the same three-term split with FP16 hi / lo parts of the data scaled by a power of
 //             two (max |operand| in [2^13, 2^15)): 22 significand bits as 3xTF32, kind::f16 runs at twice
 //             the TF32 rate and moves half the bytes; 64 halves per K block; S is rescaled in the epilogue.
+//             ELT_F16X1: the hi planes of ELT_F16 alone (KMB_PATH_TENSOR_1XF16): one hi.hi MMA per K step, the lo
+//             planes neither loaded nor counted on the barrier: 11 significand bits per operand, float16-class S.
 #include <algorithm>
 #include <cstdlib>
 
@@ -54,7 +56,7 @@ struct Params {
     float* out;          // (N, E)
     float* partial;
     int* tile_counter;
-    const float* sscale; // ELT_F16: S = sscale[1] * accumulator (2^-2p); unused for TF32
+    const float* sscale; // FP16 planes: S = sscale[1] * accumulator (2^-2p); unused for TF32
     long long N, M, row_offset;
     int E, e0;
     int n_tiles, nsb, kblocks, ksteps_last;
@@ -135,7 +137,9 @@ kprod_tensor_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_con
         // ------------------------------------ TMA producer ------------------------------------
         // all 32 lanes walk the loop (uniform control flow); one elected lane issues (see elect_one)
         {
-            constexpr int TKE = ELT == ELT_F16 ? 64 : 32;   // elements per 128-byte K block
+            constexpr int TKE = ELT == ELT_TF32 ? 32 : 64;   // elements per 128-byte K block
+            constexpr bool LO = ELT != ELT_F16X1;             // the lo planes take part
+            constexpr uint32_t TX_BYTES = LO ? STAGE_BYTES : TILE_BYTES + B_TILE_BYTES;
             uint32_t it = 0;
             WaveWork ww;
             for (int w = 0; w < P.W; ++w) {
@@ -148,11 +152,11 @@ kprod_tensor_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_con
                         mbar_wait(&empty_bar[stage], ((it / STAGES) & 1) ^ 1);
                         unsigned char* st = stages + stage * STAGE_BYTES;
                         if (elect_one()) {
-                            mbar_arrive_expect_tx(&full_bar[stage], STAGE_BYTES);
+                            mbar_arrive_expect_tx(&full_bar[stage], TX_BYTES);
                             tma_load_2d(st + 0 * TILE_BYTES, &map_ah, kb * TKE, row0, &full_bar[stage]);
-                            tma_load_2d(st + 1 * TILE_BYTES, &map_al, kb * TKE, row0, &full_bar[stage]);
+                            if constexpr (LO) tma_load_2d(st + 1 * TILE_BYTES, &map_al, kb * TKE, row0, &full_bar[stage]);
                             tma_load_2d(st + 2 * TILE_BYTES, &map_bh, kb * TKE, src0, &full_bar[stage]);
-                            tma_load_2d(st + 2 * TILE_BYTES + B_TILE_BYTES, &map_bl, kb * TKE, src0, &full_bar[stage]);
+                            if constexpr (LO) tma_load_2d(st + 2 * TILE_BYTES + B_TILE_BYTES, &map_bl, kb * TKE, src0, &full_bar[stage]);
                         }
                         __syncwarp();
                     }
@@ -187,7 +191,9 @@ kprod_tensor_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_con
                                     const uint64_t bh = umma_desc_sw128(st + 2 * TILE_BYTES, k * 32);
                                     const uint64_t bl = umma_desc_sw128(st + 2 * TILE_BYTES + B_TILE_BYTES, k * 32);
                                     // three-term split: the two small cross terms first, then hi.hi
-                                    if constexpr (ELT == ELT_F16) {
+                                    if constexpr (ELT == ELT_F16X1) {
+                                        umma_f16(d_tmem, ah, bh, idesc_f16(TN), (kb | k) != 0);
+                                    } else if constexpr (ELT == ELT_F16) {
                                         umma_f16(d_tmem, al, bh, idesc_f16(TN), (kb | k) != 0);
                                         umma_f16(d_tmem, ah, bl, idesc_f16(TN), 1);
                                         umma_f16(d_tmem, ah, bh, idesc_f16(TN), 1);
@@ -213,7 +219,7 @@ kprod_tensor_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_con
         const int lane_group = warp & 3;               // TMEM lanes this warp may access
         const int row_in_tile = lane_group * 32 + lane;
         [[maybe_unused]] float sscale = 1.f;
-        if constexpr (ELT == ELT_F16) sscale = __ldg(P.sscale + 1);
+        if constexpr (ELT != ELT_TF32) sscale = __ldg(P.sscale + 1);
         uint32_t unit = 0;
         WaveWork ww;
         for (int w = 0; w < P.W; ++w) {
@@ -257,7 +263,7 @@ kprod_tensor_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_con
                 for (int ch = 0; ch < TN / 32; ++ch) {
                     float s[32];
                     tmem_ld_32x32(t_addr + ch * 32, s);
-                    if constexpr (ELT == ELT_F16) {
+                    if constexpr (ELT != ELT_TF32) {
 #pragma unroll
                         for (int c = 0; c < 32; ++c) s[c] *= sscale;   // exact: a power of two
                     }
@@ -378,6 +384,8 @@ kprod_tensor_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_con
 //              producer arms it with the bytes of both CTAs, the peer's producer arrives remotely
 //   empty_bar  one per CTA; the leader's tcgen05.commit multicasts to both
 //   acc_full   one per CTA (multicast commit); acc_empty: leader's, 8 arrivals (4 epilogue warps of each CTA)
+// TERMS = 3: lo.hi + hi.lo + hi.hi (KMB_PATH_TENSOR_3XF16); TERMS = 1: hi.hi only, the lo planes are not loaded
+// (KMB_PATH_TENSOR_1XF16).
 namespace pair {
 
 constexpr int STAGES2 = 3;
@@ -409,7 +417,7 @@ __device__ __forceinline__ bool pair_wave_work(const Params& P, int w, int cid, 
     return true;
 }
 
-template <int EP, int KID, bool NORM>
+template <int EP, int KID, bool NORM, int TERMS>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
 kprod_tensor_pair_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant__ CUtensorMap map_al,
                          const __grid_constant__ CUtensorMap map_bh, const __grid_constant__ CUtensorMap map_bl,
@@ -457,12 +465,13 @@ kprod_tensor_pair_kernel(const __grid_constant__ CUtensorMap map_ah, const __gri
                     unsigned char* st = stages + stage * STAGE2_BYTES;
                     const uint32_t leader_full = map_to_cta(&full_bar[stage], 0);
                     if (elect_one()) {
-                        if (rank == 0) mbar_arrive_expect_tx(&full_bar[stage], 2 * STAGE2_BYTES);   // both CTAs' bytes
+                        constexpr uint32_t tx = TERMS == 3 ? STAGE2_BYTES : TILE_BYTES + BH_BYTES;
+                        if (rank == 0) mbar_arrive_expect_tx(&full_bar[stage], 2 * tx);   // both CTAs' bytes
                         else mbar_arrive_cluster(leader_full);
                         tma_load_2d_pair(st + 0 * TILE_BYTES, &map_ah, kb * 64, row0, leader_full);
-                        tma_load_2d_pair(st + 1 * TILE_BYTES, &map_al, kb * 64, row0, leader_full);
+                        if constexpr (TERMS == 3) tma_load_2d_pair(st + 1 * TILE_BYTES, &map_al, kb * 64, row0, leader_full);
                         tma_load_2d_pair(st + 2 * TILE_BYTES, &map_bh, kb * 64, src0, leader_full);
-                        tma_load_2d_pair(st + 2 * TILE_BYTES + BH_BYTES, &map_bl, kb * 64, src0, leader_full);
+                        if constexpr (TERMS == 3) tma_load_2d_pair(st + 2 * TILE_BYTES + BH_BYTES, &map_bl, kb * 64, src0, leader_full);
                     }
                     __syncwarp();
                 }
@@ -494,9 +503,13 @@ kprod_tensor_pair_kernel(const __grid_constant__ CUtensorMap map_ah, const __gri
                                     const uint64_t al = umma_desc_sw128(st + 1 * TILE_BYTES, k * 32);
                                     const uint64_t bh = umma_desc_sw128(st + 2 * TILE_BYTES, k * 32);
                                     const uint64_t bl = umma_desc_sw128(st + 2 * TILE_BYTES + BH_BYTES, k * 32);
-                                    umma2_f16(d_tmem, al, bh, idesc2_f16(), (kb | k) != 0);
-                                    umma2_f16(d_tmem, ah, bl, idesc2_f16(), 1);
-                                    umma2_f16(d_tmem, ah, bh, idesc2_f16(), 1);
+                                    if constexpr (TERMS == 3) {
+                                        umma2_f16(d_tmem, al, bh, idesc2_f16(), (kb | k) != 0);
+                                        umma2_f16(d_tmem, ah, bl, idesc2_f16(), 1);
+                                        umma2_f16(d_tmem, ah, bh, idesc2_f16(), 1);
+                                    } else {
+                                        umma2_f16(d_tmem, ah, bh, idesc2_f16(), (kb | k) != 0);
+                                    }
                                 }
                             }
                             umma2_commit_both(&empty_bar[stage]);   // both CTAs' slots are reusable
@@ -1052,12 +1065,15 @@ size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 // signal columns per pass of kprod_tensor (E = 3 runs on the EP = 4 instantiation, see launch_ep)
 int tensor_e_chunk(int E) { return E >= 4 ? 4 : E; }
 
-// which kernel family tensor_product hands the product to
-enum { KIND_TENSOR, KIND_PV, KIND_PV16 };
+// which kernel family tensor_product hands the product to (KIND_NONE: the one-term path has no TF32 P.B kernel)
+enum { KIND_TENSOR, KIND_PV, KIND_PV16, KIND_NONE };
 int tensor_kind(int D, int E, int kid, int elt) {
-    if (elt == tc::ELT_F16 && tensor_pv16_applicable(D, E, kid)) return KIND_PV16;
-    if (tensor_pv_applicable(D, E)) return KIND_PV;
+    if (elt != tc::ELT_TF32 && tensor_pv16_applicable(D, E, kid)) return KIND_PV16;
+    if (tensor_pv_applicable(D, E)) return elt == tc::ELT_F16X1 ? KIND_NONE : KIND_PV;
     return KIND_TENSOR;
+}
+int kind_unsupported(int D, int E) {
+    return set_error(KMB_ERR_UNSUPPORTED, "the one-term FP16 path has no kernel for this shape (D=%d, E=%d: the TF32 P.B family)", D, E);
 }
 
 struct TensorPlan {
@@ -1070,7 +1086,7 @@ struct TensorPlan {
 };
 
 int plan_tensor(int64_t N, int64_t M, int D, int E, int elt, TensorPlan* pl) {
-    const bool f16 = elt == tc::ELT_F16;
+    const bool f16 = elt != tc::ELT_TF32;
     pl->Dp = f16 ? (D + 15) / 16 * 16 : (D + tc::TK - 1) / tc::TK * tc::TK;
     const int tke = f16 ? 64 : 32;
     pl->kblocks = (pl->Dp + tke - 1) / tke;
@@ -1133,32 +1149,35 @@ int launch_one(const CUtensorMap* maps, const tc::Params& P, int grid, cudaStrea
     return KMB_OK;
 }
 
-template <int EP, int KID, bool NORM>
+template <int EP, int KID, bool NORM, int TERMS>
 int launch_pair_one(const CUtensorMap* maps, const tc::Params& P, int grid, cudaStream_t stream) {
     using C = tc::pair::Cfg2<EP, KID, NORM>;
-    auto fn = tc::pair::kprod_tensor_pair_kernel<EP, KID, NORM>;
+    auto fn = tc::pair::kprod_tensor_pair_kernel<EP, KID, NORM, TERMS>;
     if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(fn), C::SMEM_BYTES)) return rc;
     fn<<<grid, tc::THREADS, C::SMEM_BYTES, stream>>>(maps[0], maps[1], maps[2], maps[3], P);
     KMB_CUDA_CHECK(cudaGetLastError());
     return KMB_OK;
 }
 
-template <int KID, bool NORM>
+template <int KID, bool NORM, int TERMS>
 int launch_pair_ep(int ep, const CUtensorMap* maps, const tc::Params& P, int grid, cudaStream_t stream) {
-    if (ep == 1) return launch_pair_one<1, KID, NORM>(maps, P, grid, stream);
-    if (ep == 2) return launch_pair_one<2, KID, NORM>(maps, P, grid, stream);
-    return launch_pair_one<4, KID, NORM>(maps, P, grid, stream);
+    if (ep == 1) return launch_pair_one<1, KID, NORM, TERMS>(maps, P, grid, stream);
+    if (ep == 2) return launch_pair_one<2, KID, NORM, TERMS>(maps, P, grid, stream);
+    return launch_pair_one<4, KID, NORM, TERMS>(maps, P, grid, stream);
 }
 
+// TERMS = 1 (one-term path): Gaussian and exponential epilogues only (the inverse distance is rejected by the C ABI)
+template <int TERMS>
 int launch_pair_any(int kid, bool norm, int ep, const CUtensorMap* maps, const tc::Params& P, int grid, cudaStream_t stream) {
     switch (kid * 2 + (norm ? 1 : 0)) {
-        case 0: return launch_pair_ep<KMB_KERNEL_GAUSSIAN, false>(ep, maps, P, grid, stream);
-        case 1: return launch_pair_ep<KMB_KERNEL_GAUSSIAN, true>(ep, maps, P, grid, stream);
-        case 2: return launch_pair_ep<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false>(ep, maps, P, grid, stream);
-        case 3: return launch_pair_ep<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, true>(ep, maps, P, grid, stream);
-        case 4: return launch_pair_ep<KMB_KERNEL_INVERSE_DISTANCE, false>(ep, maps, P, grid, stream);
-        default: return launch_pair_ep<KMB_KERNEL_INVERSE_DISTANCE, true>(ep, maps, P, grid, stream);
+        case 0: return launch_pair_ep<KMB_KERNEL_GAUSSIAN, false, TERMS>(ep, maps, P, grid, stream);
+        case 1: return launch_pair_ep<KMB_KERNEL_GAUSSIAN, true, TERMS>(ep, maps, P, grid, stream);
+        case 2: return launch_pair_ep<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false, TERMS>(ep, maps, P, grid, stream);
+        case 3: return launch_pair_ep<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, true, TERMS>(ep, maps, P, grid, stream);
     }
+    if constexpr (TERMS == 1) return set_error(KMB_ERR_UNSUPPORTED, "no one-term kernel for kernel id %d", kid);
+    else if (norm) return launch_pair_ep<KMB_KERNEL_INVERSE_DISTANCE, true, TERMS>(ep, maps, P, grid, stream);
+    else return launch_pair_ep<KMB_KERNEL_INVERSE_DISTANCE, false, TERMS>(ep, maps, P, grid, stream);
 }
 
 template <int KID, bool NORM, int ELT>
@@ -1175,9 +1194,10 @@ int launch_any(int kid, bool norm, int ep, const CUtensorMap* maps, const tc::Pa
         case 1: return launch_ep<KMB_KERNEL_GAUSSIAN, true, ELT>(ep, maps, P, grid, stream);
         case 2: return launch_ep<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false, ELT>(ep, maps, P, grid, stream);
         case 3: return launch_ep<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, true, ELT>(ep, maps, P, grid, stream);
-        case 4: return launch_ep<KMB_KERNEL_INVERSE_DISTANCE, false, ELT>(ep, maps, P, grid, stream);
-        default: return launch_ep<KMB_KERNEL_INVERSE_DISTANCE, true, ELT>(ep, maps, P, grid, stream);
     }
+    if constexpr (ELT == tc::ELT_F16X1) return set_error(KMB_ERR_UNSUPPORTED, "no one-term kernel for kernel id %d", kid);
+    else if (norm) return launch_ep<KMB_KERNEL_INVERSE_DISTANCE, true, ELT>(ep, maps, P, grid, stream);
+    else return launch_ep<KMB_KERNEL_INVERSE_DISTANCE, false, ELT>(ep, maps, P, grid, stream);
 }
 
 }  // namespace
@@ -1193,8 +1213,14 @@ void tensor_plan_debug(int64_t N, int D, int E, int kid, int elt, int sms, long 
     const long long n_tiles = (N + tc::TM - 1) / tc::TM;
     const int kind = tensor_kind(D, E, kid, elt);
     int chunk;
+    if (kind == KIND_NONE) {
+        out[0] = KMB_FAMILY_UNSUPPORTED;
+        out[1] = out[2] = -1;
+        out[3] = n_tiles;
+        return;
+    }
     if (kind == KIND_TENSOR) {
-        out[0] = (elt == tc::ELT_F16 && tensor_use_pair(n_tiles, sms)) ? KMB_FAMILY_TENSOR_PAIR : KMB_FAMILY_TENSOR;
+        out[0] = (elt != tc::ELT_TF32 && tensor_use_pair(n_tiles, sms)) ? KMB_FAMILY_TENSOR_PAIR : KMB_FAMILY_TENSOR;
         chunk = tensor_e_chunk(E);
     } else if (kind == KIND_PV) {
         out[0] = KMB_FAMILY_PV;
@@ -1223,6 +1249,7 @@ int tensor_pv_plan_query(int64_t N, int64_t M, int D, int E, int kid, int elt, i
 int tensor_workspace_bytes(int64_t N, int64_t M, int D, int E, int kid, int flags, int elt, size_t* bytes) {
     (void)flags;
     const int kind = tensor_kind(D, E, kid, elt);
+    if (kind == KIND_NONE) return kind_unsupported(D, E);
     if (kind == KIND_PV16) return tensor_pv16_workspace_bytes(N, M, D, E, bytes);
     if (kind == KIND_PV) return tensor_pv_workspace_bytes(N, M, D, E, bytes);
     TensorPlan pl{};
@@ -1233,7 +1260,7 @@ int tensor_workspace_bytes(int64_t N, int64_t M, int D, int E, int kid, int flag
 
 int tensor_prepare(const float* x, const float* y, int64_t N, int64_t M, int D, int kid, int elt, void* workspace,
                    size_t workspace_bytes, cudaStream_t stream) {
-    if (elt != tc::ELT_F16) return KMB_OK;
+    if (elt == tc::ELT_TF32) return KMB_OK;
     F16PointsLayout L;
     f16_points_layout(N, M, D, &L);
     if (!workspace || workspace_bytes < L.end)
@@ -1245,8 +1272,9 @@ int tensor_product(const float* x, const float* y, const float* b, float* out, i
                    int kid, int flags, int elt, int64_t row_offset, void* workspace, size_t workspace_bytes,
                    cudaStream_t stream, cudaEvent_t ev0, cudaEvent_t ev1, bool prepared) {
     const int kind = tensor_kind(D, E, kid, elt);
+    if (kind == KIND_NONE) return kind_unsupported(D, E);
     if (kind == KIND_PV16)
-        return tensor_pv16_product(x, y, b, out, N, M, D, E, kid, flags, workspace, workspace_bytes, stream, ev0, ev1, prepared);
+        return tensor_pv16_product(x, y, b, out, N, M, D, E, kid, flags, elt, workspace, workspace_bytes, stream, ev0, ev1, prepared);
     if (kind == KIND_PV)
         return tensor_pv_product(x, y, b, out, N, M, D, E, kid, flags, row_offset, workspace, workspace_bytes, stream, ev0, ev1);
     TensorPlan pl{};
@@ -1255,7 +1283,8 @@ int tensor_product(const float* x, const float* y, const float* b, float* out, i
         return set_error(KMB_ERR_WORKSPACE, "workspace too small: need %zu bytes, got %zu", pl.total, workspace_bytes);
     if (N >= (1ll << 31) - tc::TM || M >= (1ll << 31) - tc::TN)
         return set_error(KMB_ERR_UNSUPPORTED, "tensor path indexes rows with 32-bit TMA coordinates");
-    const bool f16 = elt == tc::ELT_F16;
+    const bool f16 = elt != tc::ELT_TF32;
+    const bool x1 = elt == tc::ELT_F16X1;   // the lo planes are not read: their maps repeat the hi ones
     char* ws = static_cast<char*>(workspace);
     float* center = reinterpret_cast<float*>(ws + pl.off_center);
     float* cpart = reinterpret_cast<float*>(ws + pl.off_cpart);
@@ -1280,10 +1309,10 @@ int tensor_product(const float* x, const float* y, const float* b, float* out, i
             if (int rc = f16_points_prepass(x, y, N, M, D, kid, L, ws, stream)) return rc;
         }
         if (int rc = tc::make_tensor_map_f16(&maps[0], uh, N, pl.Dp, tc::TM)) return rc;
-        if (int rc = tc::make_tensor_map_f16(&maps[1], ul, N, pl.Dp, tc::TM)) return rc;
+        if (int rc = tc::make_tensor_map_f16(&maps[1], x1 ? uh : ul, N, pl.Dp, tc::TM)) return rc;
         // the pair kernel's CTAs each load half a source block (128 rows)
         if (int rc = tc::make_tensor_map_f16(&maps[2], vh, M, pl.Dp, pl.pair ? 128 : tc::TN)) return rc;
-        if (int rc = tc::make_tensor_map_f16(&maps[3], vl, M, pl.Dp, pl.pair ? 128 : tc::TN)) return rc;
+        if (int rc = tc::make_tensor_map_f16(&maps[3], x1 ? vh : vl, M, pl.Dp, pl.pair ? 128 : tc::TN)) return rc;
     } else {
         if (int rc = tc::tensor_prepass(x, y, N, M, D, pl.Dp, kid, center, cpart, static_cast<float*>(uh), static_cast<float*>(ul),
                                         static_cast<float*>(vh), static_cast<float*>(vl), un, vn, stream))
@@ -1321,10 +1350,13 @@ int tensor_product(const float* x, const float* y, const float* b, float* out, i
         P.slots_per_wave = pl.waves.slots_per_wave;
         if (ev0 && pass == pl.n_passes - 1) KMB_CUDA_CHECK(cudaEventRecord(ev0, stream));
         const int ekid = tc::epilogue_kid(kid);
-        if (int rc = pl.pair ? launch_pair_any(ekid, norm, pl.e_chunk, maps, P, grid, stream)
-                 : f16   ? launch_any<tc::ELT_F16>(ekid, norm, pl.e_chunk, maps, P, grid, stream)
-                         : launch_any<tc::ELT_TF32>(ekid, norm, pl.e_chunk, maps, P, grid, stream))
-            return rc;
+        int rc;
+        if (pl.pair) rc = x1 ? launch_pair_any<1>(ekid, norm, pl.e_chunk, maps, P, grid, stream)
+                             : launch_pair_any<3>(ekid, norm, pl.e_chunk, maps, P, grid, stream);
+        else if (x1) rc = launch_any<tc::ELT_F16X1>(ekid, norm, pl.e_chunk, maps, P, grid, stream);
+        else if (f16) rc = launch_any<tc::ELT_F16>(ekid, norm, pl.e_chunk, maps, P, grid, stream);
+        else rc = launch_any<tc::ELT_TF32>(ekid, norm, pl.e_chunk, maps, P, grid, stream);
+        if (rc) return rc;
         if (ev1 && pass == pl.n_passes - 1) KMB_CUDA_CHECK(cudaEventRecord(ev1, stream));
         count_launch();
     }

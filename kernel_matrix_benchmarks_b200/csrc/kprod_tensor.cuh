@@ -8,7 +8,8 @@
 
 namespace kmb {
 
-// elt: 0 = TF32 hi/lo operands (KMB_PATH_TENSOR_3XTF32), 1 = FP16 hi/lo operands (KMB_PATH_TENSOR_3XF16)
+// elt: 0 = TF32 hi/lo operands (KMB_PATH_TENSOR_3XTF32), 1 = FP16 hi/lo operands (KMB_PATH_TENSOR_3XF16),
+//      2 = the FP16 hi operands alone, one MMA term (KMB_PATH_TENSOR_1XF16)
 int tensor_workspace_bytes(int64_t N, int64_t M, int D, int E, int kid, int flags, int elt, size_t* bytes);
 
 // Enqueue the whole tensor-path product on `stream` (prepass + main kernel per signal chunk).

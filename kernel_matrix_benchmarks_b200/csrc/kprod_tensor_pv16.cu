@@ -26,6 +26,9 @@
 // S(0) .. S(SST-1), PV(0), S(SST), PV(1), ..., so the tensor side runs SST - 1 blocks ahead of the epilogue.
 // Work split: the wave schedule of kprod_tensor.cu -- every CTA of a wave walks the SAME source blocks at the same
 // time (all of them when there are at least as many row tiles as CTAs), so v and b blocks come from L2.
+// TERMS = 1 (KMB_PATH_TENSOR_1XF16): S = hi.hi and O_g += P_hi.B_hi, one MMA per K step each.  The lo planes of u, v and
+// the signal are neither loaded nor counted on the barriers, the epilogue writes P hi only and sums the weights as the
+// MMA sees them (P rounded to FP16); the extra K step, the online maximum and the flushes are those of TERMS = 3.
 #include <algorithm>
 #include <cstdlib>
 
@@ -185,13 +188,15 @@ __device__ __forceinline__ float2 neg_log2_kernel2(float2 s_raw, float2 nsscale,
 // 256 rows tall (half as many instructions per row tile -- the issuing warp is what bounds the single-CTA kernel),
 // each CTA streams half of every v block (64 sources) and half of every signal block (32 signal columns), the leader
 // CTA issues, tcgen05.commit multicasts to both CTAs' barriers and the peer's epilogue warps arrive on the leader's.
-template <int KID, bool NORM, bool PAIR>
+template <int KID, bool NORM, bool PAIR, int TERMS>
 __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUtensorMap& map_al, const CUtensorMap& map_bh,
                                           const CUtensorMap& map_bl, const CUtensorMap& map_sh, const CUtensorMap& map_sl,
                                           const CUtensorMap& map_ue, const CUtensorMap& map_ve, const Params& P) {
     constexpr bool XK = extra_k<KID>();                            // the squared norms come out of the tensor cores
     constexpr int SLOT = PAIR ? SLOT_BYTES / 2 : SLOT_BYTES;       // V: hi | lo halves of the slot
     constexpr int PANEL = PAIR ? PANEL_BYTES / 2 : PANEL_BYTES;    // signal: 4 panels (hi 0, hi 1, lo 0, lo 1)
+    constexpr bool LO = TERMS == 3;                                // the lo planes take part
+    static_assert(TERMS == 3 || TERMS == 1, "three-term or one-term split");
     extern __shared__ unsigned char smem_dyn[];
     unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) & ~uintptr_t(1023));
     unsigned char* u_region = smem;                                   // kblocks x [A hi 16 KB | A lo 16 KB] (+ the norm tile)
@@ -265,11 +270,14 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
             mbar_wait(&empty_bar[slot], ring_phase ^ 1u);
             unsigned char* dst = ring + slot * SLOT;
             if (elect_one()) {
-                arm_full(&full_bar[slot], PAIR ? 4u * (P.ebp / 2) * 128u : 4u * PANEL_BYTES);
+                constexpr uint32_t panels = LO ? 4u : 2u;
+                arm_full(&full_bar[slot], PAIR ? panels * (P.ebp / 2) * 128u : panels * PANEL_BYTES);
                 load2d(dst + 0 * PANEL, &map_sh, 0, row0, &full_bar[slot]);
                 load2d(dst + 1 * PANEL, &map_sh, 64, row0, &full_bar[slot]);
-                load2d(dst + 2 * PANEL, &map_sl, 0, row0, &full_bar[slot]);
-                load2d(dst + 3 * PANEL, &map_sl, 64, row0, &full_bar[slot]);
+                if constexpr (LO) {
+                    load2d(dst + 2 * PANEL, &map_sl, 0, row0, &full_bar[slot]);
+                    load2d(dst + 3 * PANEL, &map_sl, 64, row0, &full_bar[slot]);
+                }
             }
             __syncwarp();
             ring_next();
@@ -285,10 +293,10 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
             mbar_wait(u_free, (seg & 1) ^ 1);
             const int my_row0 = (PAIR ? ww.tile * 2 + static_cast<int>(rank) : ww.tile) * TM;
             if (elect_one()) {
-                arm_full(u_full, (P.kblocks * 2 + (XK ? 1 : 0)) * A_TILE_BYTES);
+                arm_full(u_full, (P.kblocks * (LO ? 2 : 1) + (XK ? 1 : 0)) * A_TILE_BYTES);
                 for (int kb = 0; kb < P.kblocks; ++kb) {
                     load2d(u_region + (kb * 2 + 0) * A_TILE_BYTES, &map_ah, kb * 64, my_row0, u_full);
-                    load2d(u_region + (kb * 2 + 1) * A_TILE_BYTES, &map_al, kb * 64, my_row0, u_full);
+                    if constexpr (LO) load2d(u_region + (kb * 2 + 1) * A_TILE_BYTES, &map_al, kb * 64, my_row0, u_full);
                 }
                 if constexpr (XK) load2d(u_extra, &map_ue, 0, my_row0, u_full);
             }
@@ -300,9 +308,9 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
                     unsigned char* dst = ring + slot * SLOT;
                     const int src0 = sb * TNS + (PAIR ? static_cast<int>(rank) * (TNS / 2) : 0);   // pairs: this CTA's 64 sources
                     if (elect_one()) {
-                        arm_full(&full_bar[slot], SLOT);
+                        arm_full(&full_bar[slot], LO ? SLOT : SLOT / 2);
                         load2d(dst, &map_bh, kb * 64, src0, &full_bar[slot]);
-                        load2d(dst + SLOT / 2, &map_bl, kb * 64, src0, &full_bar[slot]);
+                        if constexpr (LO) load2d(dst + SLOT / 2, &map_bl, kb * 64, src0, &full_bar[slot]);
                     }
                     __syncwarp();
                     ring_next();
@@ -371,9 +379,13 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
                     const uint64_t bl = umma_desc_sw128(sg + (2 + panel) * PANEL, koff);
                     const uint32_t a_hi = p_base + g * CPT + kk * 8, a_lo = a_hi + CPT / 2;
                     const uint32_t d_g = d_o + g * MAX_EB;
-                    mma_ts(d_g, a_lo, bh, idesc_o | (kFhSplit ? (1u << 13) : 0u), !(from_zero && kk == 0));   // (-) P_lo . B_hi
-                    mma_ts(d_g, a_hi, bl, idesc_o, 1);
-                    mma_ts(d_g, a_hi, bh, idesc_o, 1);
+                    if constexpr (LO) {
+                        mma_ts(d_g, a_lo, bh, idesc_o | (kFhSplit ? (1u << 13) : 0u), !(from_zero && kk == 0));   // (-) P_lo . B_hi
+                        mma_ts(d_g, a_hi, bl, idesc_o, 1);
+                        mma_ts(d_g, a_hi, bh, idesc_o, 1);
+                    } else {
+                        mma_ts(d_g, a_hi, bh, idesc_o, !(from_zero && kk == 0));
+                    }
                 }
                 commit(&empty_bar[slot]);
                 commit(&pv_done[a]);
@@ -410,9 +422,13 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
                                 const uint64_t al = umma_desc_sw128(at + A_TILE_BYTES, k * 32);
                                 const uint64_t bh = umma_desc_sw128(bt, k * 32);
                                 const uint64_t bl = umma_desc_sw128(bt + SLOT / 2, k * 32);
-                                mma_ss(d_s, al, bh, idesc_s, (kb | k) != 0);
-                                mma_ss(d_s, ah, bl, idesc_s, 1);
-                                mma_ss(d_s, ah, bh, idesc_s, 1);
+                                if constexpr (LO) {
+                                    mma_ss(d_s, al, bh, idesc_s, (kb | k) != 0);
+                                    mma_ss(d_s, ah, bl, idesc_s, 1);
+                                    mma_ss(d_s, ah, bh, idesc_s, 1);
+                                } else {
+                                    mma_ss(d_s, ah, bh, idesc_s, (kb | k) != 0);
+                                }
                             }
                         }
                         commit(&empty_bar[slot]);
@@ -556,6 +572,12 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
                 float2 kacc = make_float2(0.f, 0.f);     // two-level sum of the weights (see kprod_direct.cuh)
                 auto weight = [&](int c, float2 e) {     // exponent -> weight -> planes (2 MUFU.EX2 + 7 instructions)
                     const float2 pw = make_float2(ex2_approx(e.x), ex2_approx(e.y));
+                    if constexpr (!LO) {
+                        // one plane: the row's sum takes the weights the MMA multiplies, P rounded to FP16
+                        ph[c] = pack_half2(pw.x, pw.y);
+                        if constexpr (NORM) kacc = add2(kacc, __half22float2(*reinterpret_cast<const __half2*>(&ph[c])));
+                        return;
+                    }
                     if constexpr (NORM) kacc = add2(kacc, pw);   // the plain product never divides by the sum of the weights
                     if constexpr (kFhSplit) {
                         const uint32_t hi2 = pack_half2(pw.x, pw.y);
@@ -683,7 +705,7 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
                     // the group's P over the thread's own S columns: hi planes in the first half, lo planes in the second
                     const uint32_t p_addr = tmem_base + COL_S + a * TNS + col0 + lane_addr;
                     tmem_st_cols<CPT / 2>(p_addr, reinterpret_cast<const float(&)[CPT / 2]>(ph));
-                    tmem_st_cols<CPT / 2>(p_addr + CPT / 2, reinterpret_cast<const float(&)[CPT / 2]>(pl));
+                    if constexpr (LO) tmem_st_cols<CPT / 2>(p_addr + CPT / 2, reinterpret_cast<const float(&)[CPT / 2]>(pl));
                     ksum += kacc.x + kacc.y;
                 }
                 KMB_T(5);
@@ -810,21 +832,21 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
     }
 }
 
-template <int KID, bool NORM>
+template <int KID, bool NORM, int TERMS>
 __global__ void __launch_bounds__(THREADS, 1)
 kprod_tensor_pv16_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant__ CUtensorMap map_al,
                          const __grid_constant__ CUtensorMap map_bh, const __grid_constant__ CUtensorMap map_bl,
                          const __grid_constant__ CUtensorMap map_sh, const __grid_constant__ CUtensorMap map_sl,
                          const __grid_constant__ CUtensorMap map_ue, const __grid_constant__ CUtensorMap map_ve, const Params P) {
-    pv16_body<KID, NORM, false>(map_ah, map_al, map_bh, map_bl, map_sh, map_sl, map_ue, map_ve, P);
+    pv16_body<KID, NORM, false, TERMS>(map_ah, map_al, map_bh, map_bl, map_sh, map_sl, map_ue, map_ve, P);
 }
-template <int KID, bool NORM>
+template <int KID, bool NORM, int TERMS>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
 kprod_tensor_pv16_pair_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant__ CUtensorMap map_al,
                               const __grid_constant__ CUtensorMap map_bh, const __grid_constant__ CUtensorMap map_bl,
                               const __grid_constant__ CUtensorMap map_sh, const __grid_constant__ CUtensorMap map_sl,
                               const __grid_constant__ CUtensorMap map_ue, const __grid_constant__ CUtensorMap map_ve, const Params P) {
-    pv16_body<KID, NORM, true>(map_ah, map_al, map_bh, map_bl, map_sh, map_sl, map_ue, map_ve, P);
+    pv16_body<KID, NORM, true, TERMS>(map_ah, map_al, map_bh, map_bl, map_sh, map_sl, map_ue, map_ve, P);
 }
 
 // ---- signal planes -----------------------------------------------------------------------------------
@@ -864,7 +886,8 @@ static __global__ void signal_scale_kernel(const float* __restrict__ pmax, int b
 }
 // hi/lo[sb][e][jj] = FP16 hi/lo of 2^q_e b[128 sb + jj][e]: the K-major signal of the P.B contraction, one contiguous
 // (Ep x 128) slab per source block (a TMA box then reads 64 rows of 128 bytes 256 bytes apart, not 64 rows that are
-// 2 Mp bytes apart), zero padded
+// 2 Mp bytes apart), zero padded.  TERMS = 1 writes the hi plane only.
+template <int TERMS>
 static __global__ void transpose_split_signal_f16_kernel(const float* __restrict__ b, long long M, long long Mp, int E, int Ep,
                                                          const float* __restrict__ bscale, __half* __restrict__ hi,
                                                          __half* __restrict__ lo) {
@@ -875,7 +898,7 @@ static __global__ void transpose_split_signal_f16_kernel(const float* __restrict
     const __half h = __float2half_rn(v);
     const long long at = ((j / TNS) * Ep + e) * TNS + (j % TNS);
     hi[at] = h;
-    lo[at] = __float2half_rn(v - __half2float(h));
+    if constexpr (TERMS == 3) lo[at] = __float2half_rn(v - __half2float(h));
 }
 
 // Norm tiles of the extra K step (extra_k): rows of 64 BF16 (one 128-byte swizzle atom wide, 16 columns used).
@@ -980,14 +1003,14 @@ int plan_pv16(int64_t N, int64_t M, int D, int E, Pv16Plan* pl) {
     return plan_pv16_host(N, M, D, E, sms, smem_max, pl);
 }
 
-template <int KID, bool NORM>
+template <int KID, bool NORM, int TERMS>
 int launch_pv16(const CUtensorMap* m, const pv16::Params& P, int grid, int smem, bool pair, cudaStream_t stream) {
     if (pair) {
-        auto fn = pv16::kprod_tensor_pv16_pair_kernel<KID, NORM>;
+        auto fn = pv16::kprod_tensor_pv16_pair_kernel<KID, NORM, TERMS>;
         if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(fn), smem)) return rc;
         fn<<<grid, pv16::THREADS, smem, stream>>>(m[0], m[1], m[2], m[3], m[4], m[5], m[6], m[7], P);
     } else {
-        auto fn = pv16::kprod_tensor_pv16_kernel<KID, NORM>;
+        auto fn = pv16::kprod_tensor_pv16_kernel<KID, NORM, TERMS>;
         if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(fn), smem)) return rc;
         fn<<<grid, pv16::THREADS, smem, stream>>>(m[0], m[1], m[2], m[3], m[4], m[5], m[6], m[7], P);
     }
@@ -1032,7 +1055,7 @@ int tensor_pv16_workspace_bytes(int64_t N, int64_t M, int D, int E, size_t* byte
 }
 
 int tensor_pv16_product(const float* x, const float* y, const float* b, float* out, int64_t N, int64_t M, int D, int E, int kid,
-                        int flags, void* workspace, size_t workspace_bytes, cudaStream_t stream, cudaEvent_t ev0,
+                        int flags, int elt, void* workspace, size_t workspace_bytes, cudaStream_t stream, cudaEvent_t ev0,
                         cudaEvent_t ev1, bool prepared) {
     Pv16Plan pl{};
     if (int rc = plan_pv16(N, M, D, E, &pl)) return rc;
@@ -1046,6 +1069,7 @@ int tensor_pv16_product(const float* x, const float* y, const float* b, float* o
     void *uh = ws + pl.off_uh, *ul = ws + pl.off_ul, *vh = ws + pl.off_vh, *vl = ws + pl.off_vl, *sh = ws + pl.off_sh, *sl = ws + pl.off_sl;
     int* counters = reinterpret_cast<int*>(ws + pl.off_counter);
     const bool norm = flags & KMB_FLAG_NORMALIZE_ROWS;
+    const bool x1 = elt == tc::ELT_F16X1;   // one term: the lo planes are not read, their maps repeat the hi ones
 
     KMB_CUDA_CHECK(cudaMemsetAsync(counters, 0, sizeof(int) * pl.n_tiles, stream));
     if (!prepared) {
@@ -1060,17 +1084,21 @@ int tensor_pv16_product(const float* x, const float* y, const float* b, float* o
         pv16::signal_scale_kernel<<<(pl.Ep + 127) / 128, 128, 0, stream>>>(F(pl.off_bmax), blocks, E, pl.Ep, F(pl.off_bscale), F(pl.off_binv));
         KMB_CUDA_CHECK(cudaGetLastError());
         dim3 g(static_cast<unsigned>((pl.Mp + 255) / 256), pl.Ep);
-        pv16::transpose_split_signal_f16_kernel<<<g, 256, 0, stream>>>(b, M, pl.Mp, E, pl.Ep, F(pl.off_bscale), static_cast<__half*>(sh),
-                                                                        static_cast<__half*>(sl));
+        if (x1)
+            pv16::transpose_split_signal_f16_kernel<1><<<g, 256, 0, stream>>>(b, M, pl.Mp, E, pl.Ep, F(pl.off_bscale),
+                                                                               static_cast<__half*>(sh), static_cast<__half*>(sl));
+        else
+            pv16::transpose_split_signal_f16_kernel<3><<<g, 256, 0, stream>>>(b, M, pl.Mp, E, pl.Ep, F(pl.off_bscale),
+                                                                               static_cast<__half*>(sh), static_cast<__half*>(sl));
         KMB_CUDA_CHECK(cudaGetLastError());
         count_launch(3);
     }
     CUtensorMap maps[8];
     if (int rc = tc::make_tensor_map_f16(&maps[0], uh, N, pl.Dp, tc::TM)) return rc;
-    if (int rc = tc::make_tensor_map_f16(&maps[1], ul, N, pl.Dp, tc::TM)) return rc;
+    if (int rc = tc::make_tensor_map_f16(&maps[1], x1 ? uh : ul, N, pl.Dp, tc::TM)) return rc;
     // CTA pairs: each CTA loads 64 of a block's 128 sources and half of the pass's signal columns
     if (int rc = tc::make_tensor_map_f16(&maps[2], vh, M, pl.Dp, pl.pair ? pv16::TNS / 2 : pv16::TNS)) return rc;
-    if (int rc = tc::make_tensor_map_f16(&maps[3], vl, M, pl.Dp, pl.pair ? pv16::TNS / 2 : pv16::TNS)) return rc;
+    if (int rc = tc::make_tensor_map_f16(&maps[3], x1 ? vh : vl, M, pl.Dp, pl.pair ? pv16::TNS / 2 : pv16::TNS)) return rc;
     const int ekid = tc::epilogue_kid(kid);   // dot-exponential: the Gaussian instantiations
     const bool xk = (ekid == KMB_KERNEL_GAUSSIAN) ? pv16::extra_k<KMB_KERNEL_GAUSSIAN>() : pv16::extra_k<KMB_KERNEL_ABSOLUTE_EXPONENTIAL>();
     if (xk) {   // |u|^2, |v|^2 as operands of one more K step (16-bit elements: the FP16 map serves BF16 rows as well)
@@ -1107,7 +1135,7 @@ int tensor_pv16_product(const float* x, const float* y, const float* b, float* o
         {
             const int box_rows = pl.pair ? P.ebp / 2 : pv16::MAX_EB;
             if (int rc = tc::make_tensor_map_f16(&maps[4], sh, pl.nsb * pl.Ep, pv16::TNS, box_rows)) return rc;
-            if (int rc = tc::make_tensor_map_f16(&maps[5], sl, pl.nsb * pl.Ep, pv16::TNS, box_rows)) return rc;
+            if (int rc = tc::make_tensor_map_f16(&maps[5], x1 ? sh : sl, pl.nsb * pl.Ep, pv16::TNS, box_rows)) return rc;
         }
         P.n_tiles = static_cast<int>(pl.n_tiles);
         P.nsb = static_cast<int>(pl.nsb);
@@ -1124,11 +1152,15 @@ int tensor_pv16_product(const float* x, const float* y, const float* b, float* o
         P.slots_per_wave = pl.waves.slots_per_wave;
         if (ev0 && pass == n_passes - 1) KMB_CUDA_CHECK(cudaEventRecord(ev0, stream));
         int rc;
-        switch (ekid * 2 + (norm ? 1 : 0)) {
-            case 0: rc = launch_pv16<KMB_KERNEL_GAUSSIAN, false>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
-            case 1: rc = launch_pv16<KMB_KERNEL_GAUSSIAN, true>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
-            case 2: rc = launch_pv16<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
-            default: rc = launch_pv16<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, true>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
+        switch (ekid * 4 + (norm ? 2 : 0) + (x1 ? 1 : 0)) {
+            case 0: rc = launch_pv16<KMB_KERNEL_GAUSSIAN, false, 3>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
+            case 1: rc = launch_pv16<KMB_KERNEL_GAUSSIAN, false, 1>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
+            case 2: rc = launch_pv16<KMB_KERNEL_GAUSSIAN, true, 3>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
+            case 3: rc = launch_pv16<KMB_KERNEL_GAUSSIAN, true, 1>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
+            case 4: rc = launch_pv16<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false, 3>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
+            case 5: rc = launch_pv16<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false, 1>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
+            case 6: rc = launch_pv16<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, true, 3>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
+            default: rc = launch_pv16<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, true, 1>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
         }
         if (rc) return rc;
         if (ev1 && pass == n_passes - 1) KMB_CUDA_CHECK(cudaEventRecord(ev1, stream));

@@ -13,6 +13,7 @@ constexpr int TK = 32;             // floats per K block = one 128-byte swizzle 
 constexpr int UMMA_K = 8;          // TF32: 32 bytes per instruction
 constexpr int ELT_TF32 = 0;        // operand element: TF32 hi / lo planes (fp32 storage)
 constexpr int ELT_F16 = 1;         // FP16 hi / lo planes of power-of-two scaled data (see tensor_prepass_f16)
+constexpr int ELT_F16X1 = 2;       // the hi planes of ELT_F16 alone, one hi.hi MMA term (KMB_PATH_TENSOR_1XF16)
 
 // ---- PTX wrappers ---------------------------------------------------------------------------------
 __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, int c0, int c1, uint64_t* bar) {
@@ -324,8 +325,9 @@ int tensor_pv16_flush_blocks();
 // as tensor_pv_plan_debug, for kprod_tensor_pv16 (PVQ_PAIR: the CTA-pair kernel)
 int tensor_pv16_plan_debug(int64_t N, int64_t M, int D, int E, int sms, int smem_optin, long long out[PVQ_FIELDS]);
 int tensor_pv16_workspace_bytes(int64_t N, int64_t M, int D, int E, size_t* bytes);
+// elt: tc::ELT_F16 (three-term S and P.B) or tc::ELT_F16X1 (hi.hi only; the lo planes are neither loaded nor written)
 int tensor_pv16_product(const float* x, const float* y, const float* b, float* out, int64_t N, int64_t M, int D, int E, int kid,
-                        int flags, void* workspace, size_t workspace_bytes, cudaStream_t stream, cudaEvent_t ev0,
+                        int flags, int elt, void* workspace, size_t workspace_bytes, cudaStream_t stream, cudaEvent_t ev0,
                         cudaEvent_t ev1, bool prepared);
 
 // Head of the workspace of both FP16-plane kernels: everything the prepass writes from the points alone.  The layout

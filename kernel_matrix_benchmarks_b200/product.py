@@ -136,13 +136,14 @@ def prepare_points(x, y, *, kernel="gaussian", path="auto", workspace=None, min_
     later ``kernel_product(..., prepared=token)`` on the same x, y, kernel, path and workspace skips the prepass as long
     as the workspace has not been reallocated since (``token`` is compared with the buffer in use; otherwise the
     product silently does the prepass itself).  No-op (returns None) on the other paths.  The dot-exponential kernel
-    takes the FP16 tensor path at every D, so it is prepared at every D."""
+    takes the FP16 tensor path at every D, so it is prepared at every D, and so is every kernel on "tensor_f16x1"."""
     lib = _lib.load()
     _check_f32("target points", x)
     _check_f32("source points", y, x.shape[1])
     N, D = x.shape
     M = y.shape[0]
-    if (D <= 16 and kernel != "dot-exponential") or _lib.PATH_IDS[path] not in (_lib.PATH_IDS["auto"], _lib.PATH_IDS["tensor_f16"]):
+    three_term = _lib.PATH_IDS[path] in (_lib.PATH_IDS["auto"], _lib.PATH_IDS["tensor_f16"])
+    if path != "tensor_f16x1" and (not three_term or (D <= 16 and kernel != "dot-exponential")):
         return None
     kid, pid = _lib.KERNEL_IDS[kernel], _lib.PATH_IDS[path]
     need = ctypes.c_size_t(0)

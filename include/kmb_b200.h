@@ -291,6 +291,16 @@ int kmb_debug_direct_entry(int table, int index, int32_t* out11);
  * (strip, row tile) segment, units in the segment}; u outside [0, total units) only fills the first three. */
 int kmb_debug_sym_unit(int64_t n, int64_t total_ctas, int64_t u, int64_t* out8);
 
+/* Diagnostics (host logic only, no GPU needed): how kmb_product_sym_f32 would run part `part` of `n_parts` on a device
+ * with `sms` SMs -- the launcher's own geometry and partition (one CTA per SM and part).  out = {row tile rows, sources
+ * per block, TB (source blocks per row tile), units in total, this part's first unit, its end (exclusive), CTAs the part
+ * launches (min(sms, its units); 0 launches no main kernel), strips, strip width in source blocks, first (strip, tile)
+ * segment of the part, its first strip, segments and strips the part meets (0 for an empty part), evaluation forms
+ * enqueued (bit 0: difference form, bit 1: Gaussian product form), 1 if the strip-count cap widened the strips beyond
+ * what the CTA count asks for}.  Errors as kmb_product_sym_workspace_bytes; KMB_ERR_INVALID for sms < 1. */
+#define KMB_SYM_PLAN_FIELDS 15
+int kmb_debug_sym_plan(int64_t n, int D, int kernel_id, int part, int n_parts, int sms, int64_t* out);
+
 /* Number of this library's kernels the last kmb_product_f32 / kmb_cg_* call on this
  * thread launched (bench.py's gpu_launches). */
 int kmb_last_launch_count(void);

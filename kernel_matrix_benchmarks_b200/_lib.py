@@ -85,6 +85,7 @@ SIGNATURES = {
     "kmb_kernel_block_f64": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_void_p]),
     "kmb_debug_plan_waves": (c_int, [c_int64, c_int64, c_int, c_size_t, POINTER(c_int64)]),
     "kmb_debug_sym_unit": (c_int, [c_int64, c_int64, c_int64, POINTER(c_int64)]),
+    "kmb_debug_sym_plan": (c_int, [c_int64, c_int, c_int, c_int, c_int, c_int, POINTER(c_int64)]),
     "kmb_resolved_path": (c_int, [c_int, c_int, c_int, c_int]),
     "kmb_debug_product_plan": (c_int, [c_int64, c_int64, c_int, c_int, c_int, c_int, c_int, c_int, POINTER(c_int64)]),
     "kmb_debug_direct_entry": (c_int, [c_int, c_int, POINTER(c_int32)]),

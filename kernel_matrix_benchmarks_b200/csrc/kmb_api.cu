@@ -54,6 +54,7 @@ int sym_tile_rows();
 int sym_block_sources();
 int sym_grid(int sms, int* grid);
 void sym_geometry(long long n_tiles, long long nsb, long long total_ctas, SymGeom* g);
+long long sym_cta_strip_width(long long nsb, long long total_ctas);
 SymSeg sym_segment_of(const SymGeom& g, long long u);
 int sym_launch(int D, int kernel_id, int form, const SymParams& P, cudaStream_t stream);
 
@@ -215,39 +216,54 @@ struct SymPlan {
     SymGeom geom;
     long long unit_begin, unit_end;   // this part's share of the unit list
     int grid, seg_base, strip_base;
+    int n_segs, n_strips_part;        // (strip, tile) segments and strips this part's units meet (0 for an empty part)
     size_t rowseg_bytes, rowpart_bytes, colpart_bytes, total_bytes;
 };
 
-static int plan_sym(int64_t n, int D, int kernel_id, int part, int n_parts, SymPlan* sp) {
+// Arguments of a symmetric product and the direct kernels whose record layout it reads (host logic only).
+static int sym_check(int D, int kernel_id, int part, int n_parts, DirectChoice* ch) {
     if (!sym_supported(D)) return set_error(KMB_ERR_UNSUPPORTED, "symmetric path supports D <= 3 (got D=%d)", D);
     if (n_parts < 1 || part < 0 || part >= n_parts) return set_error(KMB_ERR_INVALID, "bad part %d of %d", part, n_parts);
     if (kernel_id < KMB_KERNEL_GAUSSIAN || kernel_id > KMB_KERNEL_INVERSE_DISTANCE) return set_error(KMB_ERR_UNSUPPORTED, "unknown kernel id %d", kernel_id);
-    if (int rc = plan_direct(n, n, D, 1, kernel_id, 0, KMB_PATH_DIRECT_F32, &sp->direct)) return rc;
-    for (const FormPlan& f : sp->direct.form)
-        if (f.ent && (f.ent->SB != sym_block_sources() || f.ent->RECV != 2))
+    choose_direct(D, 1, kernel_id, false, KMB_PATH_DIRECT_F32, ch);
+    if (!ch->ent[0]) return set_error(KMB_ERR_UNSUPPORTED, "no direct kernel for D=%d E=1 kernel=%d", D, kernel_id);
+    for (const DirectEntry* e : ch->ent)
+        if (e && (e->SB != sym_block_sources() || e->RECV != 2))
             return set_error(KMB_ERR_UNSUPPORTED, "no 32-byte record layout for D=%d", D);
+    return KMB_OK;
+}
+
+// Host: the strip geometry for sp->grid CTAs per part, this part's share of the unit list and the hand-over buffers.
+static void sym_partition(int64_t n, int part, int n_parts, SymPlan* sp) {
     const long long nsb = (n + sym_block_sources() - 1) / sym_block_sources();
     const long long n_tiles = (n + sym_tile_rows() - 1) / sym_tile_rows();
-    int sms = 0;
-    if (int rc = device_sm_count(&sms)) return rc;
-    if (int rc = sym_grid(sms, &sp->grid)) return rc;
     sym_geometry(n_tiles, nsb, static_cast<long long>(sp->grid) * n_parts, &sp->geom);
     const long long units = sp->geom.strip_prefix[sp->geom.n_strips];
     sp->unit_begin = units * part / n_parts;
     sp->unit_end = units * (part + 1) / n_parts;
-    int n_segs = 1, n_strips_part = 1;
+    sp->n_segs = sp->n_strips_part = 0;
     sp->seg_base = sp->strip_base = 0;
     if (sp->unit_end > sp->unit_begin) {
         const SymSeg first = sym_segment_of(sp->geom, sp->unit_begin), last = sym_segment_of(sp->geom, sp->unit_end - 1);
         sp->seg_base = sp->geom.seg_prefix[first.strip] + first.tile;
         sp->strip_base = first.strip;
-        n_segs = sp->geom.seg_prefix[last.strip] + last.tile - sp->seg_base + 1;
-        n_strips_part = last.strip - first.strip + 1;
+        sp->n_segs = sp->geom.seg_prefix[last.strip] + last.tile - sp->seg_base + 1;
+        sp->n_strips_part = last.strip - first.strip + 1;
     }
     const size_t piece_bytes = static_cast<size_t>(sp->geom.Wb) * sym_block_sources() * 4;
-    sp->rowseg_bytes = align_up(static_cast<size_t>(n_segs) * sym_tile_rows() * 4, 256);
+    sp->rowseg_bytes = align_up(static_cast<size_t>(std::max(sp->n_segs, 1)) * sym_tile_rows() * 4, 256);
     sp->rowpart_bytes = align_up(static_cast<size_t>(sp->grid) * 2 * sym_tile_rows() * 4, 256);
-    sp->colpart_bytes = align_up(static_cast<size_t>(sp->grid + n_strips_part) * piece_bytes, 256);
+    sp->colpart_bytes = align_up(static_cast<size_t>(sp->grid + std::max(sp->n_strips_part, 1)) * piece_bytes, 256);
+}
+
+static int plan_sym(int64_t n, int D, int kernel_id, int part, int n_parts, SymPlan* sp) {
+    DirectChoice ch;
+    if (int rc = sym_check(D, kernel_id, part, n_parts, &ch)) return rc;
+    if (int rc = plan_direct(n, n, D, 1, kernel_id, 0, KMB_PATH_DIRECT_F32, &sp->direct)) return rc;
+    int sms = 0;
+    if (int rc = device_sm_count(&sms)) return rc;
+    if (int rc = sym_grid(sms, &sp->grid)) return rc;
+    sym_partition(n, part, n_parts, sp);
     sp->total_bytes = sp->direct.total_bytes + sp->rowseg_bytes + sp->rowpart_bytes + sp->colpart_bytes;
     return KMB_OK;
 }
@@ -638,6 +654,25 @@ int kmb_debug_sym_unit(int64_t n, int64_t total_ctas, int64_t u, int64_t* out8) 
     out8[5] = sg.jb0 + (u - sg.begin);
     out8[6] = sg.begin;
     out8[7] = sg.len;
+    return KMB_OK;
+}
+
+int kmb_debug_sym_plan(int64_t n, int D, int kernel_id, int part, int n_parts, int sms, int64_t* out) {
+    if (!out || n < 1 || sms < 1) return set_error(KMB_ERR_INVALID, "bad arguments");
+    DirectChoice ch;
+    if (int rc = sym_check(D, kernel_id, part, n_parts, &ch)) return rc;
+    SymPlan sp;
+    sp.grid = sms;   // sym_grid: one CTA per SM
+    sym_partition(n, part, n_parts, &sp);
+    const SymGeom& g = sp.geom;
+    // the strip-count cap binds when it makes the strips wider than the CTA count alone would
+    const bool capped = g.Wb > sym_cta_strip_width(g.nsb, static_cast<long long>(sms) * n_parts);
+    const long long v[KMB_SYM_PLAN_FIELDS] = {sym_tile_rows(), sym_block_sources(), sym_tile_rows() / sym_block_sources(),
+                                              g.strip_prefix[g.n_strips], sp.unit_begin, sp.unit_end,
+                                              std::min<long long>(sms, sp.unit_end - sp.unit_begin), g.n_strips, g.Wb,
+                                              sp.seg_base, sp.strip_base, sp.n_segs, sp.n_strips_part,
+                                              (ch.ent[0] ? 1 : 0) | (ch.ent[1] ? 2 : 0), capped ? 1 : 0};
+    for (int i = 0; i < KMB_SYM_PLAN_FIELDS; ++i) out[i] = v[i];
     return KMB_OK;
 }
 

@@ -52,6 +52,7 @@ int sym_grid(int sms, int* grid) {
 }
 
 void sym_geometry(long long n_tiles, long long nsb, long long total_ctas, SymGeom* g) { sym_build_geom<SymRef::TB>(n_tiles, nsb, total_ctas, g); }
+long long sym_cta_strip_width(long long nsb, long long total_ctas) { return sym_cta_strip_tiles<SymRef::TB>(nsb, total_ctas) * SymRef::TB; }
 SymSeg sym_segment_of(const SymGeom& g, long long u) { return sym_seg_of<SymRef::TB>(g, u); }
 
 // the main kernel over P.unit_begin .. P.unit_end on P.grid CTAs, then the combine kernel.

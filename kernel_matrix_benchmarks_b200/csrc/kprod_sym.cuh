@@ -115,12 +115,19 @@ __host__ __device__ __forceinline__ SymSeg sym_seg_of(const SymGeom& g, long lon
     return sym_seg<TB>(g, s, static_cast<int>(F + k));
 }
 
+// Host: strip width in tiles that `total_ctas` CTAs over all parts ask for (Wb ~ nsb / sqrt(2 G)), before the
+// strip-count cap.
+template <int TB>
+inline long long sym_cta_strip_tiles(long long nsb, long long total_ctas) {
+    double ideal = static_cast<double>(nsb) / sqrt(2.0 * static_cast<double>(total_ctas < 1 ? 1 : total_ctas));
+    long long Wt = static_cast<long long>(ceil(ideal / TB));
+    return Wt < 1 ? 1 : Wt;
+}
+
 // Host: strip width for `total_ctas` CTAs over all parts, prefix tables.
 template <int TB>
 inline void sym_build_geom(long long n_tiles, long long nsb, long long total_ctas, SymGeom* g) {
-    double ideal = static_cast<double>(nsb) / sqrt(2.0 * static_cast<double>(total_ctas < 1 ? 1 : total_ctas));
-    long long Wt = static_cast<long long>(ceil(ideal / TB));
-    if (Wt < 1) Wt = 1;
+    long long Wt = sym_cta_strip_tiles<TB>(nsb, total_ctas);
     const long long min_wt = (n_tiles + SYM_MAX_STRIPS - 1) / SYM_MAX_STRIPS;
     if (Wt < min_wt) Wt = min_wt;
     g->nsb = nsb;

@@ -115,7 +115,23 @@ def pv_plan(N, M, D, E, *, kernel="gaussian", normalize_rows=False, path="auto",
     return plan
 
 
-DIRECT_ENTRY_FIELDS = ("KID", "NORM", "FORM", "DP", "EP", "R", "TILE_ROWS", "SB", "RECV", "PS")
+SYM_PLAN_FIELDS = ("tile_rows", "block_sources", "TB", "units", "unit_begin", "unit_end", "grid", "n_strips", "Wb",
+                   "seg_base", "strip_base", "segments", "strips", "forms", "strip_cap")
+
+
+def sym_plan(n, D, *, kernel="gaussian", part=0, n_parts=1, sms=148):
+    """How kernel_product_sym_part would run part ``part`` of ``n_parts`` on a device with ``sms`` SMs (kmb_debug_sym_plan,
+    the launcher's own geometry and partition; host logic only, no GPU needed): a dict of SYM_PLAN_FIELDS, ``forms`` as
+    the tuple of evaluation forms enqueued ("difference", and "product" for the Gaussian), ``strip_cap`` as a bool."""
+    out = (ctypes.c_int64 * len(SYM_PLAN_FIELDS))()
+    _lib.check(_lib.load().kmb_debug_sym_plan(int(n), int(D), _lib.KERNEL_IDS[kernel], int(part), int(n_parts), int(sms), out))
+    plan = dict(zip(SYM_PLAN_FIELDS, (int(v) for v in out)))
+    plan["forms"] = tuple(name for bit, name in ((1, "difference"), (2, "product")) if plan["forms"] & bit)
+    plan["strip_cap"] = bool(plan["strip_cap"])
+    return plan
+
+
+DIRECT_ENTRY_FIELDS =("KID", "NORM", "FORM", "DP", "EP", "R", "TILE_ROWS", "SB", "RECV", "PS")
 
 
 def direct_entries(table):

@@ -103,13 +103,6 @@ static void choose_direct(int D, int E, int kid, bool norm, int path, DirectChoi
 
 static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-// coordinate scale folded into x and y so the exponential is a bare ex2
-static float coord_scale(int kid) {
-    if (kid == KMB_KERNEL_GAUSSIAN) return 1.2011224087864498f;             // sqrt(log2 e)
-    if (kid == KMB_KERNEL_ABSOLUTE_EXPONENTIAL) return 1.4426950408889634f; // log2 e
-    return 1.0f;
-}
-
 struct FormPlan {   // one evaluation form's kernel and geometry
     const DirectEntry* ent = nullptr;
     long long n_tiles = 0, nsb = 0, M_pad = 0;

@@ -25,6 +25,13 @@ int device_sm_count(int* sms);
                                   __FILE__, __LINE__);                                               \
     } while (0)
 
+// coordinate scale folded into x and y so the exponential is a bare ex2
+__host__ __device__ constexpr float coord_scale(int kid) {
+    if (kid == KMB_KERNEL_GAUSSIAN) return 1.2011224087864498f;             // sqrt(log2 e)
+    if (kid == KMB_KERNEL_ABSOLUTE_EXPONENTIAL) return 1.4426950408889634f; // log2 e
+    return 1.0f;
+}
+
 // ---- PTX helpers ----------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));

@@ -34,17 +34,10 @@ namespace kmb {
 
 namespace tc {
 
-#ifndef KMB_TC_TN
-#define KMB_TC_TN 256
-#endif
-constexpr int TN = KMB_TC_TN;      // sources per tile      (UMMA N, one TMEM column per source): 128 or 256
-static_assert(TN == 128 || TN == 256, "TN");
-constexpr int STAGES = TN == 256 ? 2 : 3;
+constexpr int TN = 256;                        // sources per tile      (UMMA N, one TMEM column per source)
 constexpr int TILE_BYTES = TM * 128;           // 16 KB: one 128-row A tile of 128-byte K blocks
-constexpr int B_TILE_BYTES = TN * 128;         // one TN-row B tile
-constexpr int STAGE_BYTES = 2 * TILE_BYTES + 2 * B_TILE_BYTES;    // A hi, A lo, B hi, B lo
 constexpr int ACC_STAGES = 2;
-constexpr int TMEM_COLS = ACC_STAGES * TN;     // 256 columns of 32-bit
+constexpr int TMEM_COLS = ACC_STAGES * TN;     // 512 columns of 32-bit
 constexpr int EPI_THREADS = 128;
 constexpr int THREADS = 64 + EPI_THREADS;      // producer warp, MMA warp, 4 epilogue warps
 constexpr int MAX_EP = 4;
@@ -63,51 +56,39 @@ struct Params {
     int R, C, W, R_last, C_last, slots_per_wave;   // wave schedule (plan_waves)
 };
 
-// work of CTA `cta` in wave w: row tile, source-block range [sb_lo, sb_hi), range index c of Cw
-struct WaveWork { int tile, sb_lo, sb_hi, c, Cw, tile_in_wave; };
-__device__ __forceinline__ bool wave_work(const Params& P, int w, int cta, WaveWork& ww) {
-    const bool last = (w == P.W - 1);
-    const int Rw = last ? P.R_last : P.R, Cw = last ? P.C_last : P.C;
-    if (cta >= Rw * Cw) return false;
-    ww.Cw = Cw;
-    ww.tile_in_wave = cta / Cw;
-    ww.c = cta - ww.tile_in_wave * Cw;
-    ww.tile = w * P.R + ww.tile_in_wave;
-    ww.sb_lo = static_cast<int>(static_cast<long long>(P.nsb) * ww.c / Cw);
-    ww.sb_hi = static_cast<int>(static_cast<long long>(P.nsb) * (ww.c + 1) / Cw);
-    return true;
-}
-
-__device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "setp.ne.b32 p, %4, 0;\n"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
-        "}\n" ::"r"(tmem_d),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// instruction descriptor: D = F32, A = B = F16, both K-major
-__host__ __device__ constexpr uint32_t idesc_f16(int n) {
-    return (1u << 4) | (static_cast<uint32_t>(n >> 3) << 17) | (static_cast<uint32_t>(TM >> 4) << 24);
-}
-
-template <int EP, int KID, bool NORM>
+// ---- CTA pairs (cta_group::2), FP16 planes -----------------------------------------------------------------
+// The single-CTA kernel fetches 48 KB of operands from L2 per 6 MMAs and runs into the L2 -> SM bandwidth
+// (ncu: 11.6 TB/s, tensor pipe 72 %).  With PAIR, two CTAs on neighbouring SMs work on two adjacent 128-row tiles and the
+// same 256 sources: each loads its own A tile and HALF of the B block, and one tcgen05.mma.cta_group::2 of shape
+// 256 x 256 x 16 (issued by the leader CTA) reads A from both CTAs' shared memory and the two B halves, leaving each
+// CTA its own 128 x 256 accumulator in its own TMEM.  Operand bytes per CTA and K block: 32 KB of A + 32 KB of B
+// (was 32 + 64), and a stage of 64 KB lets three stages fit.
+//   full_bar   leader's; both producers' TMA bytes land on it (cp.async.bulk.tensor ... cta_group::2), the leader's
+//              producer arms it with the bytes of both CTAs, the peer's producer arrives remotely
+//   empty_bar  one per CTA; the leader's tcgen05.commit multicasts to both
+//   acc_full   one per CTA (multicast commit); acc_empty: leader's, 8 arrivals (4 epilogue warps of each CTA)
+template <int EP, int KID, bool NORM, bool PAIR>
 struct Cfg {
     static constexpr bool ONLINE_MAX = NORM && KID != KMB_KERNEL_INVERSE_DISTANCE;
     static constexpr int PS = EP + (NORM ? 1 : 0) + (ONLINE_MAX ? 1 : 0);
+    static constexpr int STAGES = PAIR ? 3 : 2;
+    static constexpr int B_BYTES = (PAIR ? TN / 2 : TN) * 128;     // this CTA's B tile: the source block (pairs: its half)
+    static constexpr int STAGE_BYTES = 2 * TILE_BYTES + 2 * B_BYTES;   // A hi, A lo, B hi, B lo: 96 KB (pairs: 64 KB)
     static constexpr int AUX_FLOATS = TN * (1 + EP);   // |v|^2 and the signal chunk of one source block
     static constexpr int SMEM_BYTES = 1024 /*align slack*/ + STAGES * STAGE_BYTES + 2 * AUX_FLOATS * 4 +
                                       (2 * STAGES + 2 * ACC_STAGES) * 8 + 16;
 };
 
-template <int EP, int KID, bool NORM, int ELT>
-__global__ void __launch_bounds__(THREADS, 1)
-kprod_tensor_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant__ CUtensorMap map_al,
-                    const __grid_constant__ CUtensorMap map_bh, const __grid_constant__ CUtensorMap map_bl,
-                    const Params P) {
-    using C = Cfg<EP, KID, NORM>;
+// The body of both kernels: single CTAs (PAIR = false, any ELT) and CTA pairs (PAIR = true, FP16 planes).  tid is
+// threadIdx.x as the __global__ function reads it: there __launch_bounds__ bounds it by THREADS, which lets the compiler
+// unroll the epilogue's staging loop without a bounds check (a read in this function would only be known below 1024).
+template <int EP, int KID, bool NORM, bool PAIR, int ELT>
+__device__ __forceinline__ void tensor_body(const uint32_t tid, const CUtensorMap& map_ah, const CUtensorMap& map_al,
+                                            const CUtensorMap& map_bh, const CUtensorMap& map_bl, const Params& P) {
+    static_assert(!PAIR || ELT != ELT_TF32, "CTA pairs run FP16 planes");
+    using C = Cfg<EP, KID, NORM, PAIR>;
+    constexpr int STAGES = C::STAGES, STAGE_BYTES = C::STAGE_BYTES;
+    constexpr int NCTA = PAIR ? 2 : 1;
     extern __shared__ unsigned char smem_dyn[];
     unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) & ~uintptr_t(1023));
     unsigned char* stages = smem;
@@ -119,54 +100,73 @@ kprod_tensor_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_con
     uint32_t* tmem_base_smem = reinterpret_cast<uint32_t*>(acc_empty + ACC_STAGES);
     int* s_flag = reinterpret_cast<int*>(tmem_base_smem + 1);
 
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int cta = blockIdx.x;
+    const int warp = tid >> 5, lane = tid & 31;
+    const uint32_t rank = PAIR ? pair::cluster_ctarank() : 0;   // 0 = leader (issues the MMAs), 1 = peer
+    const int cta = PAIR ? static_cast<int>(blockIdx.x >> 1) : static_cast<int>(blockIdx.x);   // unit of the wave plan
 
     if (tid == 0) {
-        for (int s = 0; s < STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
-        for (int a = 0; a < ACC_STAGES; ++a) { mbar_init(&acc_full[a], 1); mbar_init(&acc_empty[a], EPI_THREADS / 32); }
+        for (int s = 0; s < STAGES; ++s) { mbar_init(&full_bar[s], NCTA); mbar_init(&empty_bar[s], 1); }
+        for (int a = 0; a < ACC_STAGES; ++a) { mbar_init(&acc_full[a], 1); mbar_init(&acc_empty[a], NCTA * (EPI_THREADS / 32)); }
         fence_mbar_init();
     }
-    if (warp == 1) tmem_alloc(tmem_base_smem, TMEM_COLS);
+    if (warp == 1) {
+        if constexpr (PAIR) pair::tmem_alloc2(tmem_base_smem, TMEM_COLS);
+        else tmem_alloc(tmem_base_smem, TMEM_COLS);
+    }
     tc_fence_before();
     __syncthreads();
+    if constexpr (PAIR) pair::cluster_sync_all();   // the peer's barriers are initialised before anything arrives on them
     tc_fence_after();
     const uint32_t tmem_base = *tmem_base_smem;
 
     if (warp == 0) {
-        // ------------------------------------ TMA producer ------------------------------------
+        // ------------------------------------ TMA producer (pairs: both CTAs) ------------------------------------
         // all 32 lanes walk the loop (uniform control flow); one elected lane issues (see elect_one)
-        {
-            constexpr int TKE = ELT == ELT_TF32 ? 32 : 64;   // elements per 128-byte K block
-            constexpr bool LO = ELT != ELT_F16X1;             // the lo planes take part
-            constexpr uint32_t TX_BYTES = LO ? STAGE_BYTES : TILE_BYTES + B_TILE_BYTES;
-            uint32_t it = 0;
-            WaveWork ww;
-            for (int w = 0; w < P.W; ++w) {
-                if (!wave_work(P, w, cta, ww)) continue;
-                const int row0 = ww.tile * TM;
-                for (int sb = ww.sb_lo; sb < ww.sb_hi; ++sb) {
-                    const int src0 = sb * TN;
-                    for (int kb = 0; kb < P.kblocks; ++kb, ++it) {
-                        const int stage = it % STAGES;
-                        mbar_wait(&empty_bar[stage], ((it / STAGES) & 1) ^ 1);
-                        unsigned char* st = stages + stage * STAGE_BYTES;
-                        if (elect_one()) {
-                            mbar_arrive_expect_tx(&full_bar[stage], TX_BYTES);
-                            tma_load_2d(st + 0 * TILE_BYTES, &map_ah, kb * TKE, row0, &full_bar[stage]);
-                            if constexpr (LO) tma_load_2d(st + 1 * TILE_BYTES, &map_al, kb * TKE, row0, &full_bar[stage]);
-                            tma_load_2d(st + 2 * TILE_BYTES, &map_bh, kb * TKE, src0, &full_bar[stage]);
-                            if constexpr (LO) tma_load_2d(st + 2 * TILE_BYTES + B_TILE_BYTES, &map_bl, kb * TKE, src0, &full_bar[stage]);
-                        }
-                        __syncwarp();
+        constexpr int TKE = ELT == ELT_TF32 ? 32 : 64;   // elements per 128-byte K block
+        constexpr bool LO = ELT != ELT_F16X1;             // the lo planes take part
+        constexpr uint32_t TX_BYTES = LO ? STAGE_BYTES : TILE_BYTES + C::B_BYTES;   // per CTA
+        uint32_t it = 0;
+        WaveWork ww;
+        for (int w = 0; w < P.W; ++w) {
+            if (!wave_work(P, w, cta, ww)) continue;
+            const int row0 = (PAIR ? ww.tile * 2 + static_cast<int>(rank) : ww.tile) * TM;
+            for (int sb = ww.sb_lo; sb < ww.sb_hi; ++sb) {
+                const int src0 = sb * TN + (PAIR ? static_cast<int>(rank) * (TN / 2) : 0);   // pairs: this CTA's half
+                for (int kb = 0; kb < P.kblocks; ++kb, ++it) {
+                    const int stage = it % STAGES;
+                    mbar_wait(&empty_bar[stage], ((it / STAGES) & 1) ^ 1);
+                    unsigned char* st = stages + stage * STAGE_BYTES;
+                    [[maybe_unused]] const uint32_t leader_full = PAIR ? pair::map_to_cta(&full_bar[stage], 0) : 0;
+                    auto load = [&](void* dst, const CUtensorMap* map, int row) {
+                        if constexpr (PAIR) pair::tma_load_2d_pair(dst, map, kb * TKE, row, leader_full);
+                        else tma_load_2d(dst, map, kb * TKE, row, &full_bar[stage]);
+                    };
+                    if (elect_one()) {
+                        if (!PAIR) mbar_arrive_expect_tx(&full_bar[stage], TX_BYTES);
+                        else if (rank == 0) mbar_arrive_expect_tx(&full_bar[stage], 2 * TX_BYTES);   // both CTAs' bytes
+                        else pair::mbar_arrive_cluster(leader_full);
+                        load(st + 0 * TILE_BYTES, &map_ah, row0);
+                        if constexpr (LO) load(st + 1 * TILE_BYTES, &map_al, row0);
+                        load(st + 2 * TILE_BYTES, &map_bh, src0);
+                        if constexpr (LO) load(st + 2 * TILE_BYTES + C::B_BYTES, &map_bl, src0);
                     }
+                    __syncwarp();
                 }
             }
         }
     } else if (warp == 1) {
-        // ------------------------------------- MMA issuer -------------------------------------
+        // ------------------------------------- MMA issuer (pairs: the leader CTA's) -------------------------------------
         // all 32 lanes walk the loop and wait on the barriers; one elected lane issues (see elect_one)
-        {
+        if (!PAIR || rank == 0) {
+            auto mma = [&](uint32_t d, uint64_t a, uint64_t b, uint32_t accumulate) {
+                if constexpr (PAIR) pair::umma2_f16(d, a, b, idesc_f16(TN, 2 * TM), accumulate);
+                else if constexpr (ELT == ELT_TF32) umma_tf32(d, a, b, idesc_tf32(TN), accumulate);
+                else umma_f16(d, a, b, idesc_f16(TN), accumulate);
+            };
+            auto commit = [&](uint64_t* bar) {   // pairs: arrives on the barrier in both CTAs
+                if constexpr (PAIR) pair::umma2_commit_both(bar);
+                else umma_commit(bar);
+            };
             uint32_t it = 0, unit = 0;
             WaveWork ww;
             for (int w = 0; w < P.W; ++w) {
@@ -189,32 +189,27 @@ kprod_tensor_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_con
                                     const uint64_t ah = umma_desc_sw128(st + 0 * TILE_BYTES, k * 32);
                                     const uint64_t al = umma_desc_sw128(st + 1 * TILE_BYTES, k * 32);
                                     const uint64_t bh = umma_desc_sw128(st + 2 * TILE_BYTES, k * 32);
-                                    const uint64_t bl = umma_desc_sw128(st + 2 * TILE_BYTES + B_TILE_BYTES, k * 32);
-                                    // three-term split: the two small cross terms first, then hi.hi
+                                    const uint64_t bl = umma_desc_sw128(st + 2 * TILE_BYTES + C::B_BYTES, k * 32);
                                     if constexpr (ELT == ELT_F16X1) {
-                                        umma_f16(d_tmem, ah, bh, idesc_f16(TN), (kb | k) != 0);
-                                    } else if constexpr (ELT == ELT_F16) {
-                                        umma_f16(d_tmem, al, bh, idesc_f16(TN), (kb | k) != 0);
-                                        umma_f16(d_tmem, ah, bl, idesc_f16(TN), 1);
-                                        umma_f16(d_tmem, ah, bh, idesc_f16(TN), 1);
-                                    } else {
-                                        umma_tf32(d_tmem, al, bh, idesc_tf32(TN), (kb | k) != 0);
-                                        umma_tf32(d_tmem, ah, bl, idesc_tf32(TN), 1);
-                                        umma_tf32(d_tmem, ah, bh, idesc_tf32(TN), 1);
+                                        mma(d_tmem, ah, bh, (kb | k) != 0);
+                                    } else {   // three-term split: the two small cross terms first, then hi.hi
+                                        mma(d_tmem, al, bh, (kb | k) != 0);
+                                        mma(d_tmem, ah, bl, 1);
+                                        mma(d_tmem, ah, bh, 1);
                                     }
                                 }
                             }
-                            umma_commit(&empty_bar[stage]);  // smem slot reusable once these MMAs have read it
+                            commit(&empty_bar[stage]);  // smem slot reusable once these MMAs have read it
                         }
                         __syncwarp();
                     }
-                    if (elect_one()) umma_commit(&acc_full[a]);   // accumulator complete
+                    if (elect_one()) commit(&acc_full[a]);   // accumulator complete
                     __syncwarp();
                 }
             }
         }
     } else {
-        // -------------------------------------- epilogue --------------------------------------
+        // -------------------------------------- epilogue (pairs: both CTAs) --------------------------------------
         const int et = tid - 64;                       // 0..127
         const int lane_group = warp & 3;               // TMEM lanes this warp may access
         const int row_in_tile = lane_group * 32 + lane;
@@ -224,7 +219,7 @@ kprod_tensor_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_con
         WaveWork ww;
         for (int w = 0; w < P.W; ++w) {
             if (!wave_work(P, w, cta, ww)) continue;
-            const int tile = ww.tile;
+            const int tile = PAIR ? ww.tile * 2 + static_cast<int>(rank) : ww.tile;
             const long long row = static_cast<long long>(tile) * TM + row_in_tile;
             const bool row_ok = row < P.N;
             const float un = row_ok ? __ldg(P.un + row) : 0.f;
@@ -304,10 +299,13 @@ kprod_tensor_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_con
                         }
                     }
                 }
-                // accumulator drained: hand the TMEM stage back to the MMA warp
+                // accumulator drained: hand the TMEM stage back to the MMA warp (pairs: the leader's, remotely from the peer)
                 tc_fence_before();
                 __syncwarp();
-                if (lane == 0) mbar_arrive(&acc_empty[a]);
+                if (lane == 0) {
+                    if (PAIR && rank != 0) pair::mbar_arrive_cluster(pair::map_to_cta(&acc_empty[a], 0));
+                    else mbar_arrive(&acc_empty[a]);
+                }
                 // two-level summation (see kprod_direct.cuh)
 #pragma unroll
                 for (int e = 0; e < EP; ++e) tot[e] += acc[e];
@@ -315,312 +313,7 @@ kprod_tensor_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_con
             }
 
             // ------------------------------ write this row tile ------------------------------
-            if (ww.Cw == 1) {
-                if (row_ok) {
-#pragma unroll
-                    for (int e = 0; e < EP; ++e)
-                        if (P.e0 + e < P.E) P.out[row * P.E + P.e0 + e] = NORM ? tot[e] / ktot : tot[e];
-                }
-            } else {
-                // one partial per (wave, CTA); the last CTA of the row tile to arrive adds them in range order
-                const size_t slot0 = static_cast<size_t>(w) * P.slots_per_wave + static_cast<size_t>(ww.tile_in_wave) * ww.Cw;
-                float* mine = P.partial + (slot0 + ww.c) * (TM * C::PS);
-#pragma unroll
-                for (int e = 0; e < EP; ++e) mine[e * TM + row_in_tile] = tot[e];
-                if constexpr (NORM) mine[EP * TM + row_in_tile] = ktot;
-                if constexpr (C::ONLINE_MAX) mine[(EP + 1) * TM + row_in_tile] = kmax;
-                __threadfence();
-                named_bar_sync(2, EPI_THREADS);
-                if (et == 0) {
-                    const int old = atomicAdd(&P.tile_counter[tile], 1);
-                    const int last = (old == ww.Cw - 1);
-                    if (last) P.tile_counter[tile] = 0;
-                    *s_flag = last;
-                }
-                named_bar_sync(2, EPI_THREADS);
-                const bool is_last = *s_flag != 0;
-                named_bar_sync(2, EPI_THREADS);
-                if (is_last && row_ok) {
-                    __threadfence();
-                    float sum[EP], l = 0.f, mx = -INFINITY;
-#pragma unroll
-                    for (int e = 0; e < EP; ++e) sum[e] = 0.f;
-                    if constexpr (C::ONLINE_MAX) {
-                        for (int c = 0; c < ww.Cw; ++c)
-                            mx = fmaxf(mx, __ldcg(P.partial + (slot0 + c) * (TM * C::PS) + (EP + 1) * TM + row_in_tile));
-                    }
-                    for (int c = 0; c < ww.Cw; ++c) {
-                        const float* ps = P.partial + (slot0 + c) * (TM * C::PS);
-                        float wgt = 1.f;
-                        if constexpr (C::ONLINE_MAX) {
-                            const float m = __ldcg(ps + (EP + 1) * TM + row_in_tile);
-                            wgt = (m == -INFINITY) ? 0.f : ex2_approx(m - mx);
-                        }
-#pragma unroll
-                        for (int e = 0; e < EP; ++e) sum[e] = fmaf(wgt, __ldcg(ps + e * TM + row_in_tile), sum[e]);
-                        if constexpr (NORM) l = fmaf(wgt, __ldcg(ps + EP * TM + row_in_tile), l);
-                    }
-#pragma unroll
-                    for (int e = 0; e < EP; ++e)
-                        if (P.e0 + e < P.E) P.out[row * P.E + P.e0 + e] = NORM ? sum[e] / l : sum[e];
-                }
-            }
-        }
-    }
-
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) tmem_dealloc(tmem_base, TMEM_COLS);
-}
-
-// ---- CTA pairs (cta_group::2), FP16 planes -----------------------------------------------------------------
-// The single-CTA kernel above fetches 48 KB of operands from L2 per 6 MMAs and runs into the L2 -> SM bandwidth
-// (ncu: 11.6 TB/s, tensor pipe 72 %).  Here two CTAs on neighbouring SMs work on two adjacent 128-row tiles and the
-// same 256 sources: each loads its own A tile and HALF of the B block, and one tcgen05.mma.cta_group::2 of shape
-// 256 x 256 x 16 (issued by the leader CTA) reads A from both CTAs' shared memory and the two B halves, leaving each
-// CTA its own 128 x 256 accumulator in its own TMEM.  Operand bytes per CTA and K block: 32 KB of A + 32 KB of B
-// (was 32 + 64), and a stage of 64 KB lets three stages fit.
-//   full_bar   leader's; both producers' TMA bytes land on it (cp.async.bulk.tensor ... cta_group::2), the leader's
-//              producer arms it with the bytes of both CTAs, the peer's producer arrives remotely
-//   empty_bar  one per CTA; the leader's tcgen05.commit multicasts to both
-//   acc_full   one per CTA (multicast commit); acc_empty: leader's, 8 arrivals (4 epilogue warps of each CTA)
-// TERMS = 3: lo.hi + hi.lo + hi.hi (KMB_PATH_TENSOR_3XF16); TERMS = 1: hi.hi only, the lo planes are not loaded
-// (KMB_PATH_TENSOR_1XF16).
-namespace pair {
-
-constexpr int STAGES2 = 3;
-constexpr int BH_BYTES = 128 * 128;                      // this CTA's half of a B tile: 128 sources x 128 bytes
-constexpr int STAGE2_BYTES = 2 * TILE_BYTES + 2 * BH_BYTES;   // A hi, A lo, B-half hi, B-half lo = 64 KB
-
-// D = F32, A = B = F16, K-major, M = 256 (two CTAs x 128 rows), N = 256
-__host__ __device__ constexpr uint32_t idesc2_f16() {
-    return (1u << 4) | (static_cast<uint32_t>(TN >> 3) << 17) | (static_cast<uint32_t>(256 >> 4) << 24);
-}
-
-template <int EP, int KID, bool NORM>
-struct Cfg2 {
-    static constexpr int SMEM_BYTES = 1024 + STAGES2 * STAGE2_BYTES + 2 * Cfg<EP, KID, NORM>::AUX_FLOATS * 4 +
-                                      (2 * STAGES2 + 2 * ACC_STAGES) * 8 + 16;
-};
-
-// work of cluster `cid` in wave w (the wave plan counts pairs of row tiles and clusters)
-__device__ __forceinline__ bool pair_wave_work(const Params& P, int w, int cid, WaveWork& ww) {
-    const bool last = (w == P.W - 1);
-    const int Rw = last ? P.R_last : P.R, Cw = last ? P.C_last : P.C;
-    if (cid >= Rw * Cw) return false;
-    ww.Cw = Cw;
-    ww.tile_in_wave = cid / Cw;              // pair of row tiles within the wave
-    ww.c = cid - ww.tile_in_wave * Cw;
-    ww.tile = w * P.R + ww.tile_in_wave;     // pair index
-    ww.sb_lo = static_cast<int>(static_cast<long long>(P.nsb) * ww.c / Cw);
-    ww.sb_hi = static_cast<int>(static_cast<long long>(P.nsb) * (ww.c + 1) / Cw);
-    return true;
-}
-
-template <int EP, int KID, bool NORM, int TERMS>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
-kprod_tensor_pair_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant__ CUtensorMap map_al,
-                         const __grid_constant__ CUtensorMap map_bh, const __grid_constant__ CUtensorMap map_bl,
-                         const Params P) {
-    using C = Cfg<EP, KID, NORM>;
-    extern __shared__ unsigned char smem_dyn[];
-    unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) & ~uintptr_t(1023));
-    unsigned char* stages = smem;
-    float* aux = reinterpret_cast<float*>(smem + STAGES2 * STAGE2_BYTES);
-    uint64_t* full_bar = reinterpret_cast<uint64_t*>(aux + 2 * C::AUX_FLOATS);
-    uint64_t* empty_bar = full_bar + STAGES2;
-    uint64_t* acc_full = empty_bar + STAGES2;
-    uint64_t* acc_empty = acc_full + ACC_STAGES;
-    uint32_t* tmem_base_smem = reinterpret_cast<uint32_t*>(acc_empty + ACC_STAGES);
-    int* s_flag = reinterpret_cast<int*>(tmem_base_smem + 1);
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const uint32_t rank = cluster_ctarank();          // 0 = leader (issues the MMAs), 1 = peer
-    const int cid = blockIdx.x >> 1;
-
-    if (tid == 0) {
-        for (int s = 0; s < STAGES2; ++s) { mbar_init(&full_bar[s], 2); mbar_init(&empty_bar[s], 1); }
-        for (int a = 0; a < ACC_STAGES; ++a) { mbar_init(&acc_full[a], 1); mbar_init(&acc_empty[a], 2 * (EPI_THREADS / 32)); }
-        fence_mbar_init();
-    }
-    if (warp == 1) tmem_alloc2(tmem_base_smem, TMEM_COLS);
-    tc_fence_before();
-    __syncthreads();
-    cluster_sync_all();   // the peer's barriers are initialised before anything arrives on them
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_base_smem;
-
-    if (warp == 0) {
-        // ------------------------------------ TMA producer (both CTAs) ------------------------------------
-        uint32_t it = 0;
-        WaveWork ww;
-        for (int w = 0; w < P.W; ++w) {
-            if (!pair_wave_work(P, w, cid, ww)) continue;
-            const int row0 = (ww.tile * 2 + static_cast<int>(rank)) * TM;
-            for (int sb = ww.sb_lo; sb < ww.sb_hi; ++sb) {
-                const int src0 = sb * TN + static_cast<int>(rank) * 128;   // this CTA's half of the source block
-                for (int kb = 0; kb < P.kblocks; ++kb, ++it) {
-                    const int stage = it % STAGES2;
-                    mbar_wait(&empty_bar[stage], ((it / STAGES2) & 1) ^ 1);
-                    unsigned char* st = stages + stage * STAGE2_BYTES;
-                    const uint32_t leader_full = map_to_cta(&full_bar[stage], 0);
-                    if (elect_one()) {
-                        constexpr uint32_t tx = TERMS == 3 ? STAGE2_BYTES : TILE_BYTES + BH_BYTES;
-                        if (rank == 0) mbar_arrive_expect_tx(&full_bar[stage], 2 * tx);   // both CTAs' bytes
-                        else mbar_arrive_cluster(leader_full);
-                        tma_load_2d_pair(st + 0 * TILE_BYTES, &map_ah, kb * 64, row0, leader_full);
-                        if constexpr (TERMS == 3) tma_load_2d_pair(st + 1 * TILE_BYTES, &map_al, kb * 64, row0, leader_full);
-                        tma_load_2d_pair(st + 2 * TILE_BYTES, &map_bh, kb * 64, src0, leader_full);
-                        if constexpr (TERMS == 3) tma_load_2d_pair(st + 2 * TILE_BYTES + BH_BYTES, &map_bl, kb * 64, src0, leader_full);
-                    }
-                    __syncwarp();
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ------------------------------------- MMA issuer (leader CTA only) -------------------------------------
-        if (rank == 0) {
-            uint32_t it = 0, unit = 0;
-            WaveWork ww;
-            for (int w = 0; w < P.W; ++w) {
-                if (!pair_wave_work(P, w, cid, ww)) continue;
-                for (int sb = ww.sb_lo; sb < ww.sb_hi; ++sb, ++unit) {
-                    const int a = unit % ACC_STAGES;
-                    mbar_wait(&acc_empty[a], ((unit / ACC_STAGES) & 1) ^ 1);
-                    tc_fence_after();
-                    const uint32_t d_tmem = tmem_base + a * TN;
-                    for (int kb = 0; kb < P.kblocks; ++kb, ++it) {
-                        const int stage = it % STAGES2;
-                        mbar_wait(&full_bar[stage], (it / STAGES2) & 1);
-                        tc_fence_after();
-                        const unsigned char* st = stages + stage * STAGE2_BYTES;
-                        const int ksteps = (kb == P.kblocks - 1) ? P.ksteps_last : 4;
-                        if (elect_one()) {
-#pragma unroll
-                            for (int k = 0; k < 4; ++k) {
-                                if (k < ksteps) {
-                                    const uint64_t ah = umma_desc_sw128(st + 0 * TILE_BYTES, k * 32);
-                                    const uint64_t al = umma_desc_sw128(st + 1 * TILE_BYTES, k * 32);
-                                    const uint64_t bh = umma_desc_sw128(st + 2 * TILE_BYTES, k * 32);
-                                    const uint64_t bl = umma_desc_sw128(st + 2 * TILE_BYTES + BH_BYTES, k * 32);
-                                    if constexpr (TERMS == 3) {
-                                        umma2_f16(d_tmem, al, bh, idesc2_f16(), (kb | k) != 0);
-                                        umma2_f16(d_tmem, ah, bl, idesc2_f16(), 1);
-                                        umma2_f16(d_tmem, ah, bh, idesc2_f16(), 1);
-                                    } else {
-                                        umma2_f16(d_tmem, ah, bh, idesc2_f16(), (kb | k) != 0);
-                                    }
-                                }
-                            }
-                            umma2_commit_both(&empty_bar[stage]);   // both CTAs' slots are reusable
-                        }
-                        __syncwarp();
-                    }
-                    if (elect_one()) umma2_commit_both(&acc_full[a]);   // both CTAs' accumulators are complete
-                    __syncwarp();
-                }
-            }
-        }
-    } else {
-        // -------------------------------------- epilogue (both CTAs) --------------------------------------
-        const int et = tid - 64;
-        const int lane_group = warp & 3;
-        const int row_in_tile = lane_group * 32 + lane;
-        const float sscale = __ldg(P.sscale + 1);
-        uint32_t unit = 0;
-        WaveWork ww;
-        for (int w = 0; w < P.W; ++w) {
-            if (!pair_wave_work(P, w, cid, ww)) continue;
-            const int tile = ww.tile * 2 + static_cast<int>(rank);
-            const long long row = static_cast<long long>(tile) * TM + row_in_tile;
-            const bool row_ok = row < P.N;
-            const float un = row_ok ? __ldg(P.un + row) : 0.f;
-            [[maybe_unused]] const long long jz = (P.row_offset + row) % (P.M + 1);
-
-            float tot[EP], ktot = 0.f, kmax = -INFINITY;
-#pragma unroll
-            for (int e = 0; e < EP; ++e) tot[e] = 0.f;
-
-            for (int sb = ww.sb_lo; sb < ww.sb_hi; ++sb, ++unit) {
-                const long long j0 = static_cast<long long>(sb) * TN;
-                float* ax = aux + (unit & 1) * C::AUX_FLOATS;
-#pragma unroll
-                for (int jt = et; jt < TN; jt += EPI_THREADS) {
-                    const long long j = j0 + jt;
-                    const bool live = j < P.M;
-                    ax[jt] = live ? __ldg(P.vn + j) : 1.0e30f;
-#pragma unroll
-                    for (int e = 0; e < EP; ++e) {
-                        float v = 0.f;
-                        if (live && P.e0 + e < P.E) v = P.b ? __ldg(P.b + j * P.E + P.e0 + e) : 1.f;
-                        ax[TN + jt * EP + e] = v;
-                    }
-                }
-                named_bar_sync(1, EPI_THREADS);
-                const int a = unit % ACC_STAGES;
-                mbar_wait(&acc_full[a], (unit / ACC_STAGES) & 1);
-                tc_fence_after();
-                const uint32_t t_addr = tmem_base + a * TN + (static_cast<uint32_t>(lane_group * 32) << 16);
-
-                float acc[EP], ksum = 0.f;
-#pragma unroll
-                for (int e = 0; e < EP; ++e) acc[e] = 0.f;
-#pragma unroll 1
-                for (int ch = 0; ch < TN / 32; ++ch) {
-                    float s[32];
-                    tmem_ld_32x32(t_addr + ch * 32, s);
-#pragma unroll
-                    for (int c = 0; c < 32; ++c) s[c] *= sscale;
-                    if constexpr (!C::ONLINE_MAX) {
-#pragma unroll
-                        for (int c = 0; c < 32; ++c) {
-                            const int jj = ch * 32 + c;
-                            float kv = kernel_from_parts<KID>(s[c], un, ax[jj]);
-                            if constexpr (KID == KMB_KERNEL_INVERSE_DISTANCE)
-                                if (j0 + jj == jz || j0 + jj >= P.M) kv = 0.f;
-#pragma unroll
-                            for (int e = 0; e < EP; ++e) acc[e] = fmaf(kv, ax[TN + jj * EP + e], acc[e]);
-                            if constexpr (NORM) ksum += kv;
-                        }
-                    } else {
-                        float cm = -INFINITY;
-#pragma unroll
-                        for (int c = 0; c < 32; ++c) {
-                            s[c] = log2_kernel_from_parts<KID>(s[c], un, ax[ch * 32 + c]);
-                            cm = fmaxf(cm, s[c]);
-                        }
-                        const float mnew = fmaxf(kmax, cm);
-                        const float sc = (mnew == -INFINITY) ? 1.f : ex2_approx(kmax - mnew);
-                        const float moff = (mnew == -INFINITY) ? 0.f : mnew;
-                        kmax = mnew;
-                        ksum *= sc;
-                        ktot *= sc;
-#pragma unroll
-                        for (int e = 0; e < EP; ++e) { acc[e] *= sc; tot[e] *= sc; }
-#pragma unroll
-                        for (int c = 0; c < 32; ++c) {
-                            const int jj = ch * 32 + c;
-                            const float kv = ex2_approx(s[c] - moff);
-#pragma unroll
-                            for (int e = 0; e < EP; ++e) acc[e] = fmaf(kv, ax[TN + jj * EP + e], acc[e]);
-                            ksum += kv;
-                        }
-                    }
-                }
-                // accumulator drained: tell the leader's MMA warp (remote arrive from the peer)
-                tc_fence_before();
-                __syncwarp();
-                if (lane == 0) {
-                    if (rank != 0) mbar_arrive_cluster(map_to_cta(&acc_empty[a], 0));
-                    else mbar_arrive(&acc_empty[a]);
-                }
-#pragma unroll
-                for (int e = 0; e < EP; ++e) tot[e] += acc[e];
-                ktot += ksum;
-            }
-
-            // ------------------------------ write this row tile ------------------------------
-            if (tile < P.n_tiles) {   // the last pair may hold a ghost tile (odd number of row tiles)
+            if (!PAIR || tile < P.n_tiles) {   // the last pair may hold a ghost tile (odd number of row tiles)
                 if (ww.Cw == 1) {
                     if (row_ok) {
 #pragma unroll
@@ -628,9 +321,10 @@ kprod_tensor_pair_kernel(const __grid_constant__ CUtensorMap map_ah, const __gri
                             if (P.e0 + e < P.E) P.out[row * P.E + P.e0 + e] = NORM ? tot[e] / ktot : tot[e];
                     }
                 } else {
-                    // partial records of one wave: [pair in wave][range c][rank]
-                    const size_t slot0 = static_cast<size_t>(w) * P.slots_per_wave + static_cast<size_t>(ww.tile_in_wave) * ww.Cw * 2 + rank;
-                    float* mine = P.partial + (slot0 + ww.c * 2) * (TM * C::PS);
+                    // one partial per (wave, CTA), [tile in wave][range c] (pairs: [pair in wave][range c][rank]); the last
+                    // CTA of the row tile to arrive adds them in range order
+                    const size_t slot0 = static_cast<size_t>(w) * P.slots_per_wave + static_cast<size_t>(ww.tile_in_wave) * ww.Cw * NCTA + rank;
+                    float* mine = P.partial + (slot0 + ww.c * NCTA) * (TM * C::PS);
 #pragma unroll
                     for (int e = 0; e < EP; ++e) mine[e * TM + row_in_tile] = tot[e];
                     if constexpr (NORM) mine[EP * TM + row_in_tile] = ktot;
@@ -653,10 +347,10 @@ kprod_tensor_pair_kernel(const __grid_constant__ CUtensorMap map_ah, const __gri
                         for (int e = 0; e < EP; ++e) sum[e] = 0.f;
                         if constexpr (C::ONLINE_MAX) {
                             for (int c = 0; c < ww.Cw; ++c)
-                                mx = fmaxf(mx, __ldcg(P.partial + (slot0 + c * 2) * (TM * C::PS) + (EP + 1) * TM + row_in_tile));
+                                mx = fmaxf(mx, __ldcg(P.partial + (slot0 + c * NCTA) * (TM * C::PS) + (EP + 1) * TM + row_in_tile));
                         }
                         for (int c = 0; c < ww.Cw; ++c) {
-                            const float* ps = P.partial + (slot0 + c * 2) * (TM * C::PS);
+                            const float* ps = P.partial + (slot0 + c * NCTA) * (TM * C::PS);
                             float wgt = 1.f;
                             if constexpr (C::ONLINE_MAX) {
                                 const float m = __ldcg(ps + (EP + 1) * TM + row_in_tile);
@@ -677,10 +371,32 @@ kprod_tensor_pair_kernel(const __grid_constant__ CUtensorMap map_ah, const __gri
 
     tc_fence_before();
     __syncthreads();
-    cluster_sync_all();   // neither CTA frees tensor memory (or exits) while the other may still signal it
-    if (warp == 1) tmem_dealloc2(tmem_base, TMEM_COLS);
+    if constexpr (PAIR) pair::cluster_sync_all();   // neither CTA frees tensor memory (or exits) while the other may still signal it
+    if (warp == 1) {
+        if constexpr (PAIR) pair::tmem_dealloc2(tmem_base, TMEM_COLS);
+        else tmem_dealloc(tmem_base, TMEM_COLS);
+    }
 }
 
+template <int EP, int KID, bool NORM, int ELT>
+__global__ void __launch_bounds__(THREADS, 1)
+kprod_tensor_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant__ CUtensorMap map_al,
+                    const __grid_constant__ CUtensorMap map_bh, const __grid_constant__ CUtensorMap map_bl,
+                    const Params P) {
+    tensor_body<EP, KID, NORM, false, ELT>(threadIdx.x, map_ah, map_al, map_bh, map_bl, P);
+}
+
+namespace pair {
+// TERMS = 3: lo.hi + hi.lo + hi.hi (ELT_F16, KMB_PATH_TENSOR_3XF16); TERMS = 1: hi.hi only, the lo planes are not loaded
+// (ELT_F16X1, KMB_PATH_TENSOR_1XF16).
+template <int EP, int KID, bool NORM, int TERMS>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
+kprod_tensor_pair_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant__ CUtensorMap map_al,
+                         const __grid_constant__ CUtensorMap map_bh, const __grid_constant__ CUtensorMap map_bl,
+                         const Params P) {
+    static_assert(TERMS == 3 || TERMS == 1, "three-term or one-term split");
+    tensor_body<EP, KID, NORM, true, TERMS == 3 ? ELT_F16 : ELT_F16X1>(threadIdx.x, map_ah, map_al, map_bh, map_bl, P);
+}
 }  // namespace pair
 
 // ---- prepass ---------------------------------------------------------------------------------------
@@ -738,7 +454,7 @@ static __global__ void __launch_bounds__(256) split_points_kernel(const float* _
 // One warp per point of the dot-exponential kernel: operand = s p (TF32) or s 2^p p (FP16; 2^p = sscale[0]), uncentred and
 // with multiplier 1 on both planes, split into hi + lo; norm2 = 0.  S = s^2 <x, y> = log2(e) <x, y> is then what the
 // Gaussian epilogue's S - |u|^2 - |v|^2 evaluates: the log2 of exp(<x, y>).
-constexpr float kDotScale = 1.2011224087864498f;   // sqrt(log2 e)
+constexpr float kDotScale = coord_scale(KMB_KERNEL_GAUSSIAN);   // sqrt(log2 e)
 template <int ELT>
 static __global__ void __launch_bounds__(256) split_points_dot_kernel(const float* __restrict__ pts, long long n, int D, int Dp,
                                                                       float scale, const float* __restrict__ sscale, void* hi,
@@ -762,8 +478,7 @@ static __global__ void __launch_bounds__(256) split_points_dot_kernel(const floa
     if (lane == 0) norm2[row] = 0.f;
 }
 
-// (rows, cols) fp32 row-major; box = 32 floats x box_rows rows, 128-byte swizzle, out-of-bounds reads as zero
-int make_tensor_map(CUtensorMap* map, const float* base, long long rows, int cols, int box_rows) {
+int make_tensor_map(CUtensorMap* map, int elt, const void* base, long long rows, int cols, int box_rows) {
     using EncodeFn = CUresult (*)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -775,14 +490,17 @@ int make_tensor_map(CUtensorMap* map, const float* base, long long rows, int col
         if (!p || q != cudaDriverEntryPointSuccess) return set_error(KMB_ERR_CUDA, "cuTensorMapEncodeTiled not available");
         enc = reinterpret_cast<EncodeFn>(p);
     }
+    const bool f16 = elt != ELT_TF32;
+    const cuuint32_t esz = f16 ? 2 : 4;
     const cuuint64_t dims[2] = {static_cast<cuuint64_t>(cols), static_cast<cuuint64_t>(rows)};
-    const cuuint64_t strides[1] = {static_cast<cuuint64_t>(cols) * 4};
-    const cuuint32_t box[2] = {static_cast<cuuint32_t>(TK), static_cast<cuuint32_t>(box_rows)};
+    const cuuint64_t strides[1] = {static_cast<cuuint64_t>(cols) * esz};
+    const cuuint32_t box[2] = {128 / esz, static_cast<cuuint32_t>(box_rows)};
     const cuuint32_t estr[2] = {1, 1};
-    const CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), dims, strides, box, estr,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return set_error(KMB_ERR_CUDA, "cuTensorMapEncodeTiled failed with %d", static_cast<int>(r));
+    const CUresult r = enc(map, f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(base),
+                           dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+                           CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS)
+        return set_error(KMB_ERR_CUDA, "cuTensorMapEncodeTiled (%s) failed with %d", f16 ? "f16" : "f32", static_cast<int>(r));
     return KMB_OK;
 }
 
@@ -797,7 +515,7 @@ int tensor_prepass(const float* x, const float* y, int64_t N, int64_t M, int D, 
         return KMB_OK;
     }
     // scale folds log2(e) into the data as in the direct path; the A operand carries the factor 2 of 2 u.v
-    const float scale = kid == KMB_KERNEL_GAUSSIAN ? 1.2011224087864498f : kid == KMB_KERNEL_ABSOLUTE_EXPONENTIAL ? 1.4426950408889634f : 1.f;
+    const float scale = coord_scale(kid);
     const int cblocks = static_cast<int>(std::min<long long>(CENTER_BLOCKS, (M + 7) / 8));
     dim3 g(cblocks, (D + 31) / 32);
     column_sum_kernel<<<g, 256, 0, stream>>>(y, M, D, cpart);
@@ -932,33 +650,10 @@ static __global__ void __launch_bounds__(256) split_points_f16_kernel(const floa
     if (lane == 0) norm2[row] = acc;
 }
 
-int make_tensor_map_f16(CUtensorMap* map, const void* base, long long rows, int cols, int box_rows) {
-    using EncodeFn = CUresult (*)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-    static EncodeFn enc = nullptr;
-    if (!enc) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        KMB_CUDA_CHECK(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q));
-        if (!p || q != cudaDriverEntryPointSuccess) return set_error(KMB_ERR_CUDA, "cuTensorMapEncodeTiled not available");
-        enc = reinterpret_cast<EncodeFn>(p);
-    }
-    const cuuint64_t dims[2] = {static_cast<cuuint64_t>(cols), static_cast<cuuint64_t>(rows)};
-    const cuuint64_t strides[1] = {static_cast<cuuint64_t>(cols) * 2};
-    const cuuint32_t box[2] = {64u, static_cast<cuuint32_t>(box_rows)};
-    const cuuint32_t estr[2] = {1, 1};
-    const CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return set_error(KMB_ERR_CUDA, "cuTensorMapEncodeTiled (f16) failed with %d", static_cast<int>(r));
-    return KMB_OK;
-}
-
 int tensor_prepass_f16(const float* x, const float* y, int64_t N, int64_t M, int D, int Dp16, int kid, float* center,
                        float* stats, float* sscale, void* uh, void* ul, void* vh, void* vl, float* un, float* vn,
                        cudaStream_t stream) {
-    const float scale = kid == KMB_KERNEL_GAUSSIAN ? 1.2011224087864498f : kid == KMB_KERNEL_ABSOLUTE_EXPONENTIAL ? 1.4426950408889634f : 1.f;
+    const float scale = coord_scale(kid);
     const size_t plane = static_cast<size_t>(CENTER_BLOCKS) * D;
     float* ys = stats;
     float* xs = stats + 3 * plane;
@@ -1139,65 +834,38 @@ int plan_tensor(int64_t N, int64_t M, int D, int E, int elt, TensorPlan* pl) {
 
 using KernelFn = void (*)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const tc::Params);
 
-template <int EP, int KID, bool NORM, int ELT>
+// PAIR: the CTA-pair kernel (FP16 planes; ELT_F16 runs TERMS = 3, ELT_F16X1 TERMS = 1), else the single-CTA one
+template <bool PAIR, int EP, int KID, bool NORM, int ELT>
 int launch_one(const CUtensorMap* maps, const tc::Params& P, int grid, cudaStream_t stream) {
-    using C = tc::Cfg<EP, KID, NORM>;
-    auto fn = tc::kprod_tensor_kernel<EP, KID, NORM, ELT>;
-    if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(fn), C::SMEM_BYTES)) return rc;
-    fn<<<grid, tc::THREADS, C::SMEM_BYTES, stream>>>(maps[0], maps[1], maps[2], maps[3], P);
+    constexpr int smem = tc::Cfg<EP, KID, NORM, PAIR>::SMEM_BYTES;
+    KernelFn fn;
+    if constexpr (PAIR) fn = tc::pair::kprod_tensor_pair_kernel<EP, KID, NORM, ELT == tc::ELT_F16X1 ? 1 : 3>;
+    else fn = tc::kprod_tensor_kernel<EP, KID, NORM, ELT>;
+    if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(fn), smem)) return rc;
+    fn<<<grid, tc::THREADS, smem, stream>>>(maps[0], maps[1], maps[2], maps[3], P);
     KMB_CUDA_CHECK(cudaGetLastError());
     return KMB_OK;
 }
 
-template <int EP, int KID, bool NORM, int TERMS>
-int launch_pair_one(const CUtensorMap* maps, const tc::Params& P, int grid, cudaStream_t stream) {
-    using C = tc::pair::Cfg2<EP, KID, NORM>;
-    auto fn = tc::pair::kprod_tensor_pair_kernel<EP, KID, NORM, TERMS>;
-    if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(fn), C::SMEM_BYTES)) return rc;
-    fn<<<grid, tc::THREADS, C::SMEM_BYTES, stream>>>(maps[0], maps[1], maps[2], maps[3], P);
-    KMB_CUDA_CHECK(cudaGetLastError());
-    return KMB_OK;
-}
-
-template <int KID, bool NORM, int TERMS>
-int launch_pair_ep(int ep, const CUtensorMap* maps, const tc::Params& P, int grid, cudaStream_t stream) {
-    if (ep == 1) return launch_pair_one<1, KID, NORM, TERMS>(maps, P, grid, stream);
-    if (ep == 2) return launch_pair_one<2, KID, NORM, TERMS>(maps, P, grid, stream);
-    return launch_pair_one<4, KID, NORM, TERMS>(maps, P, grid, stream);
-}
-
-// TERMS = 1 (one-term path): Gaussian and exponential epilogues only (the inverse distance is rejected by the C ABI)
-template <int TERMS>
-int launch_pair_any(int kid, bool norm, int ep, const CUtensorMap* maps, const tc::Params& P, int grid, cudaStream_t stream) {
-    switch (kid * 2 + (norm ? 1 : 0)) {
-        case 0: return launch_pair_ep<KMB_KERNEL_GAUSSIAN, false, TERMS>(ep, maps, P, grid, stream);
-        case 1: return launch_pair_ep<KMB_KERNEL_GAUSSIAN, true, TERMS>(ep, maps, P, grid, stream);
-        case 2: return launch_pair_ep<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false, TERMS>(ep, maps, P, grid, stream);
-        case 3: return launch_pair_ep<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, true, TERMS>(ep, maps, P, grid, stream);
-    }
-    if constexpr (TERMS == 1) return set_error(KMB_ERR_UNSUPPORTED, "no one-term kernel for kernel id %d", kid);
-    else if (norm) return launch_pair_ep<KMB_KERNEL_INVERSE_DISTANCE, true, TERMS>(ep, maps, P, grid, stream);
-    else return launch_pair_ep<KMB_KERNEL_INVERSE_DISTANCE, false, TERMS>(ep, maps, P, grid, stream);
-}
-
-template <int KID, bool NORM, int ELT>
+template <bool PAIR, int KID, bool NORM, int ELT>
 int launch_ep(int ep, const CUtensorMap* maps, const tc::Params& P, int grid, cudaStream_t stream) {
-    if (ep == 1) return launch_one<1, KID, NORM, ELT>(maps, P, grid, stream);
-    if (ep == 2) return launch_one<2, KID, NORM, ELT>(maps, P, grid, stream);
-    return launch_one<4, KID, NORM, ELT>(maps, P, grid, stream);
+    if (ep == 1) return launch_one<PAIR, 1, KID, NORM, ELT>(maps, P, grid, stream);
+    if (ep == 2) return launch_one<PAIR, 2, KID, NORM, ELT>(maps, P, grid, stream);
+    return launch_one<PAIR, 4, KID, NORM, ELT>(maps, P, grid, stream);
 }
 
-template <int ELT>
+// ELT_F16X1 (one-term path): Gaussian and exponential epilogues only (the inverse distance is rejected by the C ABI)
+template <bool PAIR, int ELT>
 int launch_any(int kid, bool norm, int ep, const CUtensorMap* maps, const tc::Params& P, int grid, cudaStream_t stream) {
     switch (kid * 2 + (norm ? 1 : 0)) {
-        case 0: return launch_ep<KMB_KERNEL_GAUSSIAN, false, ELT>(ep, maps, P, grid, stream);
-        case 1: return launch_ep<KMB_KERNEL_GAUSSIAN, true, ELT>(ep, maps, P, grid, stream);
-        case 2: return launch_ep<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false, ELT>(ep, maps, P, grid, stream);
-        case 3: return launch_ep<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, true, ELT>(ep, maps, P, grid, stream);
+        case 0: return launch_ep<PAIR, KMB_KERNEL_GAUSSIAN, false, ELT>(ep, maps, P, grid, stream);
+        case 1: return launch_ep<PAIR, KMB_KERNEL_GAUSSIAN, true, ELT>(ep, maps, P, grid, stream);
+        case 2: return launch_ep<PAIR, KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false, ELT>(ep, maps, P, grid, stream);
+        case 3: return launch_ep<PAIR, KMB_KERNEL_ABSOLUTE_EXPONENTIAL, true, ELT>(ep, maps, P, grid, stream);
     }
     if constexpr (ELT == tc::ELT_F16X1) return set_error(KMB_ERR_UNSUPPORTED, "no one-term kernel for kernel id %d", kid);
-    else if (norm) return launch_ep<KMB_KERNEL_INVERSE_DISTANCE, true, ELT>(ep, maps, P, grid, stream);
-    else return launch_ep<KMB_KERNEL_INVERSE_DISTANCE, false, ELT>(ep, maps, P, grid, stream);
+    else if (norm) return launch_ep<PAIR, KMB_KERNEL_INVERSE_DISTANCE, true, ELT>(ep, maps, P, grid, stream);
+    else return launch_ep<PAIR, KMB_KERNEL_INVERSE_DISTANCE, false, ELT>(ep, maps, P, grid, stream);
 }
 
 }  // namespace
@@ -1308,20 +976,17 @@ int tensor_product(const float* x, const float* y, const float* b, float* out, i
             f16_points_layout(N, M, D, &L);
             if (int rc = f16_points_prepass(x, y, N, M, D, kid, L, ws, stream)) return rc;
         }
-        if (int rc = tc::make_tensor_map_f16(&maps[0], uh, N, pl.Dp, tc::TM)) return rc;
-        if (int rc = tc::make_tensor_map_f16(&maps[1], x1 ? uh : ul, N, pl.Dp, tc::TM)) return rc;
-        // the pair kernel's CTAs each load half a source block (128 rows)
-        if (int rc = tc::make_tensor_map_f16(&maps[2], vh, M, pl.Dp, pl.pair ? 128 : tc::TN)) return rc;
-        if (int rc = tc::make_tensor_map_f16(&maps[3], x1 ? vh : vl, M, pl.Dp, pl.pair ? 128 : tc::TN)) return rc;
     } else {
         if (int rc = tc::tensor_prepass(x, y, N, M, D, pl.Dp, kid, center, cpart, static_cast<float*>(uh), static_cast<float*>(ul),
                                         static_cast<float*>(vh), static_cast<float*>(vl), un, vn, stream))
             return rc;
-        if (int rc = tc::make_tensor_map(&maps[0], static_cast<float*>(uh), N, pl.Dp, tc::TM)) return rc;
-        if (int rc = tc::make_tensor_map(&maps[1], static_cast<float*>(ul), N, pl.Dp, tc::TM)) return rc;
-        if (int rc = tc::make_tensor_map(&maps[2], static_cast<float*>(vh), M, pl.Dp, tc::TN)) return rc;
-        if (int rc = tc::make_tensor_map(&maps[3], static_cast<float*>(vl), M, pl.Dp, tc::TN)) return rc;
     }
+    // the pair kernel's CTAs each load half a source block (128 rows)
+    const int b_rows = pl.pair ? tc::TN / 2 : tc::TN;
+    if (int rc = tc::make_tensor_map(&maps[0], elt, uh, N, pl.Dp, tc::TM)) return rc;
+    if (int rc = tc::make_tensor_map(&maps[1], elt, x1 ? uh : ul, N, pl.Dp, tc::TM)) return rc;
+    if (int rc = tc::make_tensor_map(&maps[2], elt, vh, M, pl.Dp, b_rows)) return rc;
+    if (int rc = tc::make_tensor_map(&maps[3], elt, x1 ? vh : vl, M, pl.Dp, b_rows)) return rc;
 
     const int grid = pl.grid;
     for (int pass = 0; pass < pl.n_passes; ++pass) {
@@ -1351,11 +1016,11 @@ int tensor_product(const float* x, const float* y, const float* b, float* out, i
         if (ev0 && pass == pl.n_passes - 1) KMB_CUDA_CHECK(cudaEventRecord(ev0, stream));
         const int ekid = tc::epilogue_kid(kid);
         int rc;
-        if (pl.pair) rc = x1 ? launch_pair_any<1>(ekid, norm, pl.e_chunk, maps, P, grid, stream)
-                             : launch_pair_any<3>(ekid, norm, pl.e_chunk, maps, P, grid, stream);
-        else if (x1) rc = launch_any<tc::ELT_F16X1>(ekid, norm, pl.e_chunk, maps, P, grid, stream);
-        else if (f16) rc = launch_any<tc::ELT_F16>(ekid, norm, pl.e_chunk, maps, P, grid, stream);
-        else rc = launch_any<tc::ELT_TF32>(ekid, norm, pl.e_chunk, maps, P, grid, stream);
+        if (pl.pair) rc = x1 ? launch_any<true, tc::ELT_F16X1>(ekid, norm, pl.e_chunk, maps, P, grid, stream)
+                             : launch_any<true, tc::ELT_F16>(ekid, norm, pl.e_chunk, maps, P, grid, stream);
+        else if (x1) rc = launch_any<false, tc::ELT_F16X1>(ekid, norm, pl.e_chunk, maps, P, grid, stream);
+        else if (f16) rc = launch_any<false, tc::ELT_F16>(ekid, norm, pl.e_chunk, maps, P, grid, stream);
+        else rc = launch_any<false, tc::ELT_TF32>(ekid, norm, pl.e_chunk, maps, P, grid, stream);
         if (rc) return rc;
         if (ev1 && pass == pl.n_passes - 1) KMB_CUDA_CHECK(cudaEventRecord(ev1, stream));
         count_launch();

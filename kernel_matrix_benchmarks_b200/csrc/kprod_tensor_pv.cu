@@ -640,12 +640,12 @@ int tensor_pv_product(const float* x, const float* y, const float* b, float* out
         count_launch();
     }
     CUtensorMap maps[6];
-    if (int rc = tc::make_tensor_map(&maps[0], uh, N, pl.Dp, tc::TM)) return rc;
-    if (int rc = tc::make_tensor_map(&maps[1], ul, N, pl.Dp, tc::TM)) return rc;
-    if (int rc = tc::make_tensor_map(&maps[2], vh, M, pl.Dp, pv::TN)) return rc;
-    if (int rc = tc::make_tensor_map(&maps[3], vl, M, pl.Dp, pv::TN)) return rc;
-    if (int rc = tc::make_tensor_map(&maps[4], sh, pl.Ep, static_cast<int>(pl.Mp), pv::MAX_EB)) return rc;
-    if (int rc = tc::make_tensor_map(&maps[5], sl, pl.Ep, static_cast<int>(pl.Mp), pv::MAX_EB)) return rc;
+    if (int rc = tc::make_tensor_map(&maps[0], tc::ELT_TF32, uh, N, pl.Dp, tc::TM)) return rc;
+    if (int rc = tc::make_tensor_map(&maps[1], tc::ELT_TF32, ul, N, pl.Dp, tc::TM)) return rc;
+    if (int rc = tc::make_tensor_map(&maps[2], tc::ELT_TF32, vh, M, pl.Dp, pv::TN)) return rc;
+    if (int rc = tc::make_tensor_map(&maps[3], tc::ELT_TF32, vl, M, pl.Dp, pv::TN)) return rc;
+    if (int rc = tc::make_tensor_map(&maps[4], tc::ELT_TF32, sh, pl.Ep, static_cast<int>(pl.Mp), pv::MAX_EB)) return rc;
+    if (int rc = tc::make_tensor_map(&maps[5], tc::ELT_TF32, sl, pl.Ep, static_cast<int>(pl.Mp), pv::MAX_EB)) return rc;
 
     const int grid = pl.grid_max;
     const int n_passes = pl.Ep / pv::MAX_EB;

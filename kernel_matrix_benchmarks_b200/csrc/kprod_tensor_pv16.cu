@@ -119,34 +119,6 @@ struct Params {
     int R, C, W, R_last, C_last, slots_per_wave;
 };
 
-// `unit`: the CTA (single-CTA kernel) or the cluster (CTA pairs: the wave plan then counts pairs of row tiles)
-struct WaveWork { int tile, sb_lo, sb_hi, c, Cw, tile_in_wave; };
-__device__ __forceinline__ bool wave_work(const Params& P, int w, int cta, WaveWork& ww) {
-    const bool last = (w == P.W - 1);
-    const int Rw = last ? P.R_last : P.R, Cw = last ? P.C_last : P.C;
-    if (cta >= Rw * Cw) return false;
-    ww.Cw = Cw;
-    ww.tile_in_wave = cta / Cw;
-    ww.c = cta - ww.tile_in_wave * Cw;
-    ww.tile = w * P.R + ww.tile_in_wave;
-    ww.sb_lo = static_cast<int>(static_cast<long long>(P.nsb) * ww.c / Cw);
-    ww.sb_hi = static_cast<int>(static_cast<long long>(P.nsb) * (ww.c + 1) / Cw);
-    return true;
-}
-
-__device__ __forceinline__ void umma_f16_ss(uint32_t d, uint64_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
-    asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n}\n" ::"r"(d),
-                 "l"(a), "l"(b), "r"(idesc), "r"(acc)
-                 : "memory");
-}
-__device__ __forceinline__ void umma_f16_ts(uint32_t d, uint32_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
-    asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n}\n" ::"r"(d),
-                 "r"(a), "l"(b), "r"(idesc), "r"(acc)
-                 : "memory");
-}
-__host__ __device__ constexpr uint32_t idesc_f16(int n) {   // D = F32, A = B = F16, K-major
-    return (1u << 4) | (static_cast<uint32_t>(n >> 3) << 17) | (static_cast<uint32_t>(TM >> 4) << 24);
-}
 // two floats -> one 32-bit word of two halves: `even` in bits [0,16), `odd` in bits [16,32)
 __device__ __forceinline__ uint32_t pack_half2(float even, float odd) {
     uint32_t r;
@@ -348,7 +320,7 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
         const uint32_t idesc_o = (1u << 4) | (static_cast<uint32_t>(P.ebp >> 3) << 17) | m_bits;
         auto mma_ss = [&](uint32_t d, uint64_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
             if constexpr (PAIR) pair::umma2_f16(d, a, b, idesc, acc);
-            else umma_f16_ss(d, a, b, idesc, acc);
+            else umma_f16(d, a, b, idesc, acc);
         };
         auto mma_ts = [&](uint32_t d, uint32_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
             if constexpr (PAIR) pair::umma2_f16_ts(d, a, b, idesc, acc);
@@ -1094,11 +1066,11 @@ int tensor_pv16_product(const float* x, const float* y, const float* b, float* o
         count_launch(3);
     }
     CUtensorMap maps[8];
-    if (int rc = tc::make_tensor_map_f16(&maps[0], uh, N, pl.Dp, tc::TM)) return rc;
-    if (int rc = tc::make_tensor_map_f16(&maps[1], x1 ? uh : ul, N, pl.Dp, tc::TM)) return rc;
+    if (int rc = tc::make_tensor_map(&maps[0], tc::ELT_F16, uh, N, pl.Dp, tc::TM)) return rc;
+    if (int rc = tc::make_tensor_map(&maps[1], tc::ELT_F16, x1 ? uh : ul, N, pl.Dp, tc::TM)) return rc;
     // CTA pairs: each CTA loads 64 of a block's 128 sources and half of the pass's signal columns
-    if (int rc = tc::make_tensor_map_f16(&maps[2], vh, M, pl.Dp, pl.pair ? pv16::TNS / 2 : pv16::TNS)) return rc;
-    if (int rc = tc::make_tensor_map_f16(&maps[3], x1 ? vh : vl, M, pl.Dp, pl.pair ? pv16::TNS / 2 : pv16::TNS)) return rc;
+    if (int rc = tc::make_tensor_map(&maps[2], tc::ELT_F16, vh, M, pl.Dp, pl.pair ? pv16::TNS / 2 : pv16::TNS)) return rc;
+    if (int rc = tc::make_tensor_map(&maps[3], tc::ELT_F16, x1 ? vh : vl, M, pl.Dp, pl.pair ? pv16::TNS / 2 : pv16::TNS)) return rc;
     const int ekid = tc::epilogue_kid(kid);   // dot-exponential: the Gaussian instantiations
     const bool xk = (ekid == KMB_KERNEL_GAUSSIAN) ? pv16::extra_k<KMB_KERNEL_GAUSSIAN>() : pv16::extra_k<KMB_KERNEL_ABSOLUTE_EXPONENTIAL>();
     if (xk) {   // |u|^2, |v|^2 as operands of one more K step (16-bit elements: the FP16 map serves BF16 rows as well)
@@ -1108,8 +1080,8 @@ int tensor_pv16_product(const float* x, const float* y, const float* b, float* o
             reinterpret_cast<__nv_bfloat16*>(ws + pl.off_ve));
         KMB_CUDA_CHECK(cudaGetLastError());
         count_launch();
-        if (int rc = tc::make_tensor_map_f16(&maps[6], ws + pl.off_ue, N, 64, tc::TM)) return rc;
-        if (int rc = tc::make_tensor_map_f16(&maps[7], ws + pl.off_ve, pl.Mp, 64, pl.pair ? pv16::TNS / 2 : pv16::TNS)) return rc;
+        if (int rc = tc::make_tensor_map(&maps[6], tc::ELT_F16, ws + pl.off_ue, N, 64, tc::TM)) return rc;
+        if (int rc = tc::make_tensor_map(&maps[7], tc::ELT_F16, ws + pl.off_ve, pl.Mp, 64, pl.pair ? pv16::TNS / 2 : pv16::TNS)) return rc;
     } else {
         maps[6] = maps[0];
         maps[7] = maps[2];
@@ -1134,8 +1106,8 @@ int tensor_pv16_product(const float* x, const float* y, const float* b, float* o
         P.ebp = (P.eb + 31) / 32 * 32;
         {
             const int box_rows = pl.pair ? P.ebp / 2 : pv16::MAX_EB;
-            if (int rc = tc::make_tensor_map_f16(&maps[4], sh, pl.nsb * pl.Ep, pv16::TNS, box_rows)) return rc;
-            if (int rc = tc::make_tensor_map_f16(&maps[5], x1 ? sh : sl, pl.nsb * pl.Ep, pv16::TNS, box_rows)) return rc;
+            if (int rc = tc::make_tensor_map(&maps[4], tc::ELT_F16, sh, pl.nsb * pl.Ep, pv16::TNS, box_rows)) return rc;
+            if (int rc = tc::make_tensor_map(&maps[5], tc::ELT_F16, x1 ? sh : sl, pl.nsb * pl.Ep, pv16::TNS, box_rows)) return rc;
         }
         P.n_tiles = static_cast<int>(pl.n_tiles);
         P.nsb = static_cast<int>(pl.nsb);

@@ -1,5 +1,5 @@
-// Shared pieces of the tensor-core kernels (kprod_tensor.cu, kprod_tensor_pv.cu): tcgen05 / TMA PTX
-// wrappers, UMMA descriptors, kernel functions on (2u.v, |u|^2, |v|^2), the prepass.
+// Shared pieces of the tensor-core kernels (kprod_tensor.cu, kprod_tensor_pv.cu, kprod_tensor_pv16.cu): tcgen05 / TMA
+// PTX wrappers, UMMA descriptors, kernel functions on (2u.v, |u|^2, |v|^2), the prepass, the wave schedule.
 #pragma once
 #include <cuda.h>
 
@@ -58,6 +58,27 @@ __device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint6
         "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
         : "memory");
 }
+__device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "setp.ne.b32 p, %4, 0;\n"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
+        "}\n" ::"r"(tmem_d),
+        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
+// the same with the A operand read from tensor memory
+__device__ __forceinline__ void umma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "setp.ne.b32 p, %4, 0;\n"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n"
+        "}\n" ::"r"(tmem_d),
+        "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
@@ -109,6 +130,10 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(const void* smem_tile, int b
 // instruction descriptor: D = F32, A = B = TF32, both K-major, N >> 3 at [17,23), M >> 4 at [24,29)
 __host__ __device__ constexpr uint32_t idesc_tf32(int n) {
     return (1u << 4) | (2u << 7) | (2u << 10) | (static_cast<uint32_t>(n >> 3) << 17) | (static_cast<uint32_t>(TM >> 4) << 24);
+}
+// D = F32, A = B = F16, both K-major; m = 256 for the MMAs of a CTA pair (two CTAs x 128 rows)
+__host__ __device__ constexpr uint32_t idesc_f16(int n, int m = TM) {
+    return (1u << 4) | (static_cast<uint32_t>(n >> 3) << 17) | (static_cast<uint32_t>(m >> 4) << 24);
 }
 // same MMA with the A operand read from tensor memory (lane = row, one 32-bit column per K element)
 __device__ __forceinline__ void umma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
@@ -253,16 +278,16 @@ __device__ __forceinline__ float log2_kernel_from_parts(float s, float un, float
 // log2 k = S - |u|^2 - |v|^2 is log2 exp(<x, y>) exactly (DESIGN.md, "The dot-exponential kernel").
 __host__ __device__ constexpr int epilogue_kid(int kid) { return kid == KMB_KERNEL_DOT_EXPONENTIAL ? KMB_KERNEL_GAUSSIAN : kid; }
 
-// ---- host helpers shared by both tensor kernels (defined in kprod_tensor.cu) ----------------------
-int make_tensor_map(CUtensorMap* map, const float* base, long long rows, int cols, int box_rows);
+// ---- host helpers shared by the tensor kernels (defined in kprod_tensor.cu) ----------------------
+// (rows, cols) row-major plane of `elt` elements (ELT_TF32: fp32, otherwise FP16); box = one 128-byte swizzle atom of
+// columns (32 floats / 64 halves) x box_rows rows, 128-byte swizzle, out-of-bounds reads as zero
+int make_tensor_map(CUtensorMap* map, int elt, const void* base, long long rows, int cols, int box_rows);
 // centre (column means of y), TF32 hi/lo split of A = 2 s (x - c) and B = s (y - c), squared norms
 int tensor_prepass(const float* x, const float* y, int64_t N, int64_t M, int D, int Dp, int kid, float* center,
                    float* cpart, float* uh, float* ul, float* vh, float* vl, float* un, float* vn, cudaStream_t stream);
 constexpr int CENTER_BLOCKS = 128;
 
-// FP16 operands.  (rows, cols) half row-major; box = 64 halves x box_rows rows, 128-byte swizzle.
-int make_tensor_map_f16(CUtensorMap* map, const void* base, long long rows, int cols, int box_rows);
-// centre (column means of y); p = power of two that brings max |s (point - c)| over x and y into [2^13, 2^14);
+// FP16 operands: centre (column means of y); p = power of two that brings max |s (point - c)| over x and y into [2^13, 2^14);
 // FP16 hi / lo split of A = 2 s 2^p (x - c) and B = s 2^p (y - c) (Dp16 = D rounded up to 16 columns, zero
 // padded), squared norms of s (point - c) in FP32; sscale[0] = 2^p, sscale[1] = 2^-2p (device).
 // stats: 6 * CENTER_BLOCKS * D floats of scratch.
@@ -274,6 +299,23 @@ int tensor_prepass_f16(const float* x, const float* y, int64_t N, int64_t M, int
 // a last wave of R_last x C_last.
 struct WavePlan { int R, C, W, R_last, C_last, slots_per_wave; long long partial_slots; };
 void plan_waves(long long n_tiles, long long nsb, int grid, size_t row_tile_bytes, WavePlan* wp);
+
+// Work of `unit` in wave w: row tile, source-block range [sb_lo, sb_hi), range index c of Cw.  The unit is a CTA, or the
+// cluster of a CTA pair, whose wave plan counts pairs of row tiles (`tile` is then the pair's index).
+struct WaveWork { int tile, sb_lo, sb_hi, c, Cw, tile_in_wave; };
+template <class Params>
+__device__ __forceinline__ bool wave_work(const Params& P, int w, int unit, WaveWork& ww) {
+    const bool last = (w == P.W - 1);
+    const int Rw = last ? P.R_last : P.R, Cw = last ? P.C_last : P.C;
+    if (unit >= Rw * Cw) return false;
+    ww.Cw = Cw;
+    ww.tile_in_wave = unit / Cw;
+    ww.c = unit - ww.tile_in_wave * Cw;
+    ww.tile = w * P.R + ww.tile_in_wave;
+    ww.sb_lo = static_cast<int>(static_cast<long long>(P.nsb) * ww.c / Cw);
+    ww.sb_hi = static_cast<int>(static_cast<long long>(P.nsb) * (ww.c + 1) / Cw);
+    return true;
+}
 
 }  // namespace tc
 

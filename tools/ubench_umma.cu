@@ -19,15 +19,6 @@ constexpr int A_BYTES = 128 * 128;    // 128 rows x one 128-byte swizzle atom
 constexpr int B_BYTES = 256 * 128;
 constexpr int SMEM = 1024 + 2 * A_BYTES + 2 * B_BYTES + 64;
 
-__device__ __forceinline__ void umma_f16(uint32_t d, uint64_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
-    asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n}\n" ::"r"(d),
-                 "l"(a), "l"(b), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void umma_f16_ts(uint32_t d, uint32_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
-    asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n}\n" ::"r"(d),
-                 "r"(a), "l"(b), "r"(idesc), "r"(acc) : "memory");
-}
-
 // traffic: 0 = none; 1 = 4 warps stream tcgen05.ld (x32) from TMEM while the chain runs; 2 = tcgen05.ld + tcgen05.st;
 // 3 = 16 warps of tcgen05.ld + tcgen05.st (the epilogue of kprod_tensor_pv16)
 template <int KIND, bool TS>

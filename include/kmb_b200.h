@@ -58,7 +58,16 @@ enum {
 enum {
     KMB_FLAG_NORMALIZE_ROWS = 1, /* attention: (K @ [b,1])[:, :-1] / [:, -1:]     :139-145 */
     KMB_FLAG_DENSITY = 2,        /* b == 1, E == 1: K.sum(-1)                      :150    */
-    KMB_FLAG_PREPARED = 4        /* the points-only work was done by kmb_product_prepare_f32 on this workspace (below) */
+    KMB_FLAG_PREPARED = 4,       /* the points-only work was done by kmb_product_prepare_f32 on this workspace (below) */
+    KMB_FLAG_CAUSAL = 8          /* causal (autoregressive) product: out[i] = sum_{j <= row_offset + i} k(x_i, y_j) b_j.  Not in
+                                    bruteforce.py (an extension).  NORMALIZE_ROWS divides by sum_{j <= row_offset + i} k,
+                                    DENSITY sums the masked kernel values, NORMALIZE_ROWS | DENSITY still fills ones; rows with
+                                    row_offset + i >= n_sources - 1 see every source, sources beyond row_offset + n_targets - 1
+                                    are never read, and the inverse-distance zeroing rule applies on top of the mask.  Runs on
+                                    KMB_PATH_TENSOR_3XF16 (what KMB_PATH_AUTO resolves to with this flag, at every D): the
+                                    source blocks above the diagonal are not scheduled, only blocks that cross it are masked.
+                                    The other paths, and inverse distance with E > 4, D <= 128 (the TF32 P.B kernel), return
+                                    KMB_ERR_UNSUPPORTED.  kmb_product_f64 supports it on every kernel. */
 };
 
 /* evaluation paths */
@@ -236,8 +245,9 @@ int kmb_kernel_block_f64(const double* x, const double* y, double* out, int64_t 
  * [n_source_blocks (b % C) / C, n_source_blocks (b % C + 1) / C). */
 int kmb_debug_plan_waves(int64_t n_tiles, int64_t n_source_blocks, int grid, size_t row_tile_bytes, int64_t* out7);
 
-/* The path KMB_PATH_AUTO stands for with this D, E and kernel (any other `path`, KMB_PATH_TENSOR_1XF16 included, is returned
- * unchanged; -1 on bad arguments):
+/* The path KMB_PATH_AUTO stands for with this D, E and kernel in a product without KMB_FLAG_CAUSAL (which resolves to
+ * KMB_PATH_TENSOR_3XF16 at every D; any other `path`, KMB_PATH_TENSOR_1XF16 included, is returned unchanged; -1 on bad
+ * arguments):
  * D > 16 -> KMB_PATH_TENSOR_3XF16; D <= 16 -> KMB_PATH_DIRECT_F32, except wide signals (E >= 32) of the Gaussian /
  * exponential kernels, whose K b is a dense contraction and runs on the tensor cores as well.  The dot-exponential
  * kernel resolves to KMB_PATH_TENSOR_3XF16 at every D.  Host logic only. */
@@ -278,6 +288,18 @@ int kmb_debug_product_plan(int64_t n_targets, int64_t n_sources, int D, int E, i
 #define KMB_PV_PLAN_FIELDS 19
 int kmb_debug_pv_plan(int64_t n_targets, int64_t n_sources, int D, int E, int kernel_id, int flags, int path, int sms,
                       int smem_optin, int64_t* out19);
+
+/* Diagnostics (host logic only, no GPU needed): the work of unit `unit` (a CTA, or a cluster of two for the CTA-pair kernels)
+ * in wave `wave` of the causal kernel that kmb_product_f32 would launch for this problem (flags must hold
+ * KMB_FLAG_CAUSAL) on a device with `sms` SMs and `smem_optin` bytes of opt-in shared memory per block.
+ * out9 = {family (KMB_FAMILY_*), waves, units per wave, sources per block, row tile (CTA pairs: the index of the pair of
+ * row tiles), first source block, end source block (exclusive), range index, ranges of the tile in this wave}; the last
+ * five are -1 when the unit has no row tile in that wave.  The ranges of a tile cover the blocks its last row can see,
+ * [0, min(blocks, (row_offset + last row) / block + 1)), and may be empty; the tiles of odd waves run in reverse order.
+ * Errors as kmb_product_workspace_bytes. */
+#define KMB_CAUSAL_WORK_FIELDS 9
+int kmb_debug_causal_work(int64_t n_targets, int64_t n_sources, int D, int E, int kernel_id, int flags, int path,
+                          int64_t row_offset, int sms, int smem_optin, int wave, int unit, int64_t* out9);
 
 /* Diagnostics (host logic only): entry `index` of direct-kernel table `table` (0..7: Gaussian difference form n0, n1,
  * exponential n0, n1, inverse distance n0, n1, Gaussian product form n0, n1; nK = row normalisation off / on).

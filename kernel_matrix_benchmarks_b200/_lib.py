@@ -18,7 +18,8 @@ KMB_OK, KMB_ERR_INVALID, KMB_ERR_UNSUPPORTED, KMB_ERR_WORKSPACE, KMB_ERR_CUDA = 
 
 # "dot-exponential" is exp(<x, y>) (softmax attention under normalize_rows): not in bruteforce.py, an extension
 KERNEL_IDS = {"gaussian": 0, "absolute-exponential": 1, "inverse-distance": 2, "dot-exponential": 3}
-FLAG_NORMALIZE_ROWS, FLAG_DENSITY, FLAG_PREPARED = 1, 2, 4
+# FLAG_CAUSAL: row i sees sources j <= row_offset + i (an extension, not in bruteforce.py)
+FLAG_NORMALIZE_ROWS, FLAG_DENSITY, FLAG_PREPARED, FLAG_CAUSAL = 1, 2, 4, 8
 # "tensor_f16x1": the FP16 tensor path with one hi.hi term (float16-class accuracy; only when asked for, never "auto")
 PATH_IDS = {"auto": 0, "direct": 1, "tensor": 5, "tensor_tf32": 2, "tensor_f16": 5, "direct_diff": 3, "direct_sym": 4,
             "tensor_f16x1": 6}
@@ -89,6 +90,10 @@ SIGNATURES = {
     "kmb_resolved_path": (c_int, [c_int, c_int, c_int, c_int]),
     "kmb_debug_product_plan": (c_int, [c_int64, c_int64, c_int, c_int, c_int, c_int, c_int, c_int, POINTER(c_int64)]),
     "kmb_debug_direct_entry": (c_int, [c_int, c_int, POINTER(c_int32)]),
+    "kmb_debug_causal_work": (
+        c_int,
+        [c_int64, c_int64, c_int, c_int, c_int, c_int, c_int, c_int64, c_int, c_int, c_int, c_int, POINTER(c_int64)],
+    ),
     "kmb_debug_pv_plan": (c_int, [c_int64, c_int64, c_int, c_int, c_int, c_int, c_int, c_int, c_int, POINTER(c_int64)]),
     "kmb_set_profiling": (c_int, [c_int]),
     "kmb_last_main_kernel_ms": (c_int, [POINTER(c_float)]),

@@ -152,8 +152,12 @@ class B200Product(BaseProduct):
     """On-the-fly kernel product / density / attention on one B200."""
 
     def __init__(self, *, kernel, dimension, normalize_rows=False, precision="float32", path="auto", device=0,
-                 distributed=False, n_gpus=1):
-        """``n_gpus=G`` (constructor argument, or ``query-args: [{n_gpus: G}]`` through ``set_query_arguments``): this ONE
+                 distributed=False, n_gpus=1, causal=False):
+        """``causal=True``: row i of the result sums the sources j <= i only (autoregressive attention; an extension, not in
+        the reference).  It runs on the FP16 tensor path ("auto" or "tensor_f16") and in float64; the other paths raise
+        NotImplementedError here.  With several GPUs each device gets an equal share of the triangle, not of the rows.
+
+        ``n_gpus=G`` (constructor argument, or ``query-args: [{n_gpus: G}]`` through ``set_query_arguments``): this ONE
         process drives devices ``device .. device+G-1`` -- the harness calls the plugin from a single thread
         (runner.py:118-148), so this is how ``run.py --local --hardware GPU`` sweeps 1/2/4/8 GPUs.  With ``same_points``
         Gaussian data the devices split the symmetric unit list and the first device adds the partial vectors through
@@ -171,6 +175,9 @@ class B200Product(BaseProduct):
             raise ValueError(f"unknown path {path!r} (expected one of {sorted(_lib.PATH_IDS)})")
         if path == "tensor_f16x1" and kernel == "inverse-distance":   # 1/|x - y| amplifies the error of a one-term S
             raise NotImplementedError("B200Product doesn't support kernel inverse-distance on path tensor_f16x1.")
+        self.causal = bool(causal)
+        if self.causal and path not in ("auto", "tensor", "tensor_f16"):
+            raise NotImplementedError(f"B200Product doesn't support causal products on path {path}.")
         self.dtype = _check_precision(precision, "B200Product", (np.float32, np.float64, np.float16))
         _lib.load()  # fail here, loudly, if the CUDA library is absent
         if not torch.cuda.is_available():
@@ -191,7 +198,7 @@ class B200Product(BaseProduct):
 
     def _set_name(self):
         gpus = self.comm.world if self.comm.world > 1 else self.n_gpus
-        extra = f", gpus={gpus}" if gpus > 1 else ""
+        extra = (", causal" if self.causal else "") + (f", gpus={gpus}" if gpus > 1 else "")
         self.name = f"B200Product({self.dtype.name}, path={self.path}{extra})"
 
     def set_query_arguments(self, n_gpus=None, **kwargs):
@@ -214,13 +221,20 @@ class B200Product(BaseProduct):
             g = _multigpu.DeviceGroup(self.device.index, self.n_gpus)
             self._ys = g.replicate(self.source_points)
             if self.same_points:
-                self._bounds = [shard_bounds(self.source_points.shape[0], i, g.n)[:2] for i in range(g.n)]
+                self._bounds = [self._row_bounds(self.source_points.shape[0], i, g.n) for i in range(g.n)]
                 self._xs = [self._ys[i][lo:hi] for i, (lo, hi) in enumerate(self._bounds)]
             else:
-                self._xs, self._bounds = g.shard_rows(self.target_points)
+                self._xs, self._bounds = g.shard_rows(self.target_points, bounds=self._row_bounds)
             g.synchronize()
             self._group = g
         return g
+
+    def _row_bounds(self, n, rank, world):
+        """Row block of a device or rank: equal rows, or under causal equal shares of the triangle (one helper for the
+        n_gpus rows mode and distributed=True)."""
+        if self.causal:
+            return _product.causal_row_bounds(n, rank, world)
+        return shard_bounds(n, rank, world)[:2]
 
     def prepare_data(self, *, source_points, target_points, same_points=False, density_estimation=False):
         """Untimed host->device copy (base.py:64-67), cast to float32 as bruteforce.py:100-106 casts."""
@@ -240,19 +254,19 @@ class B200Product(BaseProduct):
         self._prepared = None
         if self._multi():   # n_gpus given to the constructor: replicate and prepare every device's row block here
             g = self._setup_group()
-            g.prepare_rows(self._xs, self._ys, kernel=self.kernel, path=self.path)
+            g.prepare_rows(self._xs, self._ys, kernel=self.kernel, path=self.path, causal=self.causal)
             g.synchronize()
         elif self.dtype != np.float64:
             with torch.cuda.device(self.device):
                 self._prepared = _product.prepare_points(self._my_rows(), self.source_points, kernel=self.kernel,
-                                                         path=self.path, workspace=self.workspace)
+                                                         path=self.path, workspace=self.workspace, causal=self.causal)
         torch.cuda.synchronize(self.device)
 
     def _my_rows(self):
         """The target rows this process evaluates (all of them, or its block under distributed=True)."""
         if self.comm.world == 1:
             return self.target_points
-        lo, hi, _ = shard_bounds(self.target_points.shape[0], self.comm.rank, self.comm.world)
+        lo, hi = self._row_bounds(self.target_points.shape[0], self.comm.rank, self.comm.world)
         return self.target_points[lo:hi]
 
     def _prepared_token(self, E):
@@ -263,10 +277,10 @@ class B200Product(BaseProduct):
         x = self._my_rows()
         need = _product.workspace_bytes(x.shape[0], self.source_points.shape[0], x.shape[1], E, kernel=self.kernel,
                                         normalize_rows=bool(self.normalize_rows), density_estimation=self.density_estimation,
-                                        path=self.path)
+                                        path=self.path, causal=self.causal)
         if self.workspace.get(need, x.device) is not self._prepared:
             self._prepared = _product.prepare_points(x, self.source_points, kernel=self.kernel, path=self.path,
-                                                     workspace=self.workspace, min_bytes=need)
+                                                     workspace=self.workspace, min_bytes=need, causal=self.causal)
         return self._prepared
 
     def prepare_query(self, *, source_signal):
@@ -286,16 +300,17 @@ class B200Product(BaseProduct):
         E = 1 if self.density_estimation else self.source_signal.shape[1]
         N = self.target_points.shape[0]
         self.res_device = torch.empty((N, E), dtype=torch.float32, device=self.device)
-        if self.same_points and g.symmetric_applies(y0, self.kernel, bool(self.normalize_rows), self.density_estimation, E, self.path):
+        if (self.same_points and not self.causal
+                and g.symmetric_applies(y0, self.kernel, bool(self.normalize_rows), self.density_estimation, E, self.path)):
             g.product_sym(self._ys, self._bs, self.res_device, kernel=self.kernel)
             self.path_used = "direct_sym"
         else:
             if g.prepared is None:   # n_gpus arrived as a query argument: the first query with this GPU count prepares
-                g.prepare_rows(self._xs, self._ys, kernel=self.kernel, path=self.path)
+                g.prepare_rows(self._xs, self._ys, kernel=self.kernel, path=self.path, causal=self.causal)
             g.product_rows(self._xs, self._bounds, self._ys, self._bs, self.res_device, kernel=self.kernel,
                            normalize_rows=bool(self.normalize_rows), density_estimation=self.density_estimation, path=self.path,
-                           prepared=g.prepared)
-            self.path_used = _product.resolved_path(y0.shape[1], E, self.kernel, self.path)
+                           prepared=g.prepared, causal=self.causal)
+            self.path_used = _product.resolved_path(y0.shape[1], E, self.kernel, self.path, self.causal)
         self.launches = g.launches
 
     def query(self):
@@ -303,13 +318,14 @@ class B200Product(BaseProduct):
         with torch.cuda.device(self.device):
             with _GpuTimer() as t:
                 if self.dtype == np.float64:
-                    lo, hi, _ = shard_bounds(self.target_points.shape[0], self.comm.rank, self.comm.world)
+                    lo, hi = self._row_bounds(self.target_points.shape[0], self.comm.rank, self.comm.world)
                     mine = _product.kernel_product_f64(
                         self.target_points[lo:hi], self.source_points, self.source_signal, kernel=self.kernel,
-                        normalize_rows=bool(self.normalize_rows), density_estimation=self.density_estimation, row_offset=lo)
+                        normalize_rows=bool(self.normalize_rows), density_estimation=self.density_estimation, row_offset=lo,
+                        causal=self.causal)
                     self.launches = last_launch_count()
                     self.path_used = "direct_f64"
-                    self.res_device = mine if self.comm.world == 1 else self.comm.all_gather(mine, self.target_points.shape[0])
+                    self.res_device = mine if self.comm.world == 1 else self._gather_rows(mine)
                 elif self.comm.world > 1:
                     self._query_distributed()
                 elif self._multi():
@@ -326,6 +342,7 @@ class B200Product(BaseProduct):
                         path=self.path,
                         workspace=self.workspace,
                         prepared=self._prepared_token(E),
+                        causal=self.causal,
                     )
                     self.path_used = _product.last_path
                     self.launches = last_launch_count()
@@ -339,20 +356,31 @@ class B200Product(BaseProduct):
         y, b = self.source_points, self.source_signal
         E = 1 if self.density_estimation else b.shape[1]
         sym = (self.path == "auto" and self.same_points and y.shape[0] >= _product.SYM_MIN_POINTS and
-               _product.symmetric_applies(y, y, self.kernel, bool(self.normalize_rows), self.density_estimation, E))
+               _product.symmetric_applies(y, y, self.kernel, bool(self.normalize_rows), self.density_estimation, E, self.causal))
         if sym:
             self.res_device = kernel_product_sym_part(y, b, rank, world, kernel=self.kernel, workspace=self.workspace)
             self.launches = last_launch_count()
             self.comm.all_reduce(self.res_device)
             self.path_used = "direct_sym"
             return
-        lo, hi, _ = shard_bounds(self.target_points.shape[0], rank, world)
+        lo, hi = self._row_bounds(self.target_points.shape[0], rank, world)
         mine = kernel_product(self.target_points[lo:hi], y, b, kernel=self.kernel, normalize_rows=bool(self.normalize_rows),
                               density_estimation=self.density_estimation, path=self.path, row_offset=lo,
-                              workspace=self.workspace, prepared=self._prepared_token(E))
+                              workspace=self.workspace, prepared=self._prepared_token(E), causal=self.causal)
         self.launches = last_launch_count()
         self.path_used = _product.last_path
-        self.res_device = self.comm.all_gather(mine, self.target_points.shape[0])
+        self.res_device = self._gather_rows(mine)
+
+    def _gather_rows(self, mine):
+        """All ranks' row blocks (self._row_bounds) in row order on every rank.  The equal blocks of the non-causal split
+        are what comm.all_gather expects; the causal blocks are padded to the largest and cut back out."""
+        n, world = self.target_points.shape[0], self.comm.world
+        if not self.causal:
+            return self.comm.all_gather(mine, n)
+        bounds = [self._row_bounds(n, r, world) for r in range(world)]
+        per = max(hi - lo for lo, hi in bounds)
+        full = self.comm.all_gather(mine, per * world)
+        return torch.cat([full[r * per: r * per + (hi - lo)] for r, (lo, hi) in enumerate(bounds)])
 
     def get_result(self):
         """Untimed device->host copy; float64 contiguous as base.py:116."""

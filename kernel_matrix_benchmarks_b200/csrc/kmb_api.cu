@@ -274,7 +274,8 @@ static int check_product_args(int64_t N, int64_t M, int D, int E, int kid, int f
     if (kid == KMB_KERNEL_INVERSE_DISTANCE && path == KMB_PATH_TENSOR_1XF16)
         return set_error(KMB_ERR_UNSUPPORTED, "the one-term FP16 path does not support the inverse-distance kernel (1/|x-y| amplifies "
                                               "the error of a one-term S near coincident points)");
-    if (flags & ~(KMB_FLAG_NORMALIZE_ROWS | KMB_FLAG_DENSITY | KMB_FLAG_PREPARED)) return set_error(KMB_ERR_INVALID, "unknown flags 0x%x", flags);
+    if (flags & ~(KMB_FLAG_NORMALIZE_ROWS | KMB_FLAG_DENSITY | KMB_FLAG_PREPARED | KMB_FLAG_CAUSAL))
+        return set_error(KMB_ERR_INVALID, "unknown flags 0x%x", flags);
     if ((flags & KMB_FLAG_DENSITY) && E != 1) return set_error(KMB_ERR_INVALID, "density estimation implies E == 1 (got %d)", E);
     if (path < KMB_PATH_AUTO || path > KMB_PATH_TENSOR_1XF16) return set_error(KMB_ERR_INVALID, "unknown path %d", path);
     if (path == KMB_PATH_DIRECT_SYM) {
@@ -294,11 +295,25 @@ constexpr int kWideSignal = 32;
 static int tensor_elt(int path) {
     return path == KMB_PATH_TENSOR_3XTF32 ? 0 : path == KMB_PATH_TENSOR_3XF16 ? 1 : path == KMB_PATH_TENSOR_1XF16 ? 2 : -1;
 }
+// KMB_FLAG_CAUSAL: the causal kernels are the three-term FP16 ones, so the tensor path at every D as well.
 bool tensor_pv16_applicable(int D, int E, int kid);   // kprod_tensor_pv16.cu
-static int resolve_path(int D, int E, int kid, int path) {
+bool tensor_pv_applicable(int D, int E);              // kprod_tensor_pv.cu
+static int resolve_path(int D, int E, int kid, int flags, int path) {
     if (path != KMB_PATH_AUTO) return path;
-    if (D > 16 || kid == KMB_KERNEL_DOT_EXPONENTIAL) return KMB_PATH_TENSOR_3XF16;
+    if (D > 16 || kid == KMB_KERNEL_DOT_EXPONENTIAL || (flags & KMB_FLAG_CAUSAL)) return KMB_PATH_TENSOR_3XF16;
     return (E >= kWideSignal && tensor_pv16_applicable(D, E, kid)) ? KMB_PATH_TENSOR_3XF16 : KMB_PATH_DIRECT_F32;
+}
+
+// KMB_FLAG_CAUSAL runs on the three-term FP16 kernels (kprod_tensor, _pair, pv16, pv16_pair) only: the other paths, and
+// the one shape the FP16 path hands to the TF32 P.B kernel (inverse distance, E > 4, D <= 128), have no causal kernel.
+static int check_causal(int D, int E, int kid, int flags, int path) {
+    if (!(flags & KMB_FLAG_CAUSAL)) return KMB_OK;
+    if (resolve_path(D, E, kid, flags, path) != KMB_PATH_TENSOR_3XF16)
+        return set_error(KMB_ERR_UNSUPPORTED, "causal products run on the three-term FP16 tensor path only (path %d)", path);
+    if (!((flags & KMB_FLAG_NORMALIZE_ROWS) && (flags & KMB_FLAG_DENSITY)) && tensor_pv_applicable(D, E) &&
+        !tensor_pv16_applicable(D, E, kid))
+        return set_error(KMB_ERR_UNSUPPORTED, "no causal kernel for the TF32 P.B family (inverse distance, E > 4, D <= 128)");
+    return KMB_OK;
 }
 
 // Enqueue the direct pipeline on `stream`: bounding-box statistics -> source packing -> main kernels.
@@ -463,9 +478,10 @@ int kmb_product_workspace_bytes(int64_t N, int64_t M, int D, int E, int kernel_i
                                 size_t* bytes) {
     if (!bytes) return set_error(KMB_ERR_INVALID, "bytes is NULL");
     if (int rc = check_product_args(N, M, D, E, kernel_id, flags, path)) return rc;
+    if (int rc = check_causal(D, E, kernel_id, flags, path)) return rc;
     *bytes = 256;
     if ((flags & KMB_FLAG_NORMALIZE_ROWS) && (flags & KMB_FLAG_DENSITY)) return KMB_OK;
-    const int p = resolve_path(D, E, kernel_id, path);
+    const int p = resolve_path(D, E, kernel_id, flags, path);
     if (p == KMB_PATH_DIRECT_SYM) return kmb_product_sym_workspace_bytes(N, D, 0, 1, bytes);
     if (p == KMB_PATH_DIRECT_F32 || p == KMB_PATH_DIRECT_DIFF) {
         DirectPlan pl;
@@ -482,6 +498,7 @@ int kmb_product_f32(const float* x, const float* y, const float* b, float* out, 
     g_launches = 0;
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     if (int rc = check_product_args(N, M, D, E, kernel_id, flags, path)) return rc;
+    if (int rc = check_causal(D, E, kernel_id, flags, path)) return rc;
     if (N == 0) return KMB_OK;   // an empty row shard (x and out may then be NULL: empty tensors have no storage)
     if (!x || !y || !out) return set_error(KMB_ERR_INVALID, "x, y and out must not be NULL");
     const bool density = flags & KMB_FLAG_DENSITY;
@@ -493,7 +510,7 @@ int kmb_product_f32(const float* x, const float* y, const float* b, float* out, 
         count_launch();
         return KMB_OK;
     }
-    const int p = resolve_path(D, E, kernel_id, path);
+    const int p = resolve_path(D, E, kernel_id, flags, path);
     if (reinterpret_cast<uintptr_t>(workspace) % 256)
         return set_error(KMB_ERR_INVALID, "workspace must be 256-byte aligned");
     if (tensor_elt(p) >= 0) {
@@ -524,9 +541,10 @@ int kmb_product_prepare_f32(const float* x, const float* y, int64_t N, int64_t M
                             void* workspace, size_t workspace_bytes, void* stream_) {
     g_launches = 0;
     if (int rc = check_product_args(N, M, D, 1, kernel_id, flags & ~KMB_FLAG_DENSITY, path)) return rc;
+    if (int rc = check_causal(D, 1, kernel_id, flags & ~KMB_FLAG_DENSITY, path)) return rc;
     if (!x || !y) return set_error(KMB_ERR_INVALID, "x and y must not be NULL");
     if (N == 0) return KMB_OK;
-    const int p = resolve_path(D, 1, kernel_id, path);   // (D <= 16 under KMB_PATH_AUTO: the signal width decides at query time)
+    const int p = resolve_path(D, 1, kernel_id, flags, path);   // (D <= 16 under KMB_PATH_AUTO: the signal width decides at query time)
     if (p != KMB_PATH_TENSOR_3XF16 && p != KMB_PATH_TENSOR_1XF16) return KMB_OK;   // nothing worth keeping on the other paths
     if (reinterpret_cast<uintptr_t>(workspace) % 256) return set_error(KMB_ERR_INVALID, "workspace must be 256-byte aligned");
     return tensor_prepare(x, y, N, M, D, kernel_id, tensor_elt(p), workspace, workspace_bytes, static_cast<cudaStream_t>(stream_));
@@ -554,7 +572,7 @@ int kmb_resolved_path(int D, int E, int kernel_id, int path) {
     if (D < 1 || E < 1 || kernel_id < KMB_KERNEL_GAUSSIAN || kernel_id > KMB_KERNEL_DOT_EXPONENTIAL || path < KMB_PATH_AUTO ||
         path > KMB_PATH_TENSOR_1XF16)
         return -1;
-    return resolve_path(D, E, kernel_id, path);
+    return resolve_path(D, E, kernel_id, 0, path);
 }
 
 int kmb_debug_direct_entry(int table, int index, int32_t* out11) {
@@ -572,8 +590,9 @@ int kmb_debug_direct_entry(int table, int index, int32_t* out11) {
 int kmb_debug_product_plan(int64_t N, int64_t M, int D, int E, int kernel_id, int flags, int path, int sms, int64_t* out10) {
     if (!out10 || sms < 1) return set_error(KMB_ERR_INVALID, "bad arguments");
     if (int rc = check_product_args(N, M, D, E, kernel_id, flags, path)) return rc;
+    if (int rc = check_causal(D, E, kernel_id, flags, path)) return rc;
     for (int i = 0; i < 10; ++i) out10[i] = -1;
-    const int p = resolve_path(D, E, kernel_id, path);
+    const int p = resolve_path(D, E, kernel_id, flags, path);
     out10[0] = p;
     if ((flags & KMB_FLAG_NORMALIZE_ROWS) && (flags & KMB_FLAG_DENSITY)) {
         out10[1] = KMB_FAMILY_FILL;
@@ -629,6 +648,19 @@ int kmb_debug_pv_plan(int64_t N, int64_t M, int D, int E, int kernel_id, int fla
         if (int rc = tensor_pv_plan_query(N, M, D, E, kernel_id, tensor_elt(static_cast<int>(plan[0])), sms, smem_optin, o))
             return rc;
     for (int i = 0; i < KMB_PV_PLAN_FIELDS; ++i) out19[i] = o[i];
+    return KMB_OK;
+}
+
+int kmb_debug_causal_work(int64_t N, int64_t M, int D, int E, int kernel_id, int flags, int path, int64_t row_offset, int sms,
+                          int smem_optin, int wave, int unit, int64_t* out9) {
+    if (!out9 || N < 1 || sms < 1 || smem_optin < 1 || row_offset < 0) return set_error(KMB_ERR_INVALID, "bad arguments");
+    if (!(flags & KMB_FLAG_CAUSAL)) return set_error(KMB_ERR_INVALID, "kmb_debug_causal_work needs KMB_FLAG_CAUSAL");
+    if ((flags & KMB_FLAG_NORMALIZE_ROWS) && (flags & KMB_FLAG_DENSITY)) return set_error(KMB_ERR_INVALID, "a filled result has no plan");
+    if (int rc = check_product_args(N, M, D, E, kernel_id, flags, path)) return rc;
+    if (int rc = check_causal(D, E, kernel_id, flags, path)) return rc;
+    long long o[KMB_CAUSAL_WORK_FIELDS];
+    if (int rc = tensor_causal_work_debug(N, M, D, E, kernel_id, row_offset, sms, smem_optin, wave, unit, o)) return rc;
+    for (int i = 0; i < KMB_CAUSAL_WORK_FIELDS; ++i) out9[i] = o[i];
     return KMB_OK;
 }
 

@@ -37,16 +37,16 @@ __device__ __forceinline__ double kernel_value_f64(double d2) {   // d2: the sum
     else return 1.0 / sqrt(fmax(d2, 0.0));                                                          // bruteforce.py:10-11
 }
 
-// E columns e0 .. e0+EC-1 of the signal per launch (EC <= F64_MAX_E)
-template <int KID, int EC>
-__global__ void __launch_bounds__(F64_THREADS)
-kprod_f64_kernel(const double* __restrict__ x, const double* __restrict__ y, const double* __restrict__ b,
-                 double* __restrict__ out, long long N, long long M, int D, int E, int e0, int normalize,
-                 long long row_offset) {
+// E columns e0 .. e0+EC-1 of the signal per launch (EC <= F64_MAX_E).  CAUSAL (KMB_FLAG_CAUSAL): row i sums the sources
+// j <= row_offset + i only, and the CTA stops at the last source its last row sees.
+template <int KID, int EC, bool CAUSAL>
+__device__ __forceinline__ void f64_rows_body(const uint32_t tid, const double* __restrict__ x, const double* __restrict__ y, const double* __restrict__ b,
+                                              double* __restrict__ out, long long N, long long M, int D, int E, int e0, int normalize,
+                                              long long row_offset) {
     extern __shared__ double sm[];
     double* sy = sm;                        // F64_SB x D
     double* sb = sm + F64_SB * D;           // F64_SB x EC
-    const long long row = blockIdx.x * static_cast<long long>(F64_THREADS) + threadIdx.x;
+    const long long row = blockIdx.x * static_cast<long long>(F64_THREADS) + tid;
     const bool ok = row < N;
     double xr[F64_MAX_D];
 #pragma unroll
@@ -55,12 +55,14 @@ kprod_f64_kernel(const double* __restrict__ x, const double* __restrict__ y, con
 #pragma unroll
     for (int e = 0; e < EC; ++e) acc[e] = 0.0;
     [[maybe_unused]] const long long jz = (row_offset + row) % (M + 1);   // inverse-distance zeroing (bruteforce.py:12-14)
+    long long m_end = M;
+    if constexpr (CAUSAL) m_end = min(M, row_offset + min(N, (blockIdx.x + 1ll) * F64_THREADS));
 
-    for (long long j0 = 0; j0 < M; j0 += F64_SB) {
-        const int cnt = static_cast<int>(min(static_cast<long long>(F64_SB), M - j0));
+    for (long long j0 = 0; j0 < m_end; j0 += F64_SB) {
+        const int cnt = static_cast<int>(min(static_cast<long long>(F64_SB), m_end - j0));
         __syncthreads();
-        for (int i = threadIdx.x; i < cnt * D; i += F64_THREADS) sy[i] = y[j0 * D + i];
-        for (int i = threadIdx.x; i < cnt * EC; i += F64_THREADS) {
+        for (int i = tid; i < cnt * D; i += F64_THREADS) sy[i] = y[j0 * D + i];
+        for (int i = tid; i < cnt * EC; i += F64_THREADS) {
             const int j = i / EC, e = i % EC;
             sb[i] = (e0 + e < E) ? (b ? b[(j0 + j) * E + e0 + e] : 1.0) : 0.0;
         }
@@ -76,6 +78,9 @@ kprod_f64_kernel(const double* __restrict__ x, const double* __restrict__ y, con
                 if constexpr (KID == KMB_KERNEL_INVERSE_DISTANCE) {
                     if (j0 + j == jz) k = 0.0;
                 }
+                if constexpr (CAUSAL) {
+                    if (j0 + j > row_offset + row) k = 0.0;
+                }
                 ksum += k;
 #pragma unroll
                 for (int e = 0; e < EC; ++e) acc[e] = fma(k, sb[j * EC + e], acc[e]);
@@ -88,6 +93,20 @@ kprod_f64_kernel(const double* __restrict__ x, const double* __restrict__ y, con
             if (e0 + e < E) out[row * E + e0 + e] = normalize ? acc[e] / ksum : acc[e];
     }
 }
+template <int KID, int EC>
+__global__ void __launch_bounds__(F64_THREADS)
+kprod_f64_kernel(const double* __restrict__ x, const double* __restrict__ y, const double* __restrict__ b,
+                 double* __restrict__ out, long long N, long long M, int D, int E, int e0, int normalize,
+                 long long row_offset) {
+    f64_rows_body<KID, EC, false>(threadIdx.x, x, y, b, out, N, M, D, E, e0, normalize, row_offset);
+}
+template <int KID, int EC>
+__global__ void __launch_bounds__(F64_THREADS)
+kprod_f64_causal_kernel(const double* __restrict__ x, const double* __restrict__ y, const double* __restrict__ b,
+                        double* __restrict__ out, long long N, long long M, int D, int E, int e0, int normalize,
+                        long long row_offset) {
+    f64_rows_body<KID, EC, true>(threadIdx.x, x, y, b, out, N, M, D, E, e0, normalize, row_offset);
+}
 
 // ---- any D (D > 16): tiled version --------------------------------------------------------------------
 // The reference's ground truth for every dataset is its float64 brute force (datasets.py:180-195), also for the
@@ -99,17 +118,16 @@ kprod_f64_kernel(const double* __restrict__ x, const double* __restrict__ y, con
 // pass), 16 accumulators per thread in registers across all source tiles; row sums of k ride along for normalize_rows.
 constexpr int W_T = 64, W_DC = 16, W_EC = 64, W_THREADS = 256;
 
-template <int KID>
-__global__ void __launch_bounds__(W_THREADS)
-kprod_f64_wide_kernel(const double* __restrict__ x, const double* __restrict__ y, const double* __restrict__ b,
-                      double* __restrict__ out, long long N, long long M, int D, int E, int e0, int normalize,
-                      long long row_offset) {
+template <int KID, bool CAUSAL>
+__device__ __forceinline__ void f64_wide_body(const uint32_t tid_, const double* __restrict__ x, const double* __restrict__ y, const double* __restrict__ b,
+                                              double* __restrict__ out, long long N, long long M, int D, int E, int e0, int normalize,
+                                              long long row_offset) {
     extern __shared__ double wide_smem[];
     double (*xs)[W_DC + 1] = reinterpret_cast<double (*)[W_DC + 1]>(wide_smem);
     double (*ys)[W_DC + 1] = xs + W_T;
     double (*ks)[W_T + 1] = reinterpret_cast<double (*)[W_T + 1]>(wide_smem + 2 * W_T * (W_DC + 1));
     double (*bs)[W_EC] = reinterpret_cast<double (*)[W_EC]>(wide_smem + 2 * W_T * (W_DC + 1) + W_T * (W_T + 1));
-    const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
+    const int tid = tid_, tx = tid & 15, ty = tid >> 4;
     const long long row0 = blockIdx.x * static_cast<long long>(W_T);
     const int ec = min(W_EC, E - e0);
     const int pr = tid >> 2, pc = tid & 3;   // phase 2: row pr, signal columns pc, pc + 4, ...
@@ -117,7 +135,9 @@ kprod_f64_wide_kernel(const double* __restrict__ x, const double* __restrict__ y
 #pragma unroll
     for (int q = 0; q < W_EC / 4; ++q) acc[q] = 0.0;
 
-    for (long long j0 = 0; j0 < M; j0 += W_T) {
+    long long m_end = M;
+    if constexpr (CAUSAL) m_end = min(M, row_offset + min(N, row0 + W_T));
+    for (long long j0 = 0; j0 < m_end; j0 += W_T) {
         double d2[4][4];
 #pragma unroll
         for (int i = 0; i < 4; ++i)
@@ -153,6 +173,9 @@ kprod_f64_wide_kernel(const double* __restrict__ x, const double* __restrict__ y
                 if constexpr (KID == KMB_KERNEL_INVERSE_DISTANCE) {
                     if (src == (row_offset + row) % (M + 1)) k = 0.0;   // bruteforce.py:12-14
                 }
+                if constexpr (CAUSAL) {
+                    if (src > row_offset + row) k = 0.0;
+                }
                 ks[ty + 16 * i][tx + 16 * j] = k;
             }
         for (int i = tid; i < W_T * W_EC; i += W_THREADS) {
@@ -176,6 +199,20 @@ kprod_f64_wide_kernel(const double* __restrict__ x, const double* __restrict__ y
         }
     }
 }
+template <int KID>
+__global__ void __launch_bounds__(W_THREADS)
+kprod_f64_wide_kernel(const double* __restrict__ x, const double* __restrict__ y, const double* __restrict__ b,
+                      double* __restrict__ out, long long N, long long M, int D, int E, int e0, int normalize,
+                      long long row_offset) {
+    f64_wide_body<KID, false>(threadIdx.x, x, y, b, out, N, M, D, E, e0, normalize, row_offset);
+}
+template <int KID>
+__global__ void __launch_bounds__(W_THREADS)
+kprod_f64_wide_causal_kernel(const double* __restrict__ x, const double* __restrict__ y, const double* __restrict__ b,
+                             double* __restrict__ out, long long N, long long M, int D, int E, int e0, int normalize,
+                             long long row_offset) {
+    f64_wide_body<KID, true>(threadIdx.x, x, y, b, out, N, M, D, E, e0, normalize, row_offset);
+}
 
 template <int KID>
 int launch_f64_wide(const double* x, const double* y, const double* b, double* out, int64_t N, int64_t M, int D, int E, int flags,
@@ -183,9 +220,10 @@ int launch_f64_wide(const double* x, const double* y, const double* b, double* o
     const int normalize = (flags & KMB_FLAG_NORMALIZE_ROWS) ? 1 : 0;
     const unsigned grid = static_cast<unsigned>((N + W_T - 1) / W_T);
     constexpr int smem = sizeof(double) * (2 * W_T * (W_DC + 1) + W_T * (W_T + 1) + W_T * W_EC);
-    if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(&kprod_f64_wide_kernel<KID>), smem)) return rc;
+    auto fn = (flags & KMB_FLAG_CAUSAL) ? &kprod_f64_wide_causal_kernel<KID> : &kprod_f64_wide_kernel<KID>;
+    if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(fn), smem)) return rc;
     for (int e0 = 0; e0 < E; e0 += W_EC) {
-        kprod_f64_wide_kernel<KID><<<grid, W_THREADS, smem, stream>>>(x, y, b, out, N, M, D, E, e0, normalize, row_offset);
+        fn<<<grid, W_THREADS, smem, stream>>>(x, y, b, out, N, M, D, E, e0, normalize, row_offset);
         KMB_CUDA_CHECK(cudaGetLastError());
         count_launch();
     }
@@ -205,10 +243,12 @@ int launch_f64(const double* x, const double* y, const double* b, double* out, i
     for (int e0 = 0; e0 < E; e0 += F64_MAX_E) {
         const int ec = std::min(F64_MAX_E, E - e0);
         const size_t smem = sizeof(double) * F64_SB * (D + (ec <= 1 ? 1 : ec <= 2 ? 2 : ec <= 4 ? 4 : 8));
-        if (ec <= 1) kprod_f64_kernel<KID, 1><<<grid, F64_THREADS, smem, stream>>>(x, y, b, out, N, M, D, E, e0, normalize, row_offset);
-        else if (ec <= 2) kprod_f64_kernel<KID, 2><<<grid, F64_THREADS, smem, stream>>>(x, y, b, out, N, M, D, E, e0, normalize, row_offset);
-        else if (ec <= 4) kprod_f64_kernel<KID, 4><<<grid, F64_THREADS, smem, stream>>>(x, y, b, out, N, M, D, E, e0, normalize, row_offset);
-        else kprod_f64_kernel<KID, 8><<<grid, F64_THREADS, smem, stream>>>(x, y, b, out, N, M, D, E, e0, normalize, row_offset);
+        const bool causal = flags & KMB_FLAG_CAUSAL;
+        auto fn = ec <= 1 ? (causal ? &kprod_f64_causal_kernel<KID, 1> : &kprod_f64_kernel<KID, 1>)
+                : ec <= 2 ? (causal ? &kprod_f64_causal_kernel<KID, 2> : &kprod_f64_kernel<KID, 2>)
+                : ec <= 4 ? (causal ? &kprod_f64_causal_kernel<KID, 4> : &kprod_f64_kernel<KID, 4>)
+                          : (causal ? &kprod_f64_causal_kernel<KID, 8> : &kprod_f64_kernel<KID, 8>);
+        fn<<<grid, F64_THREADS, smem, stream>>>(x, y, b, out, N, M, D, E, e0, normalize, row_offset);
         KMB_CUDA_CHECK(cudaGetLastError());
         count_launch();
     }

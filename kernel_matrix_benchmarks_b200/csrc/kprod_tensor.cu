@@ -82,7 +82,7 @@ struct Cfg {
 // The body of both kernels: single CTAs (PAIR = false, any ELT) and CTA pairs (PAIR = true, FP16 planes).  tid is
 // threadIdx.x as the __global__ function reads it: there __launch_bounds__ bounds it by THREADS, which lets the compiler
 // unroll the epilogue's staging loop without a bounds check (a read in this function would only be known below 1024).
-template <int EP, int KID, bool NORM, bool PAIR, int ELT>
+template <int EP, int KID, bool NORM, bool PAIR, int ELT, bool CAUSAL = false>
 __device__ __forceinline__ void tensor_body(const uint32_t tid, const CUtensorMap& map_ah, const CUtensorMap& map_al,
                                             const CUtensorMap& map_bh, const CUtensorMap& map_bl, const Params& P) {
     static_assert(!PAIR || ELT != ELT_TF32, "CTA pairs run FP16 planes");
@@ -128,7 +128,7 @@ __device__ __forceinline__ void tensor_body(const uint32_t tid, const CUtensorMa
         uint32_t it = 0;
         WaveWork ww;
         for (int w = 0; w < P.W; ++w) {
-            if (!wave_work(P, w, cta, ww)) continue;
+            if (!wave_work<CAUSAL, TN, PAIR>(P, w, cta, ww)) continue;
             const int row0 = (PAIR ? ww.tile * 2 + static_cast<int>(rank) : ww.tile) * TM;
             for (int sb = ww.sb_lo; sb < ww.sb_hi; ++sb) {
                 const int src0 = sb * TN + (PAIR ? static_cast<int>(rank) * (TN / 2) : 0);   // pairs: this CTA's half
@@ -170,7 +170,7 @@ __device__ __forceinline__ void tensor_body(const uint32_t tid, const CUtensorMa
             uint32_t it = 0, unit = 0;
             WaveWork ww;
             for (int w = 0; w < P.W; ++w) {
-                if (!wave_work(P, w, cta, ww)) continue;
+                if (!wave_work<CAUSAL, TN, PAIR>(P, w, cta, ww)) continue;
                 for (int sb = ww.sb_lo; sb < ww.sb_hi; ++sb, ++unit) {
                     const int a = unit % ACC_STAGES;
                     mbar_wait(&acc_empty[a], ((unit / ACC_STAGES) & 1) ^ 1);
@@ -218,7 +218,7 @@ __device__ __forceinline__ void tensor_body(const uint32_t tid, const CUtensorMa
         uint32_t unit = 0;
         WaveWork ww;
         for (int w = 0; w < P.W; ++w) {
-            if (!wave_work(P, w, cta, ww)) continue;
+            if (!wave_work<CAUSAL, TN, PAIR>(P, w, cta, ww)) continue;
             const int tile = PAIR ? ww.tile * 2 + static_cast<int>(rank) : ww.tile;
             const long long row = static_cast<long long>(tile) * TM + row_in_tile;
             const bool row_ok = row < P.N;
@@ -254,6 +254,64 @@ __device__ __forceinline__ void tensor_body(const uint32_t tid, const CUtensorMa
                 float acc[EP], ksum = 0.f;
 #pragma unroll
                 for (int e = 0; e < EP; ++e) acc[e] = 0.f;
+                // CAUSAL, a block that crosses this tile's diagonal (warp-uniform): a pair with j > row_offset + row is a padded
+                // source, weight exactly 0, log2 k = -inf (no effect on the running maximum).  Fully visible blocks run the
+                // unmasked loop below.
+                bool drained = false;
+                if constexpr (CAUSAL) {
+                    if (j0 + TN - 1 > P.row_offset + static_cast<long long>(tile) * TM) {
+                    const long long lim = P.row_offset + row - j0;   // last visible jj of this row
+#pragma unroll 1
+                    for (int ch = 0; ch < TN / 32; ++ch) {
+                        float s[32];
+                        tmem_ld_32x32(t_addr + ch * 32, s);
+                        if constexpr (ELT != ELT_TF32) {
+#pragma unroll
+                            for (int c = 0; c < 32; ++c) s[c] *= sscale;   // exact: a power of two
+                        }
+                        if constexpr (!C::ONLINE_MAX) {
+#pragma unroll
+                            for (int c = 0; c < 32; ++c) {
+                                const int jj = ch * 32 + c;
+                                float kv = kernel_from_parts<KID>(s[c], un, ax[jj]);
+                                if constexpr (KID == KMB_KERNEL_INVERSE_DISTANCE)
+                                    if (j0 + jj == jz || j0 + jj >= P.M) kv = 0.f;  // zeroing rule; padding adds exactly 0
+                                if (jj > lim) kv = 0.f;
+#pragma unroll
+                                for (int e = 0; e < EP; ++e) acc[e] = fmaf(kv, ax[TN + jj * EP + e], acc[e]);
+                                if constexpr (NORM) ksum += kv;
+                            }
+                        } else {
+                            float cm = -INFINITY;
+#pragma unroll
+                            for (int c = 0; c < 32; ++c) {
+                                s[c] = log2_kernel_from_parts<KID>(s[c], un, ax[ch * 32 + c]);
+                                if (ch * 32 + c > lim) s[c] = -INFINITY;
+                                cm = fmaxf(cm, s[c]);
+                            }
+                            const float mnew = fmaxf(kmax, cm);
+                            const float sc = (mnew == -INFINITY) ? 1.f : ex2_approx(kmax - mnew);
+                            const float moff = (mnew == -INFINITY) ? 0.f : mnew;
+                            kmax = mnew;
+                            // rescale everything accumulated so far (this unit and the tile totals)
+                            ksum *= sc;
+                            ktot *= sc;
+#pragma unroll
+                            for (int e = 0; e < EP; ++e) { acc[e] *= sc; tot[e] *= sc; }
+#pragma unroll
+                            for (int c = 0; c < 32; ++c) {
+                                const int jj = ch * 32 + c;
+                                const float kv = ex2_approx(s[c] - moff);
+#pragma unroll
+                                for (int e = 0; e < EP; ++e) acc[e] = fmaf(kv, ax[TN + jj * EP + e], acc[e]);
+                                ksum += kv;
+                            }
+                        }
+                    }
+                    drained = true;
+                    }
+                }
+                if (!drained) {
 #pragma unroll 1
                 for (int ch = 0; ch < TN / 32; ++ch) {
                     float s[32];
@@ -298,6 +356,7 @@ __device__ __forceinline__ void tensor_body(const uint32_t tid, const CUtensorMa
                             ksum += kv;
                         }
                     }
+                }
                 }
                 // accumulator drained: hand the TMEM stage back to the MMA warp (pairs: the leader's, remotely from the peer)
                 tc_fence_before();
@@ -386,6 +445,15 @@ kprod_tensor_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_con
     tensor_body<EP, KID, NORM, false, ELT>(threadIdx.x, map_ah, map_al, map_bh, map_bl, P);
 }
 
+// KMB_FLAG_CAUSAL on FP16 planes: kernels of their own, so that the instantiations above stay as they were
+template <int EP, int KID, bool NORM>
+__global__ void __launch_bounds__(THREADS, 1)
+kprod_tensor_causal_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant__ CUtensorMap map_al,
+                           const __grid_constant__ CUtensorMap map_bh, const __grid_constant__ CUtensorMap map_bl,
+                           const Params P) {
+    tensor_body<EP, KID, NORM, false, ELT_F16, true>(threadIdx.x, map_ah, map_al, map_bh, map_bl, P);
+}
+
 namespace pair {
 // TERMS = 3: lo.hi + hi.lo + hi.hi (ELT_F16, KMB_PATH_TENSOR_3XF16); TERMS = 1: hi.hi only, the lo planes are not loaded
 // (ELT_F16X1, KMB_PATH_TENSOR_1XF16).
@@ -396,6 +464,13 @@ kprod_tensor_pair_kernel(const __grid_constant__ CUtensorMap map_ah, const __gri
                          const Params P) {
     static_assert(TERMS == 3 || TERMS == 1, "three-term or one-term split");
     tensor_body<EP, KID, NORM, true, TERMS == 3 ? ELT_F16 : ELT_F16X1>(threadIdx.x, map_ah, map_al, map_bh, map_bl, P);
+}
+template <int EP, int KID, bool NORM>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
+kprod_tensor_pair_causal_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant__ CUtensorMap map_al,
+                                const __grid_constant__ CUtensorMap map_bh, const __grid_constant__ CUtensorMap map_bl,
+                                const Params P) {
+    tensor_body<EP, KID, NORM, true, ELT_F16, true>(threadIdx.x, map_ah, map_al, map_bh, map_bl, P);
 }
 }  // namespace pair
 
@@ -780,6 +855,23 @@ struct TensorPlan {
     size_t off_center, off_cpart, off_sscale, off_uh, off_ul, off_vh, off_vl, off_un, off_vn, off_partial, off_counter, total;
 };
 
+// host logic only: CTA pairs or single CTAs, the grid and the wave plan of kprod_tensor on `sms` SMs (plan_tensor and
+// the causal plan query share it)
+void tensor_wave_plan(long long n_tiles, long long nsb, int Dp, bool f16, int sms, bool* pair, int* grid, tc::WavePlan* waves) {
+    const size_t esz = f16 ? 2 : 4;
+    *grid = sms;
+    *pair = f16 && tensor_use_pair(n_tiles, sms);
+    if (*pair) {
+        // the wave plan counts pairs of row tiles and clusters of two CTAs
+        *grid = sms / 2 * 2;
+        tc::plan_waves((n_tiles + 1) / 2, nsb, *grid / 2, static_cast<size_t>(tc::TM) * Dp * esz * 4, waves);
+        waves->slots_per_wave *= 2;
+        waves->partial_slots *= 2;
+    } else {
+        tc::plan_waves(n_tiles, nsb, *grid, static_cast<size_t>(tc::TM) * Dp * esz * 2, waves);
+    }
+}
+
 int plan_tensor(int64_t N, int64_t M, int D, int E, int elt, TensorPlan* pl) {
     const bool f16 = elt != tc::ELT_TF32;
     pl->Dp = f16 ? (D + 15) / 16 * 16 : (D + tc::TK - 1) / tc::TK * tc::TK;
@@ -794,17 +886,7 @@ int plan_tensor(int64_t N, int64_t M, int D, int E, int elt, TensorPlan* pl) {
     int dev = 0, sms = 0;
     KMB_CUDA_CHECK(cudaGetDevice(&dev));
     KMB_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    pl->grid = sms;
-    pl->pair = f16 && tensor_use_pair(pl->n_tiles, sms);
-    if (pl->pair) {
-        // the wave plan counts pairs of row tiles and clusters of two CTAs
-        pl->grid = sms / 2 * 2;
-        tc::plan_waves((pl->n_tiles + 1) / 2, pl->nsb, pl->grid / 2, static_cast<size_t>(tc::TM) * pl->Dp * pl->esz * 4, &pl->waves);
-        pl->waves.slots_per_wave *= 2;
-        pl->waves.partial_slots *= 2;
-    } else {
-        tc::plan_waves(pl->n_tiles, pl->nsb, pl->grid, static_cast<size_t>(tc::TM) * pl->Dp * pl->esz * 2, &pl->waves);
-    }
+    tensor_wave_plan(pl->n_tiles, pl->nsb, pl->Dp, f16, sms, &pl->pair, &pl->grid, &pl->waves);
     const int PS = tc::MAX_EP + 2;
     size_t o = 0;
     auto take = [&](size_t bytes) { size_t at = o; o += align_up(bytes, 256); return at; };
@@ -834,12 +916,16 @@ int plan_tensor(int64_t N, int64_t M, int D, int E, int elt, TensorPlan* pl) {
 
 using KernelFn = void (*)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const tc::Params);
 
-// PAIR: the CTA-pair kernel (FP16 planes; ELT_F16 runs TERMS = 3, ELT_F16X1 TERMS = 1), else the single-CTA one
-template <bool PAIR, int EP, int KID, bool NORM, int ELT>
+// PAIR: the CTA-pair kernel (FP16 planes; ELT_F16 runs TERMS = 3, ELT_F16X1 TERMS = 1), else the single-CTA one.
+// CAUSAL: the causal kernels (ELT_F16 only).
+template <bool PAIR, int EP, int KID, bool NORM, int ELT, bool CAUSAL>
 int launch_one(const CUtensorMap* maps, const tc::Params& P, int grid, cudaStream_t stream) {
+    static_assert(!CAUSAL || ELT == tc::ELT_F16, "causal products run the three-term FP16 planes");
     constexpr int smem = tc::Cfg<EP, KID, NORM, PAIR>::SMEM_BYTES;
     KernelFn fn;
-    if constexpr (PAIR) fn = tc::pair::kprod_tensor_pair_kernel<EP, KID, NORM, ELT == tc::ELT_F16X1 ? 1 : 3>;
+    if constexpr (CAUSAL && PAIR) fn = tc::pair::kprod_tensor_pair_causal_kernel<EP, KID, NORM>;
+    else if constexpr (CAUSAL) fn = tc::kprod_tensor_causal_kernel<EP, KID, NORM>;
+    else if constexpr (PAIR) fn = tc::pair::kprod_tensor_pair_kernel<EP, KID, NORM, ELT == tc::ELT_F16X1 ? 1 : 3>;
     else fn = tc::kprod_tensor_kernel<EP, KID, NORM, ELT>;
     if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(fn), smem)) return rc;
     fn<<<grid, tc::THREADS, smem, stream>>>(maps[0], maps[1], maps[2], maps[3], P);
@@ -847,25 +933,25 @@ int launch_one(const CUtensorMap* maps, const tc::Params& P, int grid, cudaStrea
     return KMB_OK;
 }
 
-template <bool PAIR, int KID, bool NORM, int ELT>
+template <bool PAIR, int KID, bool NORM, int ELT, bool CAUSAL>
 int launch_ep(int ep, const CUtensorMap* maps, const tc::Params& P, int grid, cudaStream_t stream) {
-    if (ep == 1) return launch_one<PAIR, 1, KID, NORM, ELT>(maps, P, grid, stream);
-    if (ep == 2) return launch_one<PAIR, 2, KID, NORM, ELT>(maps, P, grid, stream);
-    return launch_one<PAIR, 4, KID, NORM, ELT>(maps, P, grid, stream);
+    if (ep == 1) return launch_one<PAIR, 1, KID, NORM, ELT, CAUSAL>(maps, P, grid, stream);
+    if (ep == 2) return launch_one<PAIR, 2, KID, NORM, ELT, CAUSAL>(maps, P, grid, stream);
+    return launch_one<PAIR, 4, KID, NORM, ELT, CAUSAL>(maps, P, grid, stream);
 }
 
 // ELT_F16X1 (one-term path): Gaussian and exponential epilogues only (the inverse distance is rejected by the C ABI)
-template <bool PAIR, int ELT>
+template <bool PAIR, int ELT, bool CAUSAL = false>
 int launch_any(int kid, bool norm, int ep, const CUtensorMap* maps, const tc::Params& P, int grid, cudaStream_t stream) {
     switch (kid * 2 + (norm ? 1 : 0)) {
-        case 0: return launch_ep<PAIR, KMB_KERNEL_GAUSSIAN, false, ELT>(ep, maps, P, grid, stream);
-        case 1: return launch_ep<PAIR, KMB_KERNEL_GAUSSIAN, true, ELT>(ep, maps, P, grid, stream);
-        case 2: return launch_ep<PAIR, KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false, ELT>(ep, maps, P, grid, stream);
-        case 3: return launch_ep<PAIR, KMB_KERNEL_ABSOLUTE_EXPONENTIAL, true, ELT>(ep, maps, P, grid, stream);
+        case 0: return launch_ep<PAIR, KMB_KERNEL_GAUSSIAN, false, ELT, CAUSAL>(ep, maps, P, grid, stream);
+        case 1: return launch_ep<PAIR, KMB_KERNEL_GAUSSIAN, true, ELT, CAUSAL>(ep, maps, P, grid, stream);
+        case 2: return launch_ep<PAIR, KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false, ELT, CAUSAL>(ep, maps, P, grid, stream);
+        case 3: return launch_ep<PAIR, KMB_KERNEL_ABSOLUTE_EXPONENTIAL, true, ELT, CAUSAL>(ep, maps, P, grid, stream);
     }
     if constexpr (ELT == tc::ELT_F16X1) return set_error(KMB_ERR_UNSUPPORTED, "no one-term kernel for kernel id %d", kid);
-    else if (norm) return launch_ep<PAIR, KMB_KERNEL_INVERSE_DISTANCE, true, ELT>(ep, maps, P, grid, stream);
-    else return launch_ep<PAIR, KMB_KERNEL_INVERSE_DISTANCE, false, ELT>(ep, maps, P, grid, stream);
+    else if (norm) return launch_ep<PAIR, KMB_KERNEL_INVERSE_DISTANCE, true, ELT, CAUSAL>(ep, maps, P, grid, stream);
+    else return launch_ep<PAIR, KMB_KERNEL_INVERSE_DISTANCE, false, ELT, CAUSAL>(ep, maps, P, grid, stream);
 }
 
 }  // namespace
@@ -914,6 +1000,31 @@ int tensor_pv_plan_query(int64_t N, int64_t M, int D, int E, int kid, int elt, i
     return KMB_OK;   // an E <= 4 kernel: only the family
 }
 
+int tensor_causal_work_debug(int64_t N, int64_t M, int D, int E, int kid, int64_t row_offset, int sms, int smem_optin, int wave,
+                             int unit, long long out[CWQ_FIELDS]) {
+    static_assert(CWQ_FIELDS == KMB_CAUSAL_WORK_FIELDS, "kmb_debug_causal_work fields");
+    for (int i = 0; i < CWQ_FIELDS; ++i) out[i] = -1;
+    if (tensor_kind(D, E, kid, tc::ELT_F16) == KIND_PV16)
+        return tensor_pv16_causal_work_debug(N, M, D, E, row_offset, sms, smem_optin, wave, unit, out);
+    if (tensor_kind(D, E, kid, tc::ELT_F16) != KIND_TENSOR)
+        return set_error(KMB_ERR_UNSUPPORTED, "no causal kernel for the TF32 P.B family (inverse distance, E > 4, D <= 128)");
+    tc::Params P{};
+    P.N = N;
+    P.row_offset = row_offset;
+    P.n_tiles = static_cast<int>((N + tc::TM - 1) / tc::TM);
+    P.nsb = static_cast<int>((M + tc::TN - 1) / tc::TN);
+    bool pair;
+    int grid;
+    tc::WavePlan w;
+    tensor_wave_plan(P.n_tiles, P.nsb, (D + 15) / 16 * 16, true, sms, &pair, &grid, &w);
+    P.R = w.R; P.C = w.C; P.W = w.W; P.R_last = w.R_last; P.C_last = w.C_last;
+    tc::WaveWork ww;
+    const bool has = wave >= 0 && wave < P.W && unit >= 0 &&
+                     (pair ? tc::wave_work<true, tc::TN, true>(P, wave, unit, ww) : tc::wave_work<true, tc::TN, false>(P, wave, unit, ww));
+    causal_work_fill(pair ? KMB_FAMILY_TENSOR_PAIR : KMB_FAMILY_TENSOR, P.W, pair ? grid / 2 : grid, tc::TN, has ? &ww : nullptr, out);
+    return KMB_OK;
+}
+
 int tensor_workspace_bytes(int64_t N, int64_t M, int D, int E, int kid, int flags, int elt, size_t* bytes) {
     (void)flags;
     const int kind = tensor_kind(D, E, kid, elt);
@@ -942,7 +1053,10 @@ int tensor_product(const float* x, const float* y, const float* b, float* out, i
     const int kind = tensor_kind(D, E, kid, elt);
     if (kind == KIND_NONE) return kind_unsupported(D, E);
     if (kind == KIND_PV16)
-        return tensor_pv16_product(x, y, b, out, N, M, D, E, kid, flags, elt, workspace, workspace_bytes, stream, ev0, ev1, prepared);
+        return tensor_pv16_product(x, y, b, out, N, M, D, E, kid, flags, elt, row_offset, workspace, workspace_bytes, stream, ev0, ev1,
+                                   prepared);
+    if (kind == KIND_PV && (flags & KMB_FLAG_CAUSAL))
+        return set_error(KMB_ERR_UNSUPPORTED, "no causal kernel for the TF32 P.B family (inverse distance, E > 4, D <= 128)");
     if (kind == KIND_PV)
         return tensor_pv_product(x, y, b, out, N, M, D, E, kid, flags, row_offset, workspace, workspace_bytes, stream, ev0, ev1);
     TensorPlan pl{};
@@ -967,6 +1081,8 @@ int tensor_product(const float* x, const float* y, const float* b, float* out, i
     int* counters = reinterpret_cast<int*>(ws + pl.off_counter);
     const bool norm = flags & KMB_FLAG_NORMALIZE_ROWS;
     const bool density = flags & KMB_FLAG_DENSITY;
+    const bool causal = flags & KMB_FLAG_CAUSAL;   // the C ABI admits it with FP16 planes only
+    if (causal && elt != tc::ELT_F16) return set_error(KMB_ERR_UNSUPPORTED, "causal products run on the three-term FP16 path only");
 
     KMB_CUDA_CHECK(cudaMemsetAsync(counters, 0, sizeof(int) * pl.n_tiles, stream));
     CUtensorMap maps[4];
@@ -1016,7 +1132,9 @@ int tensor_product(const float* x, const float* y, const float* b, float* out, i
         if (ev0 && pass == pl.n_passes - 1) KMB_CUDA_CHECK(cudaEventRecord(ev0, stream));
         const int ekid = tc::epilogue_kid(kid);
         int rc;
-        if (pl.pair) rc = x1 ? launch_any<true, tc::ELT_F16X1>(ekid, norm, pl.e_chunk, maps, P, grid, stream)
+        if (causal) rc = pl.pair ? launch_any<true, tc::ELT_F16, true>(ekid, norm, pl.e_chunk, maps, P, grid, stream)
+                                 : launch_any<false, tc::ELT_F16, true>(ekid, norm, pl.e_chunk, maps, P, grid, stream);
+        else if (pl.pair) rc = x1 ? launch_any<true, tc::ELT_F16X1>(ekid, norm, pl.e_chunk, maps, P, grid, stream)
                              : launch_any<true, tc::ELT_F16>(ekid, norm, pl.e_chunk, maps, P, grid, stream);
         else if (x1) rc = launch_any<false, tc::ELT_F16X1>(ekid, norm, pl.e_chunk, maps, P, grid, stream);
         else if (f16) rc = launch_any<false, tc::ELT_F16>(ekid, norm, pl.e_chunk, maps, P, grid, stream);

@@ -36,4 +36,10 @@ void tensor_plan_debug(int64_t N, int D, int E, int kid, int elt, int sms, long 
 // only, the launchers' own plan functions; for an E <= 4 kernel only the family is filled.
 int tensor_pv_plan_query(int64_t N, int64_t M, int D, int E, int kid, int elt, int sms, int smem_optin, long long* out);
 
+// The work of `unit` in wave `wave` of the causal kernel (kprod_tensor, _pair, pv16, pv16_pair) that runs this FP16-plane
+// problem on a device of `sms` SMs with `smem_optin` bytes of opt-in shared memory per block: out = the
+// KMB_CAUSAL_WORK_FIELDS of kmb_debug_causal_work.  Host logic only, the kernels' own wave_work<CAUSAL = true>.
+int tensor_causal_work_debug(int64_t N, int64_t M, int D, int E, int kid, int64_t row_offset, int sms, int smem_optin, int wave,
+                             int unit, long long* out);
+
 }  // namespace kmb

@@ -117,6 +117,7 @@ struct Params {
     int E, e0, eb, ebp;        // this pass covers signal columns e0 .. e0+eb-1; ebp = eb rounded up to 32
     int n_tiles, nsb, kblocks, ksteps_last, stages, ep_rows, flush_blocks;
     int R, C, W, R_last, C_last, slots_per_wave;
+    long long row_offset;      // global index of row 0 (KMB_FLAG_CAUSAL: row i sees sources j <= row_offset + i)
 };
 
 // two floats -> one 32-bit word of two halves: `even` in bits [0,16), `odd` in bits [16,32)
@@ -160,7 +161,10 @@ __device__ __forceinline__ float2 neg_log2_kernel2(float2 s_raw, float2 nsscale,
 // 256 rows tall (half as many instructions per row tile -- the issuing warp is what bounds the single-CTA kernel),
 // each CTA streams half of every v block (64 sources) and half of every signal block (32 signal columns), the leader
 // CTA issues, tcgen05.commit multicasts to both CTAs' barriers and the peer's epilogue warps arrive on the leader's.
-template <int KID, bool NORM, bool PAIR, int TERMS>
+// CAUSAL: KMB_FLAG_CAUSAL -- the wave plan's source ranges end at the unit's diagonal (wave_work), a unit whose range is
+// empty loads nothing and writes an empty partial record, and the S columns of a block that crosses the diagonal are set
+// to -inf where j > row_offset + i, which every epilogue form turns into weight 0.
+template <int KID, bool NORM, bool PAIR, int TERMS, bool CAUSAL = false>
 __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUtensorMap& map_al, const CUtensorMap& map_bh,
                                           const CUtensorMap& map_bl, const CUtensorMap& map_sh, const CUtensorMap& map_sl,
                                           const CUtensorMap& map_ue, const CUtensorMap& map_ve, const Params& P) {
@@ -260,7 +264,8 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
         for (int q = 0; q < SST - 1; ++q) pend[q] = -1;
         WaveWork ww;
         for (int w = 0; w < P.W; ++w) {
-            if (!wave_work(P, w, cta, ww)) continue;
+            if (!wave_work<CAUSAL, TNS, PAIR>(P, w, cta, ww)) continue;
+            if (CAUSAL && ww.sb_lo == ww.sb_hi) continue;   // an empty range: no u tile, no S
             // new row tile: (re)load the resident u tile once the last S of the previous tile has read it
             mbar_wait(u_free, (seg & 1) ^ 1);
             const int my_row0 = (PAIR ? ww.tile * 2 + static_cast<int>(rank) : ww.tile) * TM;
@@ -368,7 +373,8 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
         uint32_t first_bits = 0;   // bit q: block n - q starts its O_g from zero
         WaveWork ww;
         for (int w = 0; w < P.W; ++w) {
-            if (!wave_work(P, w, cta, ww)) continue;
+            if (!wave_work<CAUSAL, TNS, PAIR>(P, w, cta, ww)) continue;
+            if (CAUSAL && ww.sb_lo == ww.sb_hi) continue;
             mbar_wait(u_full, seg & 1);
             ++seg;
             int until_flush = 0;   // blocks until the epilogue flushes the O_g again (a countdown: no division in the loop)
@@ -476,7 +482,8 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
         bool primed = false;
         WaveWork ww;
         for (int w = 0; w < P.W; ++w) {
-            if (!wave_work(P, w, cta, ww)) continue;
+            if (!wave_work<CAUSAL, TNS, PAIR>(P, w, cta, ww)) continue;
+            const bool empty = CAUSAL && ww.sb_lo == ww.sb_hi;   // no block, no P.B: the O_g are not this tile's
             const int tile = PAIR ? ww.tile * 2 + static_cast<int>(rank) : ww.tile;
             const long long row = static_cast<long long>(tile) * TM + row_in_tile;
             const bool row_ok = row < P.N;
@@ -493,7 +500,7 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
                     for (int c = 0; c < 16; ++c) atomicAdd(olong + (c0 + c) * TM, o[c]);   // RED: nothing to wait for
                 }
             };
-            if (!XK && !primed) {
+            if (!XK && !primed && !empty) {
                 fetch_vn(ww.sb_lo);
                 primed = true;
             }
@@ -502,7 +509,7 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
             {
                 WaveWork wn;
                 for (int w2 = w + 1; w2 < P.W && sb_next_tile < 0; ++w2)
-                    if (wave_work(P, w2, cta, wn)) sb_next_tile = wn.sb_lo;
+                    if (wave_work<CAUSAL, TNS, PAIR>(P, w2, cta, wn) && (!CAUSAL || wn.sb_lo < wn.sb_hi)) sb_next_tile = wn.sb_lo;
             }
 
             int until_flush = P.flush_blocks;   // blocks until this thread moves its O_g row to the long accumulator
@@ -524,6 +531,26 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
                 KMB_T(1);
                 float2 t2[CPT / 2];   // S as pairs of sources, then T = -log2 k / t_scale
                 tmem_ld_cols<CPT>(st_addr, reinterpret_cast<float(&)[CPT]>(t2));
+                // CAUSAL: S = -inf where j > row_offset + row, in a block whose columns of this group cross the tile's diagonal
+                // (warp-uniform); -inf makes the exponent -inf and the weight 0 in every form below, and leaves the maxima alone
+                [[maybe_unused]] bool crossing = false;
+                [[maybe_unused]] long long lim = 0;   // last visible column of this thread's row, relative to col0
+                if constexpr (CAUSAL) {
+                    const long long jb = static_cast<long long>(sb) * TNS + col0;
+                    crossing = jb + CPT - 1 > P.row_offset + static_cast<long long>(tile) * TM;
+                    lim = P.row_offset + row - jb;
+                }
+                auto mask_s = [&]() {
+                    if constexpr (CAUSAL) {
+                        if (crossing) {
+                            float* f = reinterpret_cast<float*>(t2);
+#pragma unroll
+                            for (int c = 0; c < CPT; ++c)
+                                if (c > lim) f[c] = -INFINITY;
+                        }
+                    }
+                };
+                mask_s();
                 KMB_T(2);
 
                 // Padded sources need no branch: their |v|^2 is 3.39e38, so their exponent is -3.39e38 or -inf and their
@@ -613,6 +640,7 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
                         done = !__any_sync(0xffffffffu, need);
                         if (!done) {
                             tmem_ld_cols<CPT>(st_addr, reinterpret_cast<float(&)[CPT]>(t2));
+                            mask_s();
                             kacc = make_float2(0.f, 0.f);
                         }
                     }
@@ -712,8 +740,10 @@ __device__ __forceinline__ void pv16_body(const CUtensorMap& map_ah, const CUten
             // ------------------------------ row tile done: merge the streams of the column groups ------------------------------
             refbuf[cg * TM + row_in_tile] = ref;
             ksbuf[cg * TM + row_in_tile] = ksum;
-            wait_pv(n - 1);   // the tile's last PV
-            flush_o();        // the long accumulators now hold the whole tile
+            if (!empty) {
+                wait_pv(n - 1);   // the tile's last PV
+                flush_o();        // the long accumulators now hold the whole tile
+            }
             __threadfence();
             named_bar_sync(2, EPI_THREADS);
             float rmax = -INFINITY, wg[NG], ktot = 0.f;
@@ -811,6 +841,24 @@ kprod_tensor_pv16_kernel(const __grid_constant__ CUtensorMap map_ah, const __gri
                          const __grid_constant__ CUtensorMap map_sh, const __grid_constant__ CUtensorMap map_sl,
                          const __grid_constant__ CUtensorMap map_ue, const __grid_constant__ CUtensorMap map_ve, const Params P) {
     pv16_body<KID, NORM, false, TERMS>(map_ah, map_al, map_bh, map_bl, map_sh, map_sl, map_ue, map_ve, P);
+}
+// KMB_FLAG_CAUSAL (three-term planes): kernels of their own, so that the instantiations above stay as they were
+template <int KID, bool NORM>
+__global__ void __launch_bounds__(THREADS, 1)
+kprod_tensor_pv16_causal_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant__ CUtensorMap map_al,
+                                const __grid_constant__ CUtensorMap map_bh, const __grid_constant__ CUtensorMap map_bl,
+                                const __grid_constant__ CUtensorMap map_sh, const __grid_constant__ CUtensorMap map_sl,
+                                const __grid_constant__ CUtensorMap map_ue, const __grid_constant__ CUtensorMap map_ve, const Params P) {
+    pv16_body<KID, NORM, false, 3, true>(map_ah, map_al, map_bh, map_bl, map_sh, map_sl, map_ue, map_ve, P);
+}
+template <int KID, bool NORM>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
+kprod_tensor_pv16_pair_causal_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant__ CUtensorMap map_al,
+                                     const __grid_constant__ CUtensorMap map_bh, const __grid_constant__ CUtensorMap map_bl,
+                                     const __grid_constant__ CUtensorMap map_sh, const __grid_constant__ CUtensorMap map_sl,
+                                     const __grid_constant__ CUtensorMap map_ue, const __grid_constant__ CUtensorMap map_ve,
+                                     const Params P) {
+    pv16_body<KID, NORM, true, 3, true>(map_ah, map_al, map_bh, map_bl, map_sh, map_sl, map_ue, map_ve, P);
 }
 template <int KID, bool NORM, int TERMS>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
@@ -976,7 +1024,16 @@ int plan_pv16(int64_t N, int64_t M, int D, int E, Pv16Plan* pl) {
 }
 
 template <int KID, bool NORM, int TERMS>
-int launch_pv16(const CUtensorMap* m, const pv16::Params& P, int grid, int smem, bool pair, cudaStream_t stream) {
+int launch_pv16(const CUtensorMap* m, const pv16::Params& P, int grid, int smem, bool pair, bool causal, cudaStream_t stream) {
+    if constexpr (TERMS == 3) {
+        if (causal) {
+            auto fn = pair ? pv16::kprod_tensor_pv16_pair_causal_kernel<KID, NORM> : pv16::kprod_tensor_pv16_causal_kernel<KID, NORM>;
+            if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(fn), smem)) return rc;
+            fn<<<grid, pv16::THREADS, smem, stream>>>(m[0], m[1], m[2], m[3], m[4], m[5], m[6], m[7], P);
+            KMB_CUDA_CHECK(cudaGetLastError());
+            return KMB_OK;
+        }
+    }
     if (pair) {
         auto fn = pv16::kprod_tensor_pv16_pair_kernel<KID, NORM, TERMS>;
         if (int rc = ensure_dyn_smem(reinterpret_cast<const void*>(fn), smem)) return rc;
@@ -1019,6 +1076,23 @@ int tensor_pv16_plan_debug(int64_t N, int64_t M, int D, int E, int sms, int smem
     return KMB_OK;
 }
 
+int tensor_pv16_causal_work_debug(int64_t N, int64_t M, int D, int E, int64_t row_offset, int sms, int smem_optin, int wave, int unit,
+                                  long long out[CWQ_FIELDS]) {
+    Pv16Plan pl{};
+    if (int rc = plan_pv16_host(N, M, D, E, sms, smem_optin, &pl)) return rc;
+    pv16::Params P{};
+    P.N = N;
+    P.row_offset = row_offset;
+    P.nsb = static_cast<int>(pl.nsb);
+    P.R = pl.waves.R; P.C = pl.waves.C; P.W = pl.waves.W; P.R_last = pl.waves.R_last; P.C_last = pl.waves.C_last;
+    tc::WaveWork ww;
+    const bool has = wave >= 0 && wave < P.W && unit >= 0 &&
+                     (pl.pair ? tc::wave_work<true, pv16::TNS, true>(P, wave, unit, ww) : tc::wave_work<true, pv16::TNS, false>(P, wave, unit, ww));
+    causal_work_fill(pl.pair ? KMB_FAMILY_PV16_PAIR : KMB_FAMILY_PV16, P.W, pl.pair ? pl.grid / 2 : pl.grid, pv16::TNS,
+                     has ? &ww : nullptr, out);
+    return KMB_OK;
+}
+
 int tensor_pv16_workspace_bytes(int64_t N, int64_t M, int D, int E, size_t* bytes) {
     Pv16Plan pl{};
     if (int rc = plan_pv16(N, M, D, E, &pl)) return rc;
@@ -1027,8 +1101,8 @@ int tensor_pv16_workspace_bytes(int64_t N, int64_t M, int D, int E, size_t* byte
 }
 
 int tensor_pv16_product(const float* x, const float* y, const float* b, float* out, int64_t N, int64_t M, int D, int E, int kid,
-                        int flags, int elt, void* workspace, size_t workspace_bytes, cudaStream_t stream, cudaEvent_t ev0,
-                        cudaEvent_t ev1, bool prepared) {
+                        int flags, int elt, int64_t row_offset, void* workspace, size_t workspace_bytes, cudaStream_t stream,
+                        cudaEvent_t ev0, cudaEvent_t ev1, bool prepared) {
     Pv16Plan pl{};
     if (int rc = plan_pv16(N, M, D, E, &pl)) return rc;
     if (!workspace || workspace_bytes < pl.total)
@@ -1042,6 +1116,8 @@ int tensor_pv16_product(const float* x, const float* y, const float* b, float* o
     int* counters = reinterpret_cast<int*>(ws + pl.off_counter);
     const bool norm = flags & KMB_FLAG_NORMALIZE_ROWS;
     const bool x1 = elt == tc::ELT_F16X1;   // one term: the lo planes are not read, their maps repeat the hi ones
+    const bool causal = flags & KMB_FLAG_CAUSAL;
+    if (causal && x1) return set_error(KMB_ERR_UNSUPPORTED, "causal products run on the three-term FP16 path only");
 
     KMB_CUDA_CHECK(cudaMemsetAsync(counters, 0, sizeof(int) * pl.n_tiles, stream));
     if (!prepared) {
@@ -1122,17 +1198,18 @@ int tensor_pv16_product(const float* x, const float* y, const float* b, float* o
         P.R_last = pl.waves.R_last;
         P.C_last = pl.waves.C_last;
         P.slots_per_wave = pl.waves.slots_per_wave;
+        P.row_offset = row_offset;
         if (ev0 && pass == n_passes - 1) KMB_CUDA_CHECK(cudaEventRecord(ev0, stream));
         int rc;
         switch (ekid * 4 + (norm ? 2 : 0) + (x1 ? 1 : 0)) {
-            case 0: rc = launch_pv16<KMB_KERNEL_GAUSSIAN, false, 3>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
-            case 1: rc = launch_pv16<KMB_KERNEL_GAUSSIAN, false, 1>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
-            case 2: rc = launch_pv16<KMB_KERNEL_GAUSSIAN, true, 3>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
-            case 3: rc = launch_pv16<KMB_KERNEL_GAUSSIAN, true, 1>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
-            case 4: rc = launch_pv16<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false, 3>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
-            case 5: rc = launch_pv16<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false, 1>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
-            case 6: rc = launch_pv16<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, true, 3>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
-            default: rc = launch_pv16<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, true, 1>(maps, P, pl.grid, pl.smem, pl.pair, stream); break;
+            case 0: rc = launch_pv16<KMB_KERNEL_GAUSSIAN, false, 3>(maps, P, pl.grid, pl.smem, pl.pair, causal, stream); break;
+            case 1: rc = launch_pv16<KMB_KERNEL_GAUSSIAN, false, 1>(maps, P, pl.grid, pl.smem, pl.pair, causal, stream); break;
+            case 2: rc = launch_pv16<KMB_KERNEL_GAUSSIAN, true, 3>(maps, P, pl.grid, pl.smem, pl.pair, causal, stream); break;
+            case 3: rc = launch_pv16<KMB_KERNEL_GAUSSIAN, true, 1>(maps, P, pl.grid, pl.smem, pl.pair, causal, stream); break;
+            case 4: rc = launch_pv16<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false, 3>(maps, P, pl.grid, pl.smem, pl.pair, causal, stream); break;
+            case 5: rc = launch_pv16<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, false, 1>(maps, P, pl.grid, pl.smem, pl.pair, causal, stream); break;
+            case 6: rc = launch_pv16<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, true, 3>(maps, P, pl.grid, pl.smem, pl.pair, causal, stream); break;
+            default: rc = launch_pv16<KMB_KERNEL_ABSOLUTE_EXPONENTIAL, true, 1>(maps, P, pl.grid, pl.smem, pl.pair, causal, stream); break;
         }
         if (rc) return rc;
         if (ev1 && pass == n_passes - 1) KMB_CUDA_CHECK(cudaEventRecord(ev1, stream));

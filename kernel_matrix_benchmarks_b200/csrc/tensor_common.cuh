@@ -302,18 +302,35 @@ void plan_waves(long long n_tiles, long long nsb, int grid, size_t row_tile_byte
 
 // Work of `unit` in wave w: row tile, source-block range [sb_lo, sb_hi), range index c of Cw.  The unit is a CTA, or the
 // cluster of a CTA pair, whose wave plan counts pairs of row tiles (`tile` is then the pair's index).
+//
+// CAUSAL (KMB_FLAG_CAUSAL, row i sees sources j <= row_offset + i): the Cw ranges split only the nb_t source blocks of
+// BLOCK sources that the unit's last row can see, nb_t = min(nsb, (row_offset + last row) / BLOCK + 1), so nothing above
+// the diagonal is scheduled; a range is empty when nb_t < Cw.  The tiles of odd waves are taken in reverse order
+// (serpentine): tile work grows with the tile index, and unit u then gets a light tile in one wave and a heavy one in the
+// next.  Host and device: kmb_debug_causal_work checks the plan without a GPU.
 struct WaveWork { int tile, sb_lo, sb_hi, c, Cw, tile_in_wave; };
-template <class Params>
-__device__ __forceinline__ bool wave_work(const Params& P, int w, int unit, WaveWork& ww) {
+template <bool CAUSAL = false, int BLOCK = 1, bool PAIR = false, class Params>
+__host__ __device__ __forceinline__ bool wave_work(const Params& P, int w, int unit, WaveWork& ww) {
     const bool last = (w == P.W - 1);
     const int Rw = last ? P.R_last : P.R, Cw = last ? P.C_last : P.C;
     if (unit >= Rw * Cw) return false;
     ww.Cw = Cw;
     ww.tile_in_wave = unit / Cw;
     ww.c = unit - ww.tile_in_wave * Cw;
-    ww.tile = w * P.R + ww.tile_in_wave;
-    ww.sb_lo = static_cast<int>(static_cast<long long>(P.nsb) * ww.c / Cw);
-    ww.sb_hi = static_cast<int>(static_cast<long long>(P.nsb) * (ww.c + 1) / Cw);
+    if constexpr (CAUSAL) {
+        if (w & 1) ww.tile_in_wave = Rw - 1 - ww.tile_in_wave;
+        ww.tile = w * P.R + ww.tile_in_wave;
+        const long long rows_end = static_cast<long long>(ww.tile + 1) * TM * (PAIR ? 2 : 1);
+        const long long last_row = (rows_end < P.N ? rows_end : P.N) - 1;
+        const long long nb_t = (P.row_offset + last_row) / BLOCK + 1;
+        const long long nb = nb_t < P.nsb ? nb_t : P.nsb;
+        ww.sb_lo = static_cast<int>(nb * ww.c / Cw);
+        ww.sb_hi = static_cast<int>(nb * (ww.c + 1) / Cw);
+    } else {
+        ww.tile = w * P.R + ww.tile_in_wave;
+        ww.sb_lo = static_cast<int>(static_cast<long long>(P.nsb) * ww.c / Cw);
+        ww.sb_hi = static_cast<int>(static_cast<long long>(P.nsb) * (ww.c + 1) / Cw);
+    }
     return true;
 }
 
@@ -347,6 +364,24 @@ inline void pv_plan_fill(int E, int max_eb, long long n_tiles, long long nsb, co
     out[PVQ_C_LAST] = w.C_last;
 }
 
+// What a causal tensor kernel schedules (kmb_debug_causal_work, include/kmb_b200.h): the fields of its `out`, in this order.
+enum { CWQ_FAMILY, CWQ_WAVES, CWQ_UNITS, CWQ_BLOCK, CWQ_TILE, CWQ_SB_LO, CWQ_SB_HI, CWQ_C, CWQ_CW, CWQ_FIELDS };
+inline void causal_work_fill(int family, int waves, int units, int block, const tc::WaveWork* ww, long long* out) {
+    out[CWQ_FAMILY] = family;
+    out[CWQ_WAVES] = waves;
+    out[CWQ_UNITS] = units;
+    out[CWQ_BLOCK] = block;
+    if (!ww) return;   // the unit has no row tile in this wave
+    out[CWQ_TILE] = ww->tile;
+    out[CWQ_SB_LO] = ww->sb_lo;
+    out[CWQ_SB_HI] = ww->sb_hi;
+    out[CWQ_C] = ww->c;
+    out[CWQ_CW] = ww->Cw;
+}
+// as tensor_causal_work_debug (kprod_tensor.cuh), for kprod_tensor_pv16 (kprod_tensor_pv16.cu)
+int tensor_pv16_causal_work_debug(int64_t N, int64_t M, int D, int E, int64_t row_offset, int sms, int smem_optin, int wave, int unit,
+                                  long long out[CWQ_FIELDS]);
+
 // E > 4 with D <= 128: second GEMM on the tensor cores (kprod_tensor_pv.cu)
 bool tensor_pv_applicable(int D, int E);
 // The plan of kprod_tensor_pv on a device of `sms` SMs with `smem_optin` bytes of opt-in shared memory per block (host
@@ -369,7 +404,7 @@ int tensor_pv16_plan_debug(int64_t N, int64_t M, int D, int E, int sms, int smem
 int tensor_pv16_workspace_bytes(int64_t N, int64_t M, int D, int E, size_t* bytes);
 // elt: tc::ELT_F16 (three-term S and P.B) or tc::ELT_F16X1 (hi.hi only; the lo planes are neither loaded nor written)
 int tensor_pv16_product(const float* x, const float* y, const float* b, float* out, int64_t N, int64_t M, int D, int E, int kid,
-                        int flags, int elt, void* workspace, size_t workspace_bytes, cudaStream_t stream, cudaEvent_t ev0,
+                        int flags, int elt, int64_t row_offset, void* workspace, size_t workspace_bytes, cudaStream_t stream, cudaEvent_t ev0,
                         cudaEvent_t ev1, bool prepared);
 
 // Head of the workspace of both FP16-plane kernels: everything the prepass writes from the points alone.  The layout

@@ -58,12 +58,14 @@ class DeviceGroup:
             out.append(t0.to(d, non_blocking=True))
         return out
 
-    def shard_rows(self, x0):
-        """Contiguous row blocks of ``x0`` (first device), block i copied to device i.  Returns (blocks, bounds)."""
+    def shard_rows(self, x0, bounds=None):
+        """Contiguous row blocks of ``x0`` (first device), block i copied to device i.  Returns (blocks, bounds).
+        ``bounds(n, i, n_devices) -> (lo, hi)``: the split (default: equal blocks, solver.shard_bounds)."""
         n = x0.shape[0]
+        split = bounds if bounds is not None else (lambda n_, i_, g_: shard_bounds(n_, i_, g_)[:2])
         blocks, bounds = [], []
         for i, d in enumerate(self.devices):
-            lo, hi, _ = shard_bounds(n, i, self.n)
+            lo, hi = split(n, i, self.n)
             blocks.append(x0[lo:hi] if i == 0 else x0[lo:hi].to(d, non_blocking=True).contiguous())
             bounds.append((lo, hi))
         return blocks, bounds
@@ -77,25 +79,26 @@ class DeviceGroup:
 
     # ------------------------------------------------------------------------------------------------ rows mode
 
-    def prepare_rows(self, xs, ys, *, kernel, path):
+    def prepare_rows(self, xs, ys, *, kernel, path, causal=False):
         """Per-device prepass of the tensor path (kmb_product_prepare_f32) for each device's row block; returns the
         tokens ``product_rows`` wants (None entries where nothing was prepared)."""
         tokens = []
         for i, d in enumerate(self.devices):
             with torch.cuda.device(d):
-                tokens.append(prepare_points(xs[i], ys[i], kernel=kernel, path=path, workspace=self.workspaces[i])
+                tokens.append(prepare_points(xs[i], ys[i], kernel=kernel, path=path, workspace=self.workspaces[i], causal=causal)
                               if xs[i].shape[0] else None)
         self.prepared = tokens
         return tokens
 
     def product_rows(self, xs, bounds, ys, bs, out0, *, kernel, normalize_rows=False, density_estimation=False, path="auto",
-                     prepared=None):
+                     prepared=None, causal=False):
         """Device i computes rows ``bounds[i]`` of the product and stores them straight into ``out0`` (N, E) on the
         first device through peer memory.  ``bs``: the signal per device (a list), or one tensor on the first device that
         the other devices read over NVLink.  Asynchronous; ordered on the first device's current stream."""
         lib = _lib.load()
         M, D = ys[0].shape
-        flags = (_lib.FLAG_NORMALIZE_ROWS if normalize_rows else 0) | (_lib.FLAG_DENSITY if density_estimation else 0)
+        flags = ((_lib.FLAG_NORMALIZE_ROWS if normalize_rows else 0) | (_lib.FLAG_DENSITY if density_estimation else 0)
+                 | (_lib.FLAG_CAUSAL if causal else 0))
         if density_estimation:
             E, bs = 1, [None] * self.n
         else:
@@ -107,12 +110,13 @@ class DeviceGroup:
         for i, d in enumerate(self.devices):
             lo, hi = bounds[i]
             need = workspace_bytes(max(hi - lo, 1), M, D, E, kernel=kernel, normalize_rows=normalize_rows,
-                                   density_estimation=density_estimation, path=path)
+                                   density_estimation=density_estimation, path=path, causal=causal)
             ws = self.workspaces[i].get(need, d)
             if prepared is not None and prepared[i] is not None and prepared[i] is not ws:
                 # the workspace had to grow for a wider signal: prepare once more, inside this (timed) query
                 with torch.cuda.device(d):
-                    prepared[i] = prepare_points(xs[i], ys[i], kernel=kernel, path=path, workspace=self.workspaces[i], min_bytes=need)
+                    prepared[i] = prepare_points(xs[i], ys[i], kernel=kernel, path=path, workspace=self.workspaces[i], min_bytes=need,
+                                                 causal=causal)
                 ws = self.workspaces[i].get(need, d)
             sh = shards[i]
             sh.device = d.index
